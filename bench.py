@@ -24,6 +24,9 @@ call per step).
 
 `--impl reference` times that CPU restatement with all host threads on the same config (the reference itself needs
 ROS + PCL and cannot be built in this image; see DESIGN.md).
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0's frames) as DIR/<name>.npy, see dump_outputs();
+the frames are generated from fixed seeds, so two builds run with the same arguments can be compared file for file.
 """
 import argparse
 import ctypes as C
@@ -210,6 +213,62 @@ def frame_alg_bytes(p, r):
     return b
 
 
+DUMP_FRAMES = 256        # frames of the batch whose result arrays --dump-outputs writes
+DUMP_LIMIT = 64 << 20    # bytes of all --dump-outputs files together
+SCALAR_FIELDS = ("status", "warnings", "n_input", "n_crop", "n_voxel", "n_sor", "n_remaining", "n_clusters",
+                 "n_cluster_points", "n_plane_passes", "n_plane_inliers")
+ARRAY_FIELDS = ("crop_kept_idx", "voxel_keys", "voxel_centroids", "sor_kept_idx", "plane_inlier_idx", "remaining_cloud",
+                "remaining_src_idx", "cluster_offsets", "cluster_indices", "obstacles")
+
+
+def dump_outputs(res, out_dir):
+    """Writes the host results of one pcop_process_batch call (`res`, its ctypes result array) to out_dir/<field>.npy.
+
+    Every frame: the counts and warnings (float64 [B]) and the plane records (plane_pass_points / plane_pass_inliers
+    float64 [B, 16], plane_pass_coeff float32 [B, 16, 4], zero past n_plane_passes; plane_coeff float32 [B, 4]).
+    The result arrays of a fixed sample of frames (seed 0, ascending, listed in frame_index.npy) are concatenated in
+    that order -- the frame's count fields split them: float arrays stay float32, index arrays become float64 (exact).
+    Frames are dropped from the end of the sample if all files together would exceed DUMP_LIMIT bytes."""
+    from pointcloud_obstacle_processing_b200 import Frame
+    from pointcloud_obstacle_processing_b200._ctypes_abi import MAX_PASSES
+    B = len(res)
+    out = {k: np.array([getattr(r, k) for r in res], np.float64) for k in SCALAR_FIELDS}
+    out["plane_pass_points"] = np.zeros((B, MAX_PASSES), np.float64)
+    out["plane_pass_inliers"] = np.zeros((B, MAX_PASSES), np.float64)
+    out["plane_pass_coeff"] = np.zeros((B, MAX_PASSES, 4), np.float32)
+    out["plane_coeff"] = np.zeros((B, 4), np.float32)
+    frames = {}
+    for k, r in enumerate(res):
+        f = Frame.from_c(r)
+        npass = len(f.plane_pass_points)
+        out["plane_pass_points"][k, :npass] = f.plane_pass_points
+        out["plane_pass_inliers"][k, :npass] = f.plane_pass_inliers
+        out["plane_pass_coeff"][k, :npass] = f.plane_pass_coeff
+        out["plane_coeff"][k] = f.plane_coeff
+        frames[k] = f
+    sample = np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_FRAMES), replace=False))
+    budget = DUMP_LIMIT - sum(a.nbytes for a in out.values()) - sample.size * 8 - 128 * (len(out) + len(ARRAY_FIELDS) + 1)
+    parts = {k: [] for k in ARRAY_FIELDS}
+    kept = []
+    for k in sample:
+        arrays = {name: getattr(frames[k], name) for name in ARRAY_FIELDS if getattr(frames[k], name) is not None}
+        arrays = {name: a if a.dtype == np.float32 else a.astype(np.float64) for name, a in arrays.items()}
+        size = sum(a.nbytes for a in arrays.values())
+        if size > budget:
+            break
+        budget -= size
+        kept.append(k)
+        for name, a in arrays.items():
+            parts[name].append(a)
+    out["frame_index"] = np.array(kept, np.float64)
+    for name, p in parts.items():
+        if p:
+            out[name] = np.concatenate(p)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def small_config(cfg, batch, reps, local_rank, peak, torch):
     """BASELINE configs[0] / [2] / [3]: single-frame latency (host in -> results on host) and a small device-resident
     batch, with its SURVEY 8(d) fraction."""
@@ -281,7 +340,10 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=128, help="frames of the CPU-baseline sample")
     ap.add_argument("--no-kernel-timing", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the BASELINE configs[0], [2], [3], [4] section")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -395,6 +457,8 @@ def main():
         own_wall = time.perf_counter() - t0  # this rank's own K steps (the line's time is the slowest rank's)
         barrier()
         wall = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:  # (before the next call on the handle reuses the result buffers)
+        dump_outputs(res, args.dump_outputs)
     stage_alg = {}
     for r in res:
         for k, v in frame_alg_bytes(params, r).items():
