@@ -16,6 +16,7 @@
  *   od.cpp:290-294  toROSMsg of the intermediate clouds (debug publishers)           -> pcop_cloud_to_pointcloud2
  *   od.cpp:727  build_initial_occupancy_grid_dataset  (grid part od.cpp:134-157, 184-269) -> pcop_occupancy_grid
  *   od.cpp:817-833  handle_shadow_casting per cluster (od.cpp:467-672) + obstacle marks   -> pcop_occupancy_shadows
+ *   od.cpp:699-852  pipeline + occupancy grid of a batch of frames                        -> pcop_process_batch_occupancy
  *
  * Plain C: POD structs, raw pointers and sizes, integer status codes.  No C++
  * exceptions, PCL, ROS or torch types cross this boundary.
@@ -291,6 +292,34 @@ int pcop_occupancy_grid(pcop_handle* h, const float* xyzw, int32_t n, int8_t* gr
 int pcop_occupancy_shadows(pcop_handle* h, const float* remaining_xyzw, int32_t n_remaining, const int32_t* cluster_offsets,
                            const int32_t* cluster_indices, int32_t n_clusters, const float* world_to_sensor16,
                            const float* sensor_to_world16, int8_t* grid_data, int32_t* shadow_records, uint32_t* warnings);
+
+/* ---- the node's published product for a batch of frames (od.cpp:699-852 per frame) ----------------------------
+ * Every frame of the batch through every enabled stage AND the occupancy grid it publishes, in one call: the initial
+ * data set of pcop_occupancy_grid, then the shadows and obstacle marks of pcop_occupancy_shadows on the frame's own
+ * remaining cloud and clusters.  Grid kernels run inside the batched pipeline; nothing returns to the host per frame.
+ *   xyzw, frame_stride_points, n, batch, out   as pcop_process_batch; every out[f] equals what pcop_process_batch
+ *                                              returns for the same frames (PCOP_OUT_DEVICE, pointer lifetime and
+ *                                              alternating pinned buffers included), except that
+ *                                              PCOP_WARN_SHADOW_DEGENERATE is set in the frames where a fan was skipped.
+ *                                              xyzw = NULL with batch = 1 (n ignored): the accumulated cloud, which the
+ *                                              call consumes like pcop_process_accumulated.
+ *   world_to_sensor16, sensor_to_world16       [batch][16] row-major floats (host memory), frame f's two TF lookups
+ *                                              (od.cpp:592 and od.cpp:570, 634); required
+ *   grids                                      [batch][height][width] int8 (host or device pointer; width / height
+ *                                              from pcop_occupancy_dims): frame f's grid equals, byte for byte,
+ *                                              pcop_occupancy_grid(frame f) followed by pcop_occupancy_shadows(frame f's
+ *                                              results, frame f's matrices).  Shadow records are not produced.
+ *                                              Host grids should be pinned (cudaHostAlloc): a copy into pageable memory
+ *                                              holds the calling thread until it lands, once per wave, so the lanes
+ *                                              stop overlapping.
+ * The handle keeps the counts (int32) and cells of one wave per lane, 5 bytes per cell and per frame of the largest
+ * wave the lane has run (allocated by the first call, grown when pcop_set_params enlarges the grid or a call brings
+ * larger waves): grids of more than PCOP_OCC_BATCH_MAX_CELLS cells give PCOP_ERR_CAPACITY (the single-frame calls
+ * above take grids up to 2^26 cells).  pcop_last_d2h_bytes counts the grid bytes copied to host memory. */
+#define PCOP_OCC_BATCH_MAX_CELLS (1 << 20)
+int pcop_process_batch_occupancy(pcop_handle* h, const float* xyzw, size_t frame_stride_points, const int32_t* n,
+                                 int32_t batch, const float* world_to_sensor16, const float* sensor_to_world16,
+                                 int8_t* grids, pcop_frame_result* out);
 
 /* Copies `bytes` from a device result array (PCOP_OUT_DEVICE) to host memory, or device to device when dst is a device
  * pointer; synchronous. */

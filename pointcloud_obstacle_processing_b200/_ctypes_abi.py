@@ -5,6 +5,8 @@ MAX_PASSES = 16  # PCOP_MAX_PLANE_PASSES_RECORDED
 
 OK, ERR_BAD_PARAM, ERR_CAPACITY, ERR_CUDA, ERR_INTERNAL = 0, 1, 2, 3, 4
 WARN_VOXEL_OVERFLOW_FALLBACK, WARN_SOR_TOO_FEW_POINTS, WARN_PLANE_BREAK, WARN_RNG_TABLE_EXHAUSTED = 1, 2, 4, 8
+WARN_SHADOW_DEGENERATE = 16
+OCC_BATCH_MAX_CELLS = 1 << 20  # PCOP_OCC_BATCH_MAX_CELLS
 OUT_CROP, OUT_VOXEL, OUT_SOR, OUT_PLANE, OUT_REMAINING, OUT_CLUSTERS, OUT_OBSTACLES = 1, 2, 4, 8, 16, 32, 64
 OUT_DEFAULT, OUT_ALL = 16 | 32 | 64, 127
 OUT_DEVICE = 256  # modifier: result arrays stay in device memory (pointers are device pointers)

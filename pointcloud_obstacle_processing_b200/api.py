@@ -8,6 +8,7 @@ Method names follow the reference's free functions (minibot_cr18/src/obstacle_de
   extract_euclidian_clusters   <- same name (sic)                                  (od.cpp:430-455)
   centroid_radius              <- PointWithRad/PointIndicesArray output            (msg/*.msg, od.cpp:806-814)
   process / process_batch      <- cloud_cb's process branch                        (od.cpp:699-927)
+  process_batch_occupancy      <- the same + the occupancy grid it publishes        (od.cpp:699-852)
 
 There is no CPU fallback: constructing an ObstacleProcessor without a usable B200-class device raises.
 """
@@ -44,6 +45,7 @@ EXPORTS = [
     "pcop_occupancy_grid",
     "pcop_occupancy_shadows",
     "pcop_download",
+    "pcop_process_batch_occupancy",
 ]
 
 
@@ -99,6 +101,7 @@ def load_library():
     L.pcop_occupancy_dims.argtypes = [vp, vp, vp]
     L.pcop_occupancy_grid.argtypes = [vp, vp, C.c_int32, vp, vp, vp]
     L.pcop_occupancy_shadows.argtypes = [vp, vp, C.c_int32, vp, vp, C.c_int32, vp, vp, vp, vp, vp]
+    L.pcop_process_batch_occupancy.argtypes = [vp, vp, C.c_size_t, vp, i32, vp, vp, vp, C.POINTER(FrameResult)]
     L.pcop_enable_kernel_timing.argtypes = [vp, C.c_int]
     L.pcop_kernel_timing_count.argtypes = [vp]
     L.pcop_kernel_timing_get.argtypes = [vp, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_double),
@@ -202,6 +205,51 @@ class ObstacleProcessor:
             counts = np.full(clouds.shape[0], clouds.shape[1], np.int32)
         res = self.process_batch_raw(clouds.ctypes.data, clouds.shape[1], counts)
         return [Frame.from_c(r) for r in res]
+
+    # ---- pipeline + occupancy grid (the node's published product) --------------------------
+    def occupancy_dims(self):
+        """(width, height) of the occupancy grid (od.cpp:958-959)"""
+        w, h = C.c_int32(), C.c_int32()
+        self._check(self._lib.pcop_occupancy_dims(self._h, C.byref(w), C.byref(h)))
+        return w.value, h.value
+
+    def process_batch_occupancy_raw(self, ptr, frame_stride_points: int, counts, world_to_sensor, sensor_to_world,
+                                    grids_ptr: int):
+        """pcop_process_batch_occupancy on frames at a raw host or device address (ptr = None: the accumulated cloud,
+        batch 1), grids written to a raw host or device address ([B, H, W] int8).  world_to_sensor / sensor_to_world:
+        [B, 4, 4] float32 (one pose per frame).  Returns the ctypes result array (valid until the next call)."""
+        counts = np.ascontiguousarray(np.zeros(1, np.int32) if counts is None else counts, dtype=np.int32)
+        B = len(counts)
+        ws = np.ascontiguousarray(world_to_sensor, np.float32).reshape(-1, 16)
+        sw = np.ascontiguousarray(sensor_to_world, np.float32).reshape(-1, 16)
+        if ws.shape[0] != B or sw.shape[0] != B:
+            raise ValueError(f"one world_to_sensor and one sensor_to_world matrix per frame ({B})")
+        res = (FrameResult * B)()
+        self._check(self._lib.pcop_process_batch_occupancy(
+            self._h, None if ptr is None else C.c_void_p(ptr), frame_stride_points, counts.ctypes.data_as(C.c_void_p), B,
+            ws.ctypes.data_as(C.c_void_p), sw.ctypes.data_as(C.c_void_p), C.c_void_p(grids_ptr), res))
+        return res
+
+    def process_batch_occupancy(self, clouds, world_to_sensor, sensor_to_world, counts=None):
+        """clouds: float32 [B, n, 4] (host), or None for the accumulated cloud (B = 1; the accumulator is emptied).
+        world_to_sensor / sensor_to_world: [B, 4, 4] float32, frame f's TF lookups (od.cpp:592 / 570, 634).
+        Returns (list of Frame, grids int8 [B, H, W]): every frame through the pipeline and the occupancy grid the node
+        publishes for it (initial data set, shadows, obstacle marks).  The grids land in a pageable numpy array, whose
+        copies hold the host once per wave; for throughput pass pinned or device memory to
+        process_batch_occupancy_raw."""
+        self._host_results_only()
+        w, h = self.occupancy_dims()
+        if clouds is None:
+            ptr, stride, counts = None, 1, np.zeros(1, np.int32)
+        else:
+            clouds = np.ascontiguousarray(clouds, dtype=np.float32)
+            assert clouds.ndim == 3 and clouds.shape[2] == 4
+            if counts is None:
+                counts = np.full(clouds.shape[0], clouds.shape[1], np.int32)
+            ptr, stride = clouds.ctypes.data, clouds.shape[1]
+        grids = np.empty((len(counts), h, w), np.int8)
+        res = self.process_batch_occupancy_raw(ptr, stride, counts, world_to_sensor, sensor_to_world, grids.ctypes.data)
+        return [Frame.from_c(r) for r in res], grids
 
     # ---- accumulator ingest (od.cpp:691-698) ------------------------------------------
     def accumulate(self, cloud, transform=None, is_dense=False) -> int:
