@@ -17,6 +17,7 @@
  *   od.cpp:727  build_initial_occupancy_grid_dataset  (grid part od.cpp:134-157, 184-269) -> pcop_occupancy_grid
  *   od.cpp:817-833  handle_shadow_casting per cluster (od.cpp:467-672) + obstacle marks   -> pcop_occupancy_shadows
  *   od.cpp:699-852  pipeline + occupancy grid of a batch of frames                        -> pcop_process_batch_occupancy
+ *   od.cpp:688-696 + 699-852  the same for a batch of raw PointCloud2 messages with a pose each -> pcop_process_batch_pointcloud2
  *
  * Plain C: POD structs, raw pointers and sizes, integer status codes.  No C++
  * exceptions, PCL, ROS or torch types cross this boundary.
@@ -320,6 +321,45 @@ int pcop_occupancy_shadows(pcop_handle* h, const float* remaining_xyzw, int32_t 
 int pcop_process_batch_occupancy(pcop_handle* h, const float* xyzw, size_t frame_stride_points, const int32_t* n,
                                  int32_t batch, const float* world_to_sensor16, const float* sensor_to_world16,
                                  int8_t* grids, pcop_frame_result* out);
+
+/* ---- a batch of raw sensor_msgs/PointCloud2 messages (od.cpp:688-696 + 699-852 per message) ------------------------
+ * A log replay, or several robots sharing one GPU, hands over sensor-frame messages, each with its own TF and its own
+ * driver's record layout.  pcop_process_batch_pointcloud2 decodes every message (toPCL + fromPCLPointCloud2<PointXYZ>),
+ * transforms it into the world frame (pcl_ros::transformPointCloud) and runs it through the batched pipeline -- and,
+ * with grids != NULL, the grid product of pcop_process_batch_occupancy -- in one call.  Decode and transform run on the
+ * GPU inside the batched pipeline; nothing returns to the host per message.
+ *   frames             [batch] message descriptors (host memory); layouts may differ from message to message.  A
+ *                      message with n_points == 0 may have data == NULL.  Payloads may be host or device pointers
+ *                      (classified per message).  Host payloads should be pinned (cudaHostAlloc): a copy from pageable
+ *                      memory holds the calling thread until it has been staged, once per message, so the lanes stop
+ *                      overlapping.  Device payloads are read in place.
+ *   transform16        [batch][16] row-major floats (host memory), message f's world <- sensor pose, applied with
+ *                      pcl::transformPointCloud's coefficient formula (is_dense = 0: records with a non-finite x, y or z
+ *                      are copied untransformed); NULL: no transform (payloads already in the world frame)
+ *   world_to_sensor16, sensor_to_world16, grids    as pcop_process_batch_occupancy; grids = NULL: pipeline only (the two
+ *                      matrices are then not read).  A replay of single messages passes the same array as transform16
+ *                      and sensor_to_world16.
+ *   out                [batch]
+ * out[f] equals, byte for byte, what pcop_accumulate_reset + pcop_accumulate_pointcloud2(message f, transform16 + 16 f)
+ * + pcop_process_accumulated return, i.e. pcop_process_batch on the decoded world clouds (padding float 1.0f); with grids,
+ * results and grids equal pcop_process_batch_occupancy on those clouds with the same matrices.  PCOP_OUT_DEVICE, result
+ * pointer lifetime and the alternating pinned result buffers behave as in pcop_process_batch.  The accumulator is neither
+ * read nor changed.
+ * Errors (the handle stays usable): PCOP_ERR_BAD_PARAM for a negative n_points, point_step < 4, a field offset with
+ * off + 4 > point_step, NULL data with n_points > 0, frames = NULL with batch > 0, or grids without the two matrices;
+ * PCOP_ERR_CAPACITY for n_points > max_points or a grid above PCOP_OCC_BATCH_MAX_CELLS.  batch = 0 does nothing.
+ * Every lane of the handle stages the host payloads of one wave (allocated by the first call, grown to the largest wave's
+ * payload bytes); pcop_stage_times_us counts the upload and the decode as PCOP_STAGE_H2D. */
+typedef struct pcop_pointcloud2_frame {
+  const unsigned char* data;   /* PointCloud2.data: host or device pointer                        */
+  int32_t n_points;            /* width * height records                                           */
+  int32_t point_step;          /* bytes per record                                                  */
+  int32_t off_x, off_y, off_z; /* offsets of the FLOAT32 fields "x", "y", "z" (little-endian)       */
+  int32_t is_dense;            /* 0: PCL's rule for is_dense == false, non-finite points untransformed */
+} pcop_pointcloud2_frame;
+int pcop_process_batch_pointcloud2(pcop_handle* h, const pcop_pointcloud2_frame* frames, int32_t batch,
+                                   const float* transform16, const float* world_to_sensor16,
+                                   const float* sensor_to_world16, int8_t* grids, pcop_frame_result* out);
 
 /* Copies `bytes` from a device result array (PCOP_OUT_DEVICE) to host memory, or device to device when dst is a device
  * pointer; synchronous. */

@@ -40,6 +40,14 @@ class Params(C.Structure):
         return other
 
 
+class PointCloud2Frame(C.Structure):
+    """pcop_pointcloud2_frame: one sensor_msgs/PointCloud2 message (data = host or device address)."""
+    _fields_ = [
+        ("data", C.c_void_p), ("n_points", C.c_int32), ("point_step", C.c_int32),
+        ("off_x", C.c_int32), ("off_y", C.c_int32), ("off_z", C.c_int32), ("is_dense", C.c_int32),
+    ]
+
+
 class FrameResult(C.Structure):
     """pcop_frame_result."""
     _fields_ = [

@@ -12,14 +12,22 @@ Method names follow the reference's free functions (minibot_cr18/src/obstacle_de
 
 There is no CPU fallback: constructing an ObstacleProcessor without a usable B200-class device raises.
 """
+import collections
 import ctypes as C
 import os
 
 import numpy as np
 
 from . import _ctypes_abi as abi
-from ._ctypes_abi import FrameResult, Params
+from ._ctypes_abi import FrameResult, Params, PointCloud2Frame
 from .result import Frame
+
+
+class PointCloud2Message(collections.namedtuple("PointCloud2Message",
+                                                "data n_points point_step off_x off_y off_z is_dense",
+                                                defaults=(False,))):
+    """The fields of a sensor_msgs/PointCloud2 message that the decode reads: data (bytes or uint8 array, host),
+    n_points = width * height, point_step and the byte offsets of the FLOAT32 fields x, y, z."""
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpcop.so")
@@ -46,6 +54,7 @@ EXPORTS = [
     "pcop_occupancy_shadows",
     "pcop_download",
     "pcop_process_batch_occupancy",
+    "pcop_process_batch_pointcloud2",
 ]
 
 
@@ -102,6 +111,8 @@ def load_library():
     L.pcop_occupancy_grid.argtypes = [vp, vp, C.c_int32, vp, vp, vp]
     L.pcop_occupancy_shadows.argtypes = [vp, vp, C.c_int32, vp, vp, C.c_int32, vp, vp, vp, vp, vp]
     L.pcop_process_batch_occupancy.argtypes = [vp, vp, C.c_size_t, vp, i32, vp, vp, vp, C.POINTER(FrameResult)]
+    L.pcop_process_batch_pointcloud2.argtypes = [vp, C.POINTER(PointCloud2Frame), i32, vp, vp, vp, vp,
+                                                 C.POINTER(FrameResult)]
     L.pcop_enable_kernel_timing.argtypes = [vp, C.c_int]
     L.pcop_kernel_timing_count.argtypes = [vp]
     L.pcop_kernel_timing_get.argtypes = [vp, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_double),
@@ -250,6 +261,60 @@ class ObstacleProcessor:
         grids = np.empty((len(counts), h, w), np.int8)
         res = self.process_batch_occupancy_raw(ptr, stride, counts, world_to_sensor, sensor_to_world, grids.ctypes.data)
         return [Frame.from_c(r) for r in res], grids
+
+    # ---- raw PointCloud2 messages, one pose each (od.cpp:688-696 + 699-852 per message) ------------------
+    def process_batch_pointcloud2_raw(self, frames, transforms=None, world_to_sensor=None, sensor_to_world=None,
+                                      grids_ptr=None):
+        """pcop_process_batch_pointcloud2.  frames: a sequence of PointCloud2Frame (data = host or device address).
+        transforms / world_to_sensor / sensor_to_world: [B, 4, 4] float32 or None; grids_ptr: raw host or device
+        address of [B, H, W] int8, or None (pipeline only).  Returns the ctypes result array (valid until the next
+        call)."""
+        B = len(frames)
+        arr = (PointCloud2Frame * max(B, 1))(*frames)
+
+        def mats(m, what):
+            if m is None:
+                return None, None
+            m = np.ascontiguousarray(m, np.float32).reshape(-1, 16)
+            if m.shape[0] != B:
+                raise ValueError(f"one {what} matrix per message ({B})")
+            return m, m.ctypes.data_as(C.c_void_p)
+        (t, tp), (ws, wsp), (sw, swp) = mats(transforms, "transform"), mats(world_to_sensor, "world_to_sensor"), \
+            mats(sensor_to_world, "sensor_to_world")
+        res = (FrameResult * max(B, 1))()
+        self._check(self._lib.pcop_process_batch_pointcloud2(
+            self._h, arr, B, tp, wsp, swp, None if grids_ptr is None else C.c_void_p(grids_ptr), res))
+        return res[:B] if B else []
+
+    def process_batch_pointcloud2(self, messages, transforms=None, world_to_sensor=None, sensor_to_world=None,
+                                  grids=False):
+        """messages: a sequence of PointCloud2Message (host payloads).  transforms: [B, 4, 4] float32, message f's
+        world <- sensor pose, or None when the payloads are already in the world frame.  Returns the list of Frame, or
+        (frames, grids int8 [B, H, W]) with grids=True (then world_to_sensor / sensor_to_world are required, as in
+        process_batch_occupancy; a replay of single messages passes its poses as transforms and sensor_to_world).
+        Pageable payloads and grids hold the host per copy; for throughput pass pinned or device memory to
+        process_batch_pointcloud2_raw."""
+        self._host_results_only()
+        keep, frames = [], []
+        for m in messages:
+            m = PointCloud2Message(*m)
+            if m.data is None:
+                buf = np.zeros(0, np.uint8)
+            elif isinstance(m.data, np.ndarray):
+                buf = np.ascontiguousarray(m.data.reshape(-1)).view(np.uint8)
+            else:
+                buf = np.frombuffer(m.data, np.uint8)
+            keep.append(buf)
+            frames.append(PointCloud2Frame(buf.ctypes.data if buf.size else None, m.n_points, m.point_step, m.off_x,
+                                           m.off_y, m.off_z, 1 if m.is_dense else 0))
+        g = None
+        if grids:
+            w, h = self.occupancy_dims()
+            g = np.empty((len(frames), h, w), np.int8)
+        res = self.process_batch_pointcloud2_raw(frames, transforms, world_to_sensor, sensor_to_world,
+                                                 None if g is None else g.ctypes.data)
+        out = [Frame.from_c(r) for r in res]
+        return (out, g) if grids else out
 
     # ---- accumulator ingest (od.cpp:691-698) ------------------------------------------
     def accumulate(self, cloud, transform=None, is_dense=False) -> int:

@@ -77,6 +77,13 @@ struct PackMeta {  // device -> host in one copy
   int overflow;     // the wave's arrays do not fit the pack buffer (nothing was packed)
 };
 
+struct Pc2Frame {  // decode descriptor of one PointCloud2 message (device memory, read by k_pc2_ingest)
+  const unsigned char* data;  // payload on the device
+  int n, point_step, off_x, off_y, off_z;
+  int is_dense, apply_transform, aligned;
+  Mat34 t;
+};
+
 thread_local std::string g_global_error;
 
 constexpr int PCOP_MIN_LANE_WAVE = 8;  // a call is split over the lanes only when every lane gets at least this many frames
@@ -149,8 +156,10 @@ struct pcop_handle {
     bool grids_on_device;
   };
   const OccCall* occ = nullptr;
-  unsigned char* d_raw = nullptr;  // staging for a raw PointCloud2 payload (grown on demand)
-  size_t raw_cap = 0;
+  unsigned char* d_raw = nullptr;  // staging of raw PointCloud2 payloads from host memory: one message, or the host
+  size_t raw_cap = 0;              // messages of one wave at 256-byte aligned offsets (grown on demand)
+  Pc2Frame* d_pc2 = nullptr;       // [maxB] decode descriptors of k_pc2_ingest
+  Pc2Frame* h_pc2 = nullptr;       // [maxB] pinned staging of the same (the batched PointCloud2 wave)
   int acc_count = 0;
   size_t pack_cap = 0;
   uint32_t alloc_outputs = 0;
@@ -372,6 +381,18 @@ int ensure_host_pack(pcop_handle* h, size_t need) {
   return PCOP_OK;
 }
 
+// the raw PointCloud2 staging of lane h holds at least `bytes` (grown by a quarter more, never shrunk)
+int ensure_raw(pcop_handle* h, size_t bytes) {
+  if (bytes <= h->raw_cap) return PCOP_OK;
+  PCOP_CUDA_TRY(cudaStreamSynchronize(h->stream));
+  if (h->d_raw) cudaFree(h->d_raw);  // (not tracked in dev_allocs)
+  h->d_raw = nullptr;
+  h->raw_cap = 0;
+  PCOP_CUDA_TRY(cudaMalloc((void**)&h->d_raw, bytes + bytes / 4 + 256));
+  h->raw_cap = bytes + bytes / 4 + 256;
+  return PCOP_OK;
+}
+
 // ---- small kernels owned by the API layer -----------------------------------------
 __global__ void k_copy_counts(const int* __restrict__ src, int* __restrict__ dst, int B) {
   const int f = blockIdx.x * blockDim.x + threadIdx.x;
@@ -407,21 +428,66 @@ __device__ __forceinline__ float pc2_load_f32(const unsigned char* p) {
   const uint32_t b = (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
   return __uint_as_float(b);
 }
+__device__ __forceinline__ float pc2_lane(const float4& v, int k) {  // (compares, not an indexed register array)
+  return k == 0 ? v.x : (k == 1 ? v.y : (k == 2 ? v.z : v.w));
+}
+// One decode per message (pcop_accumulate_pointcloud2 / pcop_pointcloud2_to_xyz: one frame; the batched PointCloud2
+// wave: one frame per message).  blockIdx.y = frame, records along x.  Every per-frame quantity comes from the
+// descriptor table in device memory.  aligned = 1 (point_step % 16 == 0, 16-byte aligned base, x / y / z inside one
+// aligned 16-byte word of the record): one 16-byte load per record instead of three 4-byte (or twelve 1-byte) loads.
 __global__ void __launch_bounds__(256)
-    k_pc2_ingest(const unsigned char* __restrict__ data, int n, int point_step, int off_x, int off_y, int off_z, Mat34 t,
-                 int apply_transform, int is_dense, float4* __restrict__ out) {
+    k_pc2_ingest(const Pc2Frame* __restrict__ frames, float4* __restrict__ out, size_t out_stride) {
+  const int f = blockIdx.y;
+  const int n = frames[f].n;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const unsigned char* rec = data + (size_t)i * (size_t)point_step;
-  const float x = pc2_load_f32(rec + off_x), y = pc2_load_f32(rec + off_y), z = pc2_load_f32(rec + off_z);
+  const Pc2Frame& d = frames[f];
+  const unsigned char* rec = d.data + (size_t)i * (size_t)d.point_step;
+  float x, y, z;
+  if (d.aligned) {
+    const float4 v = __ldg(reinterpret_cast<const float4*>(rec + (d.off_x & ~15)));
+    x = pc2_lane(v, (d.off_x & 15) >> 2);
+    y = pc2_lane(v, (d.off_y & 15) >> 2);
+    z = pc2_lane(v, (d.off_z & 15) >> 2);
+  } else {
+    x = pc2_load_f32(rec + d.off_x);
+    y = pc2_load_f32(rec + d.off_y);
+    z = pc2_load_f32(rec + d.off_z);
+  }
   float4 o = make_float4(x, y, z, 1.0f);
   const bool finite = fabsf(x) <= 3.402823466e+38f && fabsf(y) <= 3.402823466e+38f && fabsf(z) <= 3.402823466e+38f;
-  if (apply_transform && (is_dense || finite)) {
+  if (d.apply_transform && (d.is_dense || finite)) {
+    const Mat34& t = d.t;
     o.x = fadd(fadd(fadd(fmul(t.m[0], x), fmul(t.m[1], y)), fmul(t.m[2], z)), t.m[3]);
     o.y = fadd(fadd(fadd(fmul(t.m[4], x), fmul(t.m[5], y)), fmul(t.m[6], z)), t.m[7]);
     o.z = fadd(fadd(fadd(fmul(t.m[8], x), fmul(t.m[9], y)), fmul(t.m[10], z)), t.m[11]);
   }
-  out[i] = o;
+  out[(size_t)f * out_stride + i] = o;
+}
+
+// the descriptor of one message whose payload sits at `src` on the device (validated by the caller)
+Pc2Frame make_pc2_frame(const unsigned char* src, int n, int point_step, int ox, int oy, int oz, const float* t16,
+                        int is_dense) {
+  Pc2Frame d{};
+  d.data = src;
+  d.n = n;
+  d.point_step = point_step;
+  d.off_x = ox;
+  d.off_y = oy;
+  d.off_z = oz;
+  d.is_dense = is_dense ? 1 : 0;
+  d.apply_transform = t16 ? 1 : 0;
+  const float ident[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};
+  memcpy(d.t.m, t16 ? t16 : ident, sizeof(d.t.m));
+  const bool word4 = (ox & 3) == 0 && (oy & 3) == 0 && (oz & 3) == 0;
+  const bool one_word = (ox >> 4) == (oy >> 4) && (ox >> 4) == (oz >> 4);
+  d.aligned = (point_step % 16 == 0 && (reinterpret_cast<uintptr_t>(src) & 15u) == 0u && word4 && one_word) ? 1 : 0;
+  return d;
+}
+
+bool pc2_layout_ok(int point_step, int ox, int oy, int oz) {
+  return point_step >= 4 && ox >= 0 && oy >= 0 && oz >= 0 && ox <= point_step - 4 && oy <= point_step - 4 &&
+         oz <= point_step - 4;
 }
 
 // pcl::PointXYZ -> sensor_msgs/PointCloud2 payload (pcl::toROSMsg, od.cpp:290-294): the (16, 0, 4, 8) layout is the
@@ -981,12 +1047,49 @@ int run_wave_cluster(pcop_handle* h, int B, int max_n, bool with_generic) {
   return PCOP_OK;
 }
 
+// the messages of a pcop_process_batch_pointcloud2 call
+struct Pc2Call {
+  const pcop_pointcloud2_frame* frames;
+  const float* transform16;       // [batch][16] or nullptr
+  std::vector<char> on_device;    // per message: the payload is a device pointer (used in place)
+};
+
 struct WaveInput {
   const float* xyzw;
   size_t frame_stride_points;
   const int32_t* n;
   bool on_device;
+  const Pc2Call* pc2;  // non-null: the frames are PointCloud2 messages, decoded into d_in by the wave (xyzw unused)
 };
+
+size_t pc2_payload_bytes(const pcop_pointcloud2_frame& m) { return (size_t)m.n_points * (size_t)m.point_step; }
+
+// PointCloud2 wave, input half: the descriptors go up through the pinned staging (the lane's previous wave no longer
+// reads it), every host payload into the lane's raw staging at a 256-byte aligned offset, device payloads are read in
+// place; one k_pc2_ingest launch decodes (and transforms) every message into d_in.  A repeat of the wave (voxel
+// decline) decodes again from the same staging -- the plane stage has overwritten d_in, the staging is intact.
+int enqueue_wave_decode(pcop_handle* h, const Pc2Call& pc, int w0, int B, int max_n) {
+  if (h->vox_redo < 0) {
+    size_t off = 0;
+    for (int f = 0; f < B; ++f) {
+      const pcop_pointcloud2_frame& m = pc.frames[w0 + f];
+      const size_t bytes = pc2_payload_bytes(m);
+      const unsigned char* src = m.data;
+      if (bytes > 0 && !pc.on_device[w0 + f]) {
+        PCOP_CUDA_TRY(cudaMemcpyAsync(h->d_raw + off, m.data, bytes, cudaMemcpyHostToDevice, h->stream));
+        src = h->d_raw + off;
+        off += (bytes + 255) & ~(size_t)255;
+      }
+      h->h_pc2[f] = make_pc2_frame(src, m.n_points, m.point_step, m.off_x, m.off_y, m.off_z,
+                                   pc.transform16 ? pc.transform16 + (size_t)(w0 + f) * 16 : nullptr, m.is_dense);
+    }
+    PCOP_CUDA_TRY(cudaMemcpyAsync(h->d_pc2, h->h_pc2, sizeof(Pc2Frame) * B, cudaMemcpyHostToDevice, h->stream));
+  }
+  Ctx c = make_ctx(h, B, max_n);
+  KL(c, "k_pc2_ingest", k_pc2_ingest<<<dim3(cdiv(max_n, 256), B), 256, 0, h->stream>>>(h->d_pc2, h->d_in, (size_t)h->cap));
+  count_launch(c);
+  return PCOP_OK;
+}
 
 // Second half of a wave: clustering, result packing, and the copy of the wave's counts / plane records / pack sizes
 // into pinned memory, followed by ev_meta.
@@ -1114,11 +1217,17 @@ int enqueue_wave(pcop_handle* h, const WaveInput& wi, int w0, int B, uint32_t ma
   const float4* in;
   size_t stride;
   const int32_t* n = wi.n;
+  int max_n = 1;
+  for (int f = 0; f < B; ++f) max_n = std::max(max_n, (int)n[w0 + f]);
   {
     StageTimer t(h, PCOP_STAGE_H2D);
     memcpy(h->h_n_in, n + w0, sizeof(int) * B);  // (the lane's previous wave has been collected: the staging is free)
     PCOP_CUDA_TRY(cudaMemcpyAsync(h->cnt(CNT_IN), h->h_n_in, sizeof(int) * B, cudaMemcpyHostToDevice, h->stream));
-    if (wi.on_device) {
+    if (wi.pc2) {  // from the decode on, the wave is a host-input wave
+      TRY(enqueue_wave_decode(h, *wi.pc2, w0, B, max_n));
+      in = h->d_in;
+      stride = h->cap;
+    } else if (wi.on_device) {
       in = reinterpret_cast<const float4*>(wi.xyzw) + (size_t)w0 * wi.frame_stride_points;
       stride = wi.frame_stride_points;
     } else {
@@ -1138,8 +1247,6 @@ int enqueue_wave(pcop_handle* h, const WaveInput& wi, int w0, int B, uint32_t ma
       stride = h->cap;
     }
   }
-  int max_n = 1;
-  for (int f = 0; f < B; ++f) max_n = std::max(max_n, (int)n[w0 + f]);
   if (h->occ) TRY(enqueue_wave_counts(h, w0, B, in, stride, max_n));
   TRY(run_wave_stages(h, B, in, stride, max_n));
   h->pending = true;
@@ -1294,6 +1401,7 @@ int finish_wave(pcop_handle* h, const WaveInput& wi, uint32_t mask, pcop_frame_r
     // algorithmic bytes (SURVEY 8d)
     double b = 0.0;
     const pcop_params& p = h->params;
+    if (wi.pc2) b += (double)(wi.pc2->frames[w0 + f].point_step + 16) * r.n_input;  // the decode: payload in, PointXYZ out
     if (p.enable_crop) b += 16.0 * r.n_input + 20.0 * r.n_crop;
     if (p.enable_voxel) b += 16.0 * r.n_crop + 20.0 * r.n_voxel;
     if (p.enable_sor) b += 16.0 * r.n_voxel + 20.0 * r.n_sor;
@@ -1374,10 +1482,11 @@ int ensure_occ_scratch(pcop_handle* h, size_t frames, size_t cells) {
 }
 
 // occ: the grid product of every frame as well (pcop_process_batch_occupancy), nullptr: pcop_process_batch
+// pc2: the frames are PointCloud2 messages (pcop_process_batch_pointcloud2; xyzw unused, n = their record counts)
 int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, const int32_t* n, int32_t batch,
-                 pcop_frame_result* out, const pcop_handle::OccCall* occ = nullptr) {
+                 pcop_frame_result* out, const pcop_handle::OccCall* occ = nullptr, const Pc2Call* pc2 = nullptr) {
   if (!h) return fail(nullptr, PCOP_ERR_BAD_PARAM, "null handle");
-  if (!xyzw || !n || !out || batch < 0) return fail(h, PCOP_ERR_BAD_PARAM, "null argument");
+  if ((!xyzw && !pc2) || !n || !out || batch < 0) return fail(h, PCOP_ERR_BAD_PARAM, "null argument");
   PCOP_CUDA_TRY(cudaSetDevice(h->device));
   for (int f = 0; f < batch; ++f) {
     if (n[f] < 0) return fail(h, PCOP_ERR_BAD_PARAM, "negative point count");
@@ -1385,7 +1494,7 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
     if ((size_t)n[f] > frame_stride_points && batch > 1) return fail(h, PCOP_ERR_BAD_PARAM, "frame_stride_points < n");
   }
   const uint32_t mask = effective_outputs(h->params);
-  const WaveInput wi{xyzw, frame_stride_points, n, is_device_pointer(xyzw)};
+  const WaveInput wi{xyzw, frame_stride_points, n, pc2 ? false : is_device_pointer(xyzw), pc2};
   // lanes used by this call: per-kernel timing needs each kernel alone on the GPU, so it serialises the lanes
   std::vector<pcop_handle*> lanes(1, h);
   if (!h->kt.enabled)
@@ -1407,11 +1516,20 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
       w0 += B;
     }
   }
+  size_t raw_need = 0;  // PointCloud2 messages: host payload bytes of the largest wave, as staged (256-byte aligned)
+  if (pc2)
+    for (const auto& w : waves) {
+      size_t bytes = 0;
+      for (int f = w.first; f < w.first + w.second; ++f)
+        if (!pc2->on_device[f]) bytes += (pc2_payload_bytes(pc2->frames[f]) + 255) & ~(size_t)255;
+      raw_need = std::max(raw_need, bytes);
+    }
   h->occ = nullptr;  // (lanes the call does not use must not see a previous call's grid request)
   for (pcop_handle* l : h->extra_lanes) l->occ = nullptr;
   for (pcop_handle* l : lanes) {
     l->occ = occ;
     if (occ && !waves.empty()) TRY(ensure_occ_scratch(l, (size_t)waves[0].second, (size_t)occ->g.cells));  // (the first wave is the largest)
+    if (raw_need) TRY(ensure_raw(l, raw_need));
     l->params = h->params;
     l->vplan = h->vplan;
     l->vox_mode = h->vox_mode;
@@ -1715,6 +1833,8 @@ static int create_lane(const pcop_params* params, int device, size_t max_points,
   A(dalloc(h, &h->d_pack_off, (size_t)PK_N * B));
   A(dalloc(h, &h->d_meta, 1));
   A(dalloc(h, &h->d_pack_cursor, 1));
+  A(dalloc(h, &h->d_pc2, B));
+  A(halloc(h, &h->h_pc2, B));
   A(halloc(h, &h->h_n_active, 16));
   A(halloc(h, &h->h_counts, (size_t)CNT_ROWS * B));
   A(halloc(h, &h->h_warnings, B));
@@ -1862,6 +1982,22 @@ int pcop_process_batch(pcop_handle* h, const float* xyzw, size_t frame_stride_po
 
 static int occ_grid_of(pcop_handle* h, OccGrid* g);
 
+// the grid request of a batched call: the handle's grid (PCOP_ERR_CAPACITY above PCOP_OCC_BATCH_MAX_CELLS) + poses
+static int occ_call_of(pcop_handle* h, const char* who, const float* world_to_sensor16, const float* sensor_to_world16,
+                       int8_t* grids, pcop_handle::OccCall* oc) {
+  TRY(occ_grid_of(h, &oc->g));
+  if (oc->g.cells > PCOP_OCC_BATCH_MAX_CELLS)
+    return fail(h, PCOP_ERR_CAPACITY,
+                std::string(who) + ": grid of " + std::to_string(oc->g.W) + " x " + std::to_string(oc->g.H) +
+                    " cells exceeds PCOP_OCC_BATCH_MAX_CELLS (use pcop_occupancy_grid + pcop_occupancy_shadows)");
+  PCOP_CUDA_TRY(cudaSetDevice(h->device));
+  oc->world_to_sensor16 = world_to_sensor16;
+  oc->sensor_to_world16 = sensor_to_world16;
+  oc->grids = grids;
+  oc->grids_on_device = is_device_pointer(grids);
+  return PCOP_OK;
+}
+
 int pcop_process_batch_occupancy(pcop_handle* h, const float* xyzw, size_t frame_stride_points, const int32_t* n,
                                  int32_t batch, const float* world_to_sensor16, const float* sensor_to_world16,
                                  int8_t* grids, pcop_frame_result* out) {
@@ -1869,16 +2005,7 @@ int pcop_process_batch_occupancy(pcop_handle* h, const float* xyzw, size_t frame
   if (!world_to_sensor16 || !sensor_to_world16 || !grids || !out || batch < 0 || (!xyzw && batch != 1))
     return fail(h, PCOP_ERR_BAD_PARAM, "pcop_process_batch_occupancy: null argument (xyzw = NULL takes batch = 1)");
   pcop_handle::OccCall oc{};
-  TRY(occ_grid_of(h, &oc.g));
-  if (oc.g.cells > PCOP_OCC_BATCH_MAX_CELLS)
-    return fail(h, PCOP_ERR_CAPACITY,
-                "pcop_process_batch_occupancy: grid of " + std::to_string(oc.g.W) + " x " + std::to_string(oc.g.H) +
-                    " cells exceeds PCOP_OCC_BATCH_MAX_CELLS (use pcop_occupancy_grid + pcop_occupancy_shadows)");
-  PCOP_CUDA_TRY(cudaSetDevice(h->device));
-  oc.world_to_sensor16 = world_to_sensor16;
-  oc.sensor_to_world16 = sensor_to_world16;
-  oc.grids = grids;
-  oc.grids_on_device = is_device_pointer(grids);
+  TRY(occ_call_of(h, "pcop_process_batch_occupancy", world_to_sensor16, sensor_to_world16, grids, &oc));
   int st;
   if (!xyzw) {  // the accumulated cloud, consumed by this run (od.cpp:701), as pcop_process_accumulated
     const int32_t acc_n = h->acc_count;
@@ -1887,6 +2014,39 @@ int pcop_process_batch_occupancy(pcop_handle* h, const float* xyzw, size_t frame
   } else {
     st = process_impl(h, xyzw, frame_stride_points, n, batch, out, &oc);
   }
+  h->occ = nullptr;
+  for (pcop_handle* l : h->extra_lanes) l->occ = nullptr;
+  return st;
+}
+
+int pcop_process_batch_pointcloud2(pcop_handle* h, const pcop_pointcloud2_frame* frames, int32_t batch,
+                                   const float* transform16, const float* world_to_sensor16,
+                                   const float* sensor_to_world16, int8_t* grids, pcop_frame_result* out) {
+  if (!h) return fail(nullptr, PCOP_ERR_BAD_PARAM, "null handle");
+  if (!out || batch < 0 || (!frames && batch > 0) || (grids && (!world_to_sensor16 || !sensor_to_world16)))
+    return fail(h, PCOP_ERR_BAD_PARAM,
+                "pcop_process_batch_pointcloud2: null argument (grids need world_to_sensor16 and sensor_to_world16)");
+  Pc2Call pc;
+  pc.frames = frames;
+  pc.transform16 = transform16;
+  std::vector<int32_t> n((size_t)batch + 1, 0);
+  for (int f = 0; f < batch; ++f) {
+    const pcop_pointcloud2_frame& m = frames[f];
+    if (m.n_points < 0 || (!m.data && m.n_points > 0))
+      return fail(h, PCOP_ERR_BAD_PARAM, "pcop_process_batch_pointcloud2: frame " + std::to_string(f) + ": bad count or NULL data");
+    if (!pc2_layout_ok(m.point_step, m.off_x, m.off_y, m.off_z))
+      return fail(h, PCOP_ERR_BAD_PARAM,
+                  "pcop_process_batch_pointcloud2: frame " + std::to_string(f) + ": PointCloud2 field offsets do not fit point_step");
+    if (m.n_points > h->cap)
+      return fail(h, PCOP_ERR_CAPACITY, "pcop_process_batch_pointcloud2: frame " + std::to_string(f) + " has more points than max_points");
+    n[f] = m.n_points;
+  }
+  pcop_handle::OccCall oc{};
+  if (grids) TRY(occ_call_of(h, "pcop_process_batch_pointcloud2", world_to_sensor16, sensor_to_world16, grids, &oc));
+  PCOP_CUDA_TRY(cudaSetDevice(h->device));
+  pc.on_device.resize((size_t)batch);
+  for (int f = 0; f < batch; ++f) pc.on_device[f] = frames[f].n_points > 0 && is_device_pointer(frames[f].data);
+  const int st = process_impl(h, nullptr, (size_t)h->cap, n.data(), batch, out, grids ? &oc : nullptr, &pc);
   h->occ = nullptr;
   for (pcop_handle* l : h->extra_lanes) l->occ = nullptr;
   return st;
@@ -1994,27 +2154,19 @@ int pcop_transform(pcop_handle* h, const float* xyzw, int32_t n, const float* tr
 
 static int pc2_ingest(pcop_handle* h, const unsigned char* data, int32_t n, int32_t point_step, int32_t ox, int32_t oy,
                       int32_t oz, const float* t16, int is_dense, float4* dst) {
-  if (point_step < 4 || ox < 0 || oy < 0 || oz < 0 || ox + 4 > point_step || oy + 4 > point_step || oz + 4 > point_step)
-    return fail(h, PCOP_ERR_BAD_PARAM, "PointCloud2 field offsets do not fit point_step");
+  if (!pc2_layout_ok(point_step, ox, oy, oz)) return fail(h, PCOP_ERR_BAD_PARAM, "PointCloud2 field offsets do not fit point_step");
   const size_t bytes = (size_t)n * (size_t)point_step;
   const unsigned char* src = data;
   if (!is_device_pointer(data)) {
-    if (bytes > h->raw_cap) {
-      PCOP_CUDA_TRY(cudaStreamSynchronize(h->stream));
-      if (h->d_raw) cudaFree(h->d_raw);
-      h->d_raw = nullptr;
-      h->raw_cap = 0;
-      PCOP_CUDA_TRY(cudaMalloc((void**)&h->d_raw, bytes + bytes / 4 + 256));
-      h->raw_cap = bytes + bytes / 4 + 256;
-    }
+    TRY(ensure_raw(h, bytes));
     PCOP_CUDA_TRY(cudaMemcpyAsync(h->d_raw, data, bytes, cudaMemcpyHostToDevice, h->stream));
     src = h->d_raw;
   }
-  Mat34 t;
-  const float ident[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};
-  memcpy(t.m, t16 ? t16 : ident, sizeof(t.m));
+  // the batched decode with one frame; the descriptor goes up from pageable memory (staged before the call returns)
+  const Pc2Frame d = make_pc2_frame(src, n, point_step, ox, oy, oz, t16, is_dense);
+  PCOP_CUDA_TRY(cudaMemcpyAsync(h->d_pc2, &d, sizeof(d), cudaMemcpyHostToDevice, h->stream));
   Ctx c = make_ctx(h, 1, n);
-  KL(c, "k_pc2_ingest", k_pc2_ingest<<<cdiv(n, 256), 256, 0, h->stream>>>(src, n, point_step, ox, oy, oz, t, t16 ? 1 : 0, is_dense, dst));
+  KL(c, "k_pc2_ingest", k_pc2_ingest<<<dim3(cdiv(n, 256), 1), 256, 0, h->stream>>>(h->d_pc2, dst, (size_t)0));
   count_launch(c);
   if (src != data) PCOP_CUDA_TRY(cudaStreamSynchronize(h->stream));  // the caller may reuse its buffer
   return PCOP_OK;
@@ -2062,14 +2214,7 @@ int pcop_cloud_to_pointcloud2(pcop_handle* h, const float* xyzw, int32_t n, int3
   unsigned char* dst = out_data;
   const bool out_on_device = is_device_pointer(out_data);
   if (!out_on_device) {  // staged through the raw-payload buffer of the ingest path
-    if (bytes > h->raw_cap) {
-      PCOP_CUDA_TRY(cudaStreamSynchronize(h->stream));
-      if (h->d_raw) cudaFree(h->d_raw);
-      h->d_raw = nullptr;
-      h->raw_cap = 0;
-      PCOP_CUDA_TRY(cudaMalloc((void**)&h->d_raw, bytes + bytes / 4 + 256));
-      h->raw_cap = bytes + bytes / 4 + 256;
-    }
+    TRY(ensure_raw(h, bytes));
     dst = h->d_raw;
   }
   Ctx c = make_ctx(h, 1, n);
