@@ -8,7 +8,7 @@
 //                  per frame, 16-bit shared-memory counters), min/max of the survivors, the NaN-y/z flag;
 //   k_vp_scan      per frame: bucket starts (exclusive scan), per-chunk offsets inside each bucket, M, and the work
 //                  list of the reduce kernel: consecutive non-empty buckets are grouped greedily up to 2048 elements
-//                  or the bitmap's range (131072 keys);
+//                  or the bitmap's range (262144 keys);
 //   k_vp_scatter   second read of the input: every survivor goes to a slot of its (chunk, bucket) range -- slot taken
 //                  with a shared-memory atomic -- as {x, y, z, original index};
 //   k_vp_reduce    one block per group (<= 2048 elements), everything in shared memory: a bitmap over the group's key
@@ -34,7 +34,9 @@
 
 namespace pcop {
 #ifdef PCOP_VP_DEBUG_CLK
-__device__ long long g_vp_reduce_clk[16];  // phase timestamps of one block (tools/vp_phases.py)
+// phase timestamps of one block in [0, 10); [12, 16): groups, groups on the binary search, groups of more than 64
+// buckets, elements, summed over the blocks since the last read (tools/vp_phases.py)
+__device__ long long g_vp_reduce_clk[16];
 #define VP_CLK(k)                                                                          \
   do {                                                                                     \
     if (blockIdx.x == 5 && blockIdx.y == 20 && threadIdx.x == 0) g_vp_reduce_clk[k] = clock64(); \
@@ -55,7 +57,7 @@ constexpr int VP_EMAX = 2048;           // elements per group (and per bucket)
 constexpr int VPR_THREADS = 512;        // reduce kernel: 16 warps per group, 4 elements per thread, all kept in registers
 constexpr int VPR_WARPS = VPR_THREADS / 32;
 constexpr int VP_EPT = VP_EMAX / VPR_THREADS;
-constexpr int VP_BITMAP_WORDS = 4096;   // 131072 keys per group
+constexpr int VP_BITMAP_WORDS = 8192;   // 262144 keys per group (128 buckets at S = 11)
 constexpr int VP_KMAX = 256;            // buckets per group (<= VP_BITMAP_WORDS * 32 >> S)
 constexpr int VP_SCAN_THREADS = 512;
 constexpr int VP_SCAN_WARPS = VP_SCAN_THREADS / 32;
@@ -426,23 +428,29 @@ __global__ void __launch_bounds__(VPS_THREADS)
   }
 }
 
-constexpr int VP_ORD_TAB = 1024;  // span of bucket ids a group may cover for the direct bucket -> ordinal table
+constexpr int VP_ORD_TAB = 4096;  // span of bucket ids a group may cover for the direct bucket -> ordinal table
 
 struct alignas(16) VpReduceSmem {
-  uint32_t bitmap[VP_BITMAP_WORDS];         // one bit per key of the group's range
-  unsigned short wprefix[VP_BITMAP_WORDS];  // voxels before each bitmap word, inside its round of 128 words
-  uint32_t rbase[VP_BITMAP_WORDS / 128 + 4];  // voxels before each round of 128 bitmap words (sized to keep `start` 16-byte aligned)
+  union {
+    struct {                                    // setup .. pass 2
+      uint32_t bitmap[VP_BITMAP_WORDS];         // one bit per key of the group's range
+      unsigned short wprefix[VP_BITMAP_WORDS];  // voxels before each bitmap word, inside its round of 128 words
+    } k;
+    struct {                                    // pass 3 .. sums (first written after the last read of `k`)
+      int sidx[VP_EMAX];                        // original indices, grouped by voxel (any order inside a run)
+      float sx[VP_EMAX], sy[VP_EMAX], sz[VP_EMAX];  // coordinates, grouped by voxel, ascending original index inside a run
+    } e;
+  };
+  uint32_t rtot[VP_BITMAP_WORDS / 128];     // voxels in each round of 128 bitmap words
   uint32_t start[VP_EMAX + 4];              // per voxel: point count, then first position of its run
-  uint32_t srt[VP_EMAX / 128 + 1];          // scratch of the run-length scan
-  int sidx[VP_EMAX];                        // original indices, grouped by voxel (any order inside a run)
-  float sx[VP_EMAX], sy[VP_EMAX], sz[VP_EMAX];  // coordinates, grouped by voxel, ascending original index inside a run
-  uint32_t bkt_start[VP_KMAX + 1];          // element start of the group's buckets
-  unsigned short bkt_id[VP_KMAX];
+  uint32_t srt[VP_EMAX / 128];              // run lengths in each round of 128 voxels
+  uint32_t bkt_start[VP_KMAX + 1];          // element start of the group's buckets (binary-search groups only)
   unsigned char ord_tab[VP_ORD_TAB];        // bucket id - first bucket id -> ordinal inside the group
-  unsigned vbase, nvox;
+  unsigned vbase;
 };
 
-static_assert(offsetof(VpReduceSmem, start) % 16 == 0 && offsetof(VpReduceSmem, wprefix) % 8 == 0, "vector accesses");
+static_assert(offsetof(VpReduceSmem, start) % 16 == 0 && offsetof(VpReduceSmem, k.wprefix) % 8 == 0, "vector accesses");
+static_assert(VP_BITMAP_WORDS / 128 <= 64 && VP_EMAX / 128 <= VPR_WARPS, "the block scans: two rounds per lane, one per warp");
 
 // exclusive scan of four consecutive values per lane over a round of 128 values: returns the lane's exclusive prefix
 // inside the round (of its first value) and the round's total (all lanes)
@@ -487,19 +495,26 @@ __global__ void __launch_bounds__(VPR_THREADS, 3)
   const int S = pl.part_shift;
   const int wpb = (1 << S) >> 5;  // bitmap words per bucket (S >= 5)
   const int nwords = KB * wpb;    // <= VP_BITMAP_WORDS
-  int my_bucket = 0;
-  if (tid < KB) {
-    my_bucket = ne_bucket[(size_t)f * VP_NB_MAX + o0 + tid];
-    sm.bkt_id[tid] = (unsigned short)my_bucket;
+  // every thread reads the group's first and last bucket ids itself: the table is filled without a barrier in front
+  const unsigned short* nb = ne_bucket + (size_t)f * VP_NB_MAX + o0;
+  const int b_first = nb[0];
+  const bool direct = (int)nb[KB - 1] - b_first < VP_ORD_TAB;  // (else: binary search on the bucket starts)
+  if (direct) {
+    if (tid < KB) sm.ord_tab[nb[tid] - b_first] = (unsigned char)tid;
+  } else if (tid <= KB) {
+    sm.bkt_start[tid] = ne_start[(size_t)f * (VP_NB_MAX + 1) + o0 + tid];  // (entry NE holds M)
   }
-  if (tid <= KB) sm.bkt_start[tid] = ne_start[(size_t)f * (VP_NB_MAX + 1) + o0 + tid];  // (entry NE holds M)
   for (int w = 4 * tid; w < nwords; w += 4 * VPR_THREADS)  // (whole uint4s: the scans read them as such)
-    *reinterpret_cast<uint4*>(&sm.bitmap[w]) = make_uint4(0u, 0u, 0u, 0u);
+    *reinterpret_cast<uint4*>(&sm.k.bitmap[w]) = make_uint4(0u, 0u, 0u, 0u);
   for (int v = 4 * tid; v < E + 4; v += 4 * VPR_THREADS) *reinterpret_cast<uint4*>(&sm.start[v]) = make_uint4(0u, 0u, 0u, 0u);
-  __syncthreads();
-  const int b_first = sm.bkt_id[0];
-  const bool direct = (int)sm.bkt_id[KB - 1] - b_first < VP_ORD_TAB;  // (else: binary search on the bucket starts)
-  if (direct && tid < KB) sm.ord_tab[my_bucket - b_first] = (unsigned char)tid;
+#ifdef PCOP_VP_DEBUG_CLK
+  if (tid == 0) {
+    atomicAdd(reinterpret_cast<unsigned long long*>(&g_vp_reduce_clk[12]), 1ull);
+    atomicAdd(reinterpret_cast<unsigned long long*>(&g_vp_reduce_clk[13]), direct ? 0ull : 1ull);
+    atomicAdd(reinterpret_cast<unsigned long long*>(&g_vp_reduce_clk[14]), KB > 64 ? 1ull : 0ull);
+    atomicAdd(reinterpret_cast<unsigned long long*>(&g_vp_reduce_clk[15]), (unsigned long long)E);
+  }
+#endif
   __syncthreads();
   VP_CLK(1);
 
@@ -526,57 +541,63 @@ __global__ void __launch_bounds__(VPR_THREADS, 3)
       }
       const uint32_t s = ((uint32_t)ord << S) | (key & ((1u << S) - 1u));
       slot[k] = s;
-      atomicOr(&sm.bitmap[s >> 5], 1u << (s & 31u));
+      atomicOr(&sm.k.bitmap[s >> 5], 1u << (s & 31u));
     }
   }
   __syncthreads();
   VP_CLK(2);
   // ---- voxel ranks: exclusive popcount prefix over the bitmap words; a warp takes a round of 128 words, four consecutive
   // words per lane (one 16-byte load) ----------------------------------------------------------------------------------------
-  const int nr = cdiv(nwords, 128);
+  const int nr = cdiv(nwords, 128);  // <= 64
   for (int r = warp; r < nr; r += VPR_WARPS) {
     const int w = 128 * r + 4 * lane;
-    const uint4 bw = (w < nwords) ? *reinterpret_cast<const uint4*>(&sm.bitmap[w]) : make_uint4(0u, 0u, 0u, 0u);  // (nwords % 4 == 0)
+    const uint4 bw = (w < nwords) ? *reinterpret_cast<const uint4*>(&sm.k.bitmap[w]) : make_uint4(0u, 0u, 0u, 0u);  // (nwords % 4 == 0)
     const unsigned c[4] = {(unsigned)__popc(bw.x), (unsigned)__popc(bw.y), (unsigned)__popc(bw.z), (unsigned)__popc(bw.w)};
     unsigned total;
     const unsigned ex = vp_round_scan(c, total);
     if (w < nwords) {
       const unsigned a0 = ex, a1 = a0 + c[0], a2 = a1 + c[1], a3 = a2 + c[2];
-      *reinterpret_cast<uint2*>(&sm.wprefix[w]) = make_uint2(a0 | (a1 << 16), a2 | (a3 << 16));
+      *reinterpret_cast<uint2*>(&sm.k.wprefix[w]) = make_uint2(a0 | (a1 << 16), a2 | (a3 << 16));
     }
-    if (lane == 0) sm.rbase[r] = total;
+    if (lane == 0) sm.rtot[r] = total;
   }
   __syncthreads();
-  if (warp == 0) {
-    const unsigned v = warp0_excl_scan<1>(sm.rbase, nr);  // (<= 32 rounds)
-    if (lane == 0) sm.nvox = v;
+  VP_CLK(3);
+  // every warp scans the round totals itself (rounds 2 * lane and 2 * lane + 1 in lane `lane`) and keeps the voxels
+  // before both rounds in one register (<= 2048 each); pass 2 takes a round's base from its lane by shuffle
+  unsigned rbase2;
+  int V;
+  {
+    const unsigned t0 = (2 * lane < nr) ? sm.rtot[2 * lane] : 0u, t1 = (2 * lane + 1 < nr) ? sm.rtot[2 * lane + 1] : 0u;
+    const unsigned incl = warp_incl_scan(t0 + t1);
+    const unsigned b0 = incl - t0 - t1;
+    rbase2 = b0 | ((b0 + t0) << 16);
+    V = (int)__shfl_sync(FULL, incl, 31);
   }
-  __syncthreads();
-  const int V = (int)sm.nvox;
   unsigned* dd = desc + (size_t)f * gstride;
   if (tid == 0) st_volatile_u32(dd + g, ((g == 0) ? LB_PREFIX : LB_AGG) | (unsigned)V);  // early publish
-  VP_CLK(3);
   // ---- pass 2: a place for every element inside its voxel's run (any order), run lengths -------------------------------
 #pragma unroll
   for (int k = 0; k < VP_EPT; ++k) {
     const int e = tid + k * VPR_THREADS;
+    const uint32_t s = slot[k];
+    const uint32_t rb = __shfl_sync(FULL, rbase2, (int)(s >> 13)) >> ((s >> 8) & 16u);  // round s >> 12
     if (e < E) {
-      const uint32_t s = slot[k];
-      const uint32_t r = sm.rbase[s >> 12] + (uint32_t)sm.wprefix[s >> 5] +
-                         (uint32_t)__popc(sm.bitmap[s >> 5] & ((1u << (s & 31u)) - 1u));
+      const uint32_t r = (rb & 0xffffu) + (uint32_t)sm.k.wprefix[s >> 5] +
+                         (uint32_t)__popc(sm.k.bitmap[s >> 5] & ((1u << (s & 31u)) - 1u));
       const uint32_t j = atomicAdd(&sm.start[r], 1u);
       slot[k] = (r << 16) | j;
     }
   }
   __syncthreads();
   VP_CLK(4);
-  {  // exclusive scan of the run lengths, in place: rounds of 128 voxels, four consecutive voxels per lane
+  {  // exclusive scan of the run lengths, in place: warp r takes the round of voxels 128 r .. 128 r + 127 (V <= 2048),
+     // four consecutive voxels per lane
     const int vr = cdiv(V, 128);
     unsigned keep[4] = {0u, 0u, 0u, 0u};
-    int my_r = -1;
-    for (int r = warp; r < vr; r += VPR_WARPS) {  // (at most one round per warp: V <= 2048 = 16 rounds)
-      const int v = 128 * r + 4 * lane;
-      const uint4 cw = *reinterpret_cast<const uint4*>(&sm.start[v]);  // (entries past V are zero)
+    if (warp < vr) {
+      const int v = 128 * warp + 4 * lane;
+      const uint4 cw = *reinterpret_cast<const uint4*>(&sm.start[v]);  // (counts past E + 3 are stale: they only reach entries past V)
       const unsigned c[4] = {cw.x, cw.y, cw.z, cw.w};
       unsigned total;
       const unsigned ex = vp_round_scan(c, total);
@@ -584,31 +605,56 @@ __global__ void __launch_bounds__(VPR_THREADS, 3)
       keep[1] = ex + c[0];
       keep[2] = keep[1] + c[1];
       keep[3] = keep[2] + c[2];
-      my_r = r;
-      if (lane == 0) sm.srt[r] = total;
+      if (lane == 0) sm.srt[warp] = total;
+    }
+    // voxels of the earlier groups of this frame (decoupled look-back; the aggregates were published after the popcount,
+    // the wait is on lower group ids only).  The last warp has no round unless V > 1920, so the L2 round trip hides
+    // behind the run-length scan; `vbase` is read after the barriers below.
+    if (warp == VPR_WARPS - 1 && g > 0) {
+      unsigned excl = 0u;
+      int look = g - 1;
+      while (true) {
+        const int idx = look - lane;
+        unsigned d = LB_PREFIX;  // lanes past the first group read as "prefix 0"
+        if (idx >= 0) {
+          d = lookback_wait(dd + idx);
+        }
+        const unsigned is_prefix = __ballot_sync(FULL, (d >> 30) == 2u);
+        const int first = is_prefix ? (__ffs(is_prefix) - 1) : 31;
+        unsigned v = (lane <= first) ? (d & LB_VALUE) : 0u;
+        v = __reduce_add_sync(FULL, v);
+        excl += v;
+        if (is_prefix) break;
+        look -= 32;
+      }
+      if (lane == 0) {
+        st_volatile_u32(dd + g, LB_PREFIX | (excl + (unsigned)V));
+        sm.vbase = excl;
+      }
+    } else if (tid == 0 && g == 0) {
+      sm.vbase = 0u;
     }
     __syncthreads();
-    if (warp == 0) warp0_excl_scan<1>(sm.srt, vr);
-    __syncthreads();
-    if (my_r >= 0) {
-      const unsigned base = sm.srt[my_r];
-      const int v = 128 * my_r + 4 * lane;
+    VP_CLK(5);
+    if (warp < vr) {
+      const unsigned base = __reduce_add_sync(FULL, (lane < warp) ? sm.srt[lane] : 0u);
+      const int v = 128 * warp + 4 * lane;
       *reinterpret_cast<uint4*>(&sm.start[v]) = make_uint4(base + keep[0], base + keep[1], base + keep[2], base + keep[3]);
     }
-    __syncthreads();
-    if (tid == 0) sm.start[V] = (unsigned)E;  // (V may be the first entry of a round that no warp took)
+    // (entry V is E: written above when a round holds it, the counts at V .. V + 3 being zero; here when none does)
+    if (tid == 0 && (V & 127) == 0) sm.start[V] = (unsigned)E;
   }
   __syncthreads();
-  VP_CLK(5);
+  VP_CLK(6);
   // ---- pass 3: original indices grouped by voxel; then every element counts the smaller indices of its run and puts its
   // coordinates at that place (runs are ~2 points; a dense blob costs its run length per element) -----------------------
 #pragma unroll
   for (int k = 0; k < VP_EPT; ++k) {
     const int e = tid + k * VPR_THREADS;
-    if (e < E) sm.sidx[sm.start[slot[k] >> 16] + (slot[k] & 0xffffu)] = __float_as_int(p[k].w);
+    if (e < E) sm.e.sidx[sm.start[slot[k] >> 16] + (slot[k] & 0xffffu)] = __float_as_int(p[k].w);
   }
   __syncthreads();
-  VP_CLK(6);
+  VP_CLK(7);
 #pragma unroll
   for (int k = 0; k < VP_EPT; ++k) {
     const int e = tid + k * VPR_THREADS;
@@ -620,16 +666,16 @@ __global__ void __launch_bounds__(VPR_THREADS, 3)
       if (cnt > 2) {
         const int mine = __float_as_int(p[k].w);
         rank = 0;
-        for (int t = 0; t < cnt; ++t) rank += (sm.sidx[s0 + t] < mine) ? 1 : 0;
+        for (int t = 0; t < cnt; ++t) rank += (sm.e.sidx[s0 + t] < mine) ? 1 : 0;
       }
-      sm.sx[s0 + rank] = p[k].x;
-      sm.sy[s0 + rank] = p[k].y;
-      sm.sz[s0 + rank] = p[k].z;
+      sm.e.sx[s0 + rank] = p[k].x;
+      sm.e.sy[s0 + rank] = p[k].y;
+      sm.e.sz[s0 + rank] = p[k].z;
     }
   }
   __syncthreads();
-  VP_CLK(7);
-  // ---- one thread per voxel: sequential sum of its run, centroid (kept in registers while warp 0 resolves the look-back) --
+  VP_CLK(8);
+  // ---- one thread per voxel: sequential sum of its run, centroid, stored at (voxels of the earlier groups) + rank -----
   VoxelFrame vfr;
   float fb0 = 0.f, fb1 = 0.f, fb2 = 0.f;
   if (WITH_KEYS) {
@@ -638,69 +684,30 @@ __global__ void __launch_bounds__(VPR_THREADS, 3)
     fb1 = (float)vfr.min_b[1];
     fb2 = (float)vfr.min_b[2];
   }
+  const unsigned vbase = sm.vbase;
+  if (g == ng - 1 && tid == 0) n_out[f] = (int)(vbase + (unsigned)V);
   constexpr int VPT = VP_EMAX / VPR_THREADS;  // voxels per thread
-  float4 cen[VPT];
-  uint32_t vkey[VPT];
 #pragma unroll
   for (int k = 0; k < VPT; ++k) {
     const int v = tid + k * VPR_THREADS;
-    cen[k] = make_float4(0.f, 0.f, 0.f, 1.0f);
-    vkey[k] = 0u;
     if (v < V) {
       const int s0 = (int)sm.start[v], s1 = (int)sm.start[v + 1];
       float ax = 0.0f, ay = 0.0f, az = 0.0f;
       for (int t = s0; t < s1; ++t) {
-        ax = fadd(ax, sm.sx[t]);
-        ay = fadd(ay, sm.sy[t]);
-        az = fadd(az, sm.sz[t]);
+        ax = fadd(ax, sm.e.sx[t]);
+        ay = fadd(ay, sm.e.sy[t]);
+        az = fadd(az, sm.e.sz[t]);
       }
       const float c = (float)(s1 - s0);
-      // (x / 1.0f == x exactly: the single-point voxels, more than half of them, skip the three divisions)
-      cen[k] = (s1 - s0 == 1) ? make_float4(ax, ay, az, 1.0f) : make_float4(fdiv(ax, c), fdiv(ay, c), fdiv(az, c), 1.0f);
-      if (WITH_KEYS) {  // PCL's key of this voxel, from one of its points (voxel_grid.hpp: ijk = floor(p*inv) - min_b)
-        const int i0 = cvt_f2i(fsub(floorf(fmul(sm.sx[s0], vfr.inv)), fb0));
-        const int i1 = cvt_f2i(fsub(floorf(fmul(sm.sy[s0], vfr.inv)), fb1));
-        const int i2 = cvt_f2i(fsub(floorf(fmul(sm.sz[s0], vfr.inv)), fb2));
-        vkey[k] = (uint32_t)i0 + (uint32_t)i1 * vfr.mul1 + (uint32_t)i2 * vfr.mul2;
-      }
-    }
-  }
-  // voxels of the earlier groups of this frame (decoupled look-back; the aggregate was published above)
-  if (warp == 0 && g > 0) {
-    unsigned excl = 0u;
-    int look = g - 1;
-    while (true) {
-      const int idx = look - lane;
-      unsigned d = LB_PREFIX;  // lanes past the first group read as "prefix 0"
-      if (idx >= 0) {
-        d = lookback_wait(dd + idx);
-      }
-      const unsigned is_prefix = __ballot_sync(FULL, (d >> 30) == 2u);
-      const int first = is_prefix ? (__ffs(is_prefix) - 1) : 31;
-      unsigned v = (lane <= first) ? (d & LB_VALUE) : 0u;
-      v = __reduce_add_sync(FULL, v);
-      excl += v;
-      if (is_prefix) break;
-      look -= 32;
-    }
-    if (lane == 0) {
-      st_volatile_u32(dd + g, LB_PREFIX | (excl + (unsigned)V));
-      sm.vbase = excl;
-    }
-  } else if (tid == 0 && g == 0) {
-    sm.vbase = 0u;
-  }
-  __syncthreads();
-  VP_CLK(8);
-  const unsigned vbase = sm.vbase;
-  if (g == ng - 1 && tid == 0) n_out[f] = (int)(vbase + (unsigned)V);
-#pragma unroll
-  for (int k = 0; k < VPT; ++k) {
-    const int v = tid + k * VPR_THREADS;
-    if (v < V) {
       const size_t o = (size_t)f * cap + vbase + (unsigned)v;
-      out[o] = cen[k];
-      if (WITH_KEYS) out_keys[o] = vkey[k];
+      // (x / 1.0f == x exactly: the single-point voxels, more than half of them, skip the three divisions)
+      out[o] = (s1 - s0 == 1) ? make_float4(ax, ay, az, 1.0f) : make_float4(fdiv(ax, c), fdiv(ay, c), fdiv(az, c), 1.0f);
+      if (WITH_KEYS) {  // PCL's key of this voxel, from one of its points (voxel_grid.hpp: ijk = floor(p*inv) - min_b)
+        const int i0 = cvt_f2i(fsub(floorf(fmul(sm.e.sx[s0], vfr.inv)), fb0));
+        const int i1 = cvt_f2i(fsub(floorf(fmul(sm.e.sy[s0], vfr.inv)), fb1));
+        const int i2 = cvt_f2i(fsub(floorf(fmul(sm.e.sz[s0], vfr.inv)), fb2));
+        out_keys[o] = (uint32_t)i0 + (uint32_t)i1 * vfr.mul1 + (uint32_t)i2 * vfr.mul2;
+      }
     }
   }
   VP_CLK(9);
@@ -787,6 +794,9 @@ void run_voxel_part(const Ctx& c, const VoxelPartArgs& a) {
 
 #ifdef PCOP_VP_DEBUG_CLK
 extern "C" int pcop_debug_vp_reduce_cycles(long long* out16) {
-  return (int)cudaMemcpyFromSymbol(out16, pcop::g_vp_reduce_clk, sizeof(long long) * 16);
+  cudaError_t e = cudaMemcpyFromSymbol(out16, pcop::g_vp_reduce_clk, sizeof(long long) * 16);
+  static const long long zero[4] = {0, 0, 0, 0};
+  if (e == cudaSuccess) e = cudaMemcpyToSymbol(pcop::g_vp_reduce_clk, zero, sizeof(zero), sizeof(long long) * 12);
+  return (int)e;
 }
 #endif
