@@ -14,7 +14,7 @@ LIB = os.path.join(HERE, "libpcop.so")
 SYNTH_SRC = os.path.join(HERE, "synth", "synth.cpp")
 SYNTH_LIB = os.path.join(HERE, "synth", "libpcop_synth.so")
 
-CU_SOURCES = ["pcop_api.cu", "radix_sort.cu", "stage_crop.cu", "stage_voxel.cu", "stage_voxel_fused.cu", "stage_voxel_part.cu", "stage_sor.cu", "stage_plane.cu",
+CU_SOURCES = ["pcop_api.cu", "batch.cu", "radix_sort.cu", "stage_crop.cu", "stage_voxel.cu", "stage_voxel_fused.cu", "stage_voxel_part.cu", "stage_sor.cu", "stage_plane.cu",
               "stage_cluster.cu", "stage_cluster_small.cu", "stage_occupancy.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -13,7 +13,7 @@ pytestmark = pytest.mark.gpu
 @pytest.fixture(params=["fused", "generic"])
 def ece_path(request, monkeypatch):
     """Euclidean clustering has two device paths: the fused shared-memory kernel for small clouds and the generic
-    multi-kernel path.  PCOP_ECE_SMALL_MAX=0 forces the generic one (read by the library at every call)."""
+    multi-kernel path.  PCOP_ECE_SMALL_MAX=0 forces the generic one (read when the handle is created)."""
     if request.param == "generic":
         monkeypatch.setenv("PCOP_ECE_SMALL_MAX", "0")
     else:
