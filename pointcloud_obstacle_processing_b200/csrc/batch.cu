@@ -269,22 +269,37 @@ int ensure_host_pack(Lane* l, size_t need) {
   return PCOP_OK;
 }
 
-// The plane loop of one wave on the stage input recorded in the lane.  large_tier: see run_plane.
-int run_wave_plane(Lane* l, int B, int max_n, bool large_tier) {
+// The first route of a wave whose largest frame has max_n points, from the handle's plan and knobs and the lane's
+// history: the LSD voxel path while a partition-path decline is recent, a reduce grid sized by the frames seen lately,
+// and the plane tiers and clustering kernels the last waves needed.
+WaveRoute next_route(const Lane* l, int max_n) {
+  const pcop_handle* h = l->h;
+  WaveRoute r;
+  if (h->vplan.part_ok && l->vox_lsd_waves <= 0) {
+    r.vox = WaveRoute::VOX_PARTITION;
+    r.vox_groups = std::min(l->vp_group_hint, vox_part_group_bound(h->vplan, max_n));
+  } else if (h->vplan.ok) {
+    r.vox = WaveRoute::VOX_LSD;
+  }
+  if (!h->plane_resident || l->plane_hostloop_waves > 0) r.plane = WaveRoute::PLANE_HOSTLOOP;
+  else if (l->expect_large_plane) r.plane = WaveRoute::PLANE_RESIDENT;
+  r.cluster_generic = l->expect_big_remaining || h->ece_small_max <= 0;  // (no fused kernel at all: run_cluster)
+  return r;
+}
+
+// The plane loop of one wave on the stage input recorded in the lane.  Tiers: see run_plane.
+int run_wave_plane(Lane* l, int B, int max_n, const WaveRoute& r) {
   const pcop_params& p = l->h->params;
   Ctx c = make_ctx(l, B, max_n);  // (no frame holds more points than the largest input frame)
   StageTimer t(l, PCOP_STAGE_PLANE);
-  l->wave_plane_speculated = false;
   if (p.enable_plane) {
     PlaneArgs a = make_plane_args(l, l->plane_in, l->plane_stride, l->plane_n);
     a.n_in_copy = p.enable_sor ? nullptr : l->cnt(CNT_SOR);
-    a.large_tier = large_tier ? 1 : 0;
-    if (l->plane_hostloop_waves > 0) a.resident = 0;
-    l->wave_plane_resident = a.resident != 0;
+    a.resident = r.plane != WaveRoute::PLANE_HOSTLOOP;
+    a.large_tier = r.plane == WaveRoute::PLANE_RESIDENT;
     if (!(effective_outputs(p) & PCOP_OUT_PLANE)) a.inlier_idx = nullptr;  // the inlier list is only written on request
     cudaError_t e = run_plane(c, a);
     if (e != cudaSuccess) return fail_cuda(l->h, e, "run_plane", __FILE__, __LINE__);
-    l->wave_plane_speculated = a.resident && !large_tier && max_n > plane_small_tier_max();
   } else {
     KL(c, "k_copy_counts", k_copy_counts<<<cdiv(B, 256), 256, 0, l->stream>>>(l->plane_n, l->cnt(CNT_REM), B));
     KL(c, "k_copy_cloud", k_copy_cloud<<<dim3(cdiv(c.grid_cap, CT_TILE), B), CT_THREADS, 0, l->stream>>>(
@@ -295,13 +310,11 @@ int run_wave_plane(Lane* l, int B, int max_n, bool large_tier) {
 }
 
 // All stages of one wave up to the plane loop.  `in`/`stride` already on the device; counts row CNT_IN already set.
-int run_wave_stages(Lane* l, int B, const float4* in, size_t stride, int max_n) {
+int run_wave_stages(Lane* l, int B, const float4* in, size_t stride, int max_n, const WaveRoute& r) {
   pcop_handle* h = l->h;
   const pcop_params& p = h->params;
   Ctx c = make_ctx(l, B, max_n);  // no stage ever holds more points per frame than the largest input frame
-  const int vmode = (l->vox_redo >= 0) ? l->vox_redo : ((h->vox_mode == 2 && l->vox_lsd_waves > 0) ? 1 : h->vox_mode);
-  const bool fused_path = vmode != 0;
-  if (!fused_path || (effective_outputs(p) & PCOP_OUT_CROP)) {  // (the fused voxel path zeroes the warnings itself)
+  if (r.vox == WaveRoute::VOX_GENERIC || (effective_outputs(p) & PCOP_OUT_CROP)) {  // (the fused voxel path zeroes the warnings itself)
     KL(c, "k_zero_u32", k_zero_u32<<<cdiv(B, 256), 256, 0, l->stream>>>(l->d_warnings, B));
     count_launch(c);
   }
@@ -311,9 +324,7 @@ int run_wave_stages(Lane* l, int B, const float4* in, size_t stride, int max_n) 
   const int* cur_n = l->cnt(CNT_IN);
   bool have_minmax = false;
 
-  const bool fused = fused_path;
-  l->wave_used_fused = fused;
-  if (fused && vmode == 2) {
+  if (r.vox == WaveRoute::VOX_PARTITION) {
     {
       StageTimer t(l, PCOP_STAGE_CROP);
       if (effective_outputs(p) & PCOP_OUT_CROP) run_crop(c, make_crop_args(l, cur, cur_stride, cur_n));
@@ -336,7 +347,7 @@ int run_wave_stages(Lane* l, int B, const float4* in, size_t stride, int max_n) 
     a.part = l->d_sorted;  // (the search-grid point list of SOR / clustering is not live yet)
     a.desc = l->d_vp_desc;
     a.group_stride = l->vp_gstride;
-    a.group_launch = l->vox_full_groups ? l->vp_gstride - 1 : std::min(l->vp_group_hint, vox_part_group_bound(h->vplan, max_n));
+    a.group_launch = r.vox_groups;
     a.flags = l->d_vf_flags;
     a.warnings = (effective_outputs(p) & PCOP_OUT_CROP) ? nullptr : l->d_warnings;  // zeroed by k_vp_init
     a.n_crop = l->cnt(CNT_CROP);
@@ -348,7 +359,7 @@ int run_wave_stages(Lane* l, int B, const float4* in, size_t stride, int max_n) 
     cur = l->d_vox;
     cur_stride = h->cap;
     cur_n = l->cnt(CNT_VOX);
-  } else if (fused) {
+  } else if (r.vox == WaveRoute::VOX_LSD) {
     // crop + VoxelGrid in one pass over the input (stage_voxel_fused.cu); the cropped cloud itself is only
     // materialised when it is a requested output
     {
@@ -422,16 +433,16 @@ int run_wave_stages(Lane* l, int B, const float4* in, size_t stride, int max_n) 
   l->plane_in = cur;
   l->plane_stride = cur_stride;
   l->plane_n = cur_n;
-  TRY(run_wave_plane(l, B, max_n, l->expect_large_plane));
+  TRY(run_wave_plane(l, B, max_n, r));
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail_cuda(h, e, "stage launches", __FILE__, __LINE__);
   return PCOP_OK;
 }
 
-// Clustering + centroid / radius of one wave.  The host does not know the remaining-cloud sizes yet; with_generic =
-// false launches only the fused small-cloud kernel (finish_wave repeats the stage with the generic kernels if a frame
-// turned out larger, see run_cluster).
-int run_wave_cluster(Lane* l, int B, int max_n, bool with_generic) {
+// Clustering + centroid / radius of one wave.  The host does not know the remaining-cloud sizes yet; without
+// r.cluster_generic only the fused small-cloud kernel runs (settle_wave repeats the stage with the generic kernels if a
+// frame turned out larger, see run_cluster).
+int run_wave_cluster(Lane* l, int B, int max_n, const WaveRoute& r) {
   pcop_handle* h = l->h;
   const pcop_params& p = h->params;
   Ctx c = make_ctx(l, B, max_n);
@@ -440,7 +451,7 @@ int run_wave_cluster(Lane* l, int B, int max_n, bool with_generic) {
   {
     StageTimer t(l, PCOP_STAGE_CLUSTER);
     if (p.enable_cluster) {
-      generic_centroid = run_cluster(c, ca, with_generic);  // the fused small-cloud kernel writes the obstacles itself
+      generic_centroid = run_cluster(c, ca, r.cluster_generic);  // the fused small-cloud kernel writes the obstacles itself
     } else {
       cudaMemsetAsync(l->cnt(CNT_CLUS), 0, sizeof(int) * B, l->stream);
       cudaMemsetAsync(l->cnt(CNT_CLPTS), 0, sizeof(int) * B, l->stream);
@@ -450,7 +461,6 @@ int run_wave_cluster(Lane* l, int B, int max_n, bool with_generic) {
     StageTimer t(l, PCOP_STAGE_CENTROID);
     if (p.enable_cluster && generic_centroid) run_centroid_radius(c, ca);
   }
-  l->wave_cluster_speculated = p.enable_cluster && !generic_centroid && max_n > h->ece_small_max;
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail_cuda(h, e, "stage launches", __FILE__, __LINE__);
   return PCOP_OK;
@@ -462,9 +472,9 @@ size_t pc2_payload_bytes(const pcop_pointcloud2_frame& m) { return (size_t)m.n_p
 // reads it), every host payload into the lane's raw staging at a 256-byte aligned offset, device payloads are read in
 // place; one k_pc2_ingest launch decodes (and transforms) every message into d_in.  A repeat of the wave (voxel
 // decline) decodes again from the same staging -- the plane stage has overwritten d_in, the staging is intact.
-int enqueue_wave_decode(Lane* l, const Pc2Call& pc, int w0, int B, int max_n) {
+int enqueue_wave_decode(Lane* l, const Pc2Call& pc, int w0, int B, int max_n, bool repeat) {
   pcop_handle* h = l->h;
-  if (l->vox_redo < 0) {
+  if (!repeat) {
     size_t off = 0;
     for (int f = 0; f < B; ++f) {
       const pcop_pointcloud2_frame& m = pc.frames[w0 + f];
@@ -488,7 +498,7 @@ int enqueue_wave_decode(Lane* l, const Pc2Call& pc, int w0, int B, int max_n) {
 
 // Second half of a wave: clustering, result packing, and the copy of the wave's counts / plane records / pack sizes
 // into pinned memory, followed by ev_meta.
-int enqueue_wave_pack(Lane* l, int B, int max_n, uint32_t mask) {
+int enqueue_wave_pack(Lane* l, int B, int max_n, uint32_t mask, const WaveRoute& r) {
   pcop_handle* h = l->h;
   // pack the requested outputs of all frames of the wave
   Ctx c = make_ctx(l, B, max_n);
@@ -525,7 +535,7 @@ int enqueue_wave_pack(Lane* l, int B, int max_n, uint32_t mask) {
     seg(l->d_warnings, l->h_warnings, sizeof(uint32_t) * B);
     seg(l->d_prec, l->h_prec, sizeof(PlaneRecord) * B);
     seg(l->d_meta, l->h_meta, sizeof(PackMeta));
-    if (l->wave_used_fused) seg(l->d_vf_flags, l->h_vf_flags, sizeof(uint32_t) * B);
+    if (r.vox != WaveRoute::VOX_GENERIC) seg(l->d_vf_flags, l->h_vf_flags, sizeof(uint32_t) * B);
     static_assert(PK_N >= 5, "one pack block per metadata segment");
     if (any) {  // the (frame < 4, array k < 5) blocks of the pack kernel also carry metadata segment k out
       // (parts per (frame, array): 16 for the batched waves; a call of a few large frames gets enough to fill the GPU)
@@ -601,27 +611,27 @@ int enqueue_wave_grids(Lane* l, const OccCall& oc, int B, int max_n) {
   return PCOP_OK;
 }
 
-int enqueue_wave_back(Lane* l, const WaveInput& wi, int B, int max_n, uint32_t mask, bool cluster_with_generic) {
-  TRY(run_wave_cluster(l, B, max_n, cluster_with_generic));
+int enqueue_wave_back(Lane* l, const WaveInput& wi, int B, int max_n, uint32_t mask, const WaveRoute& r) {
+  TRY(run_wave_cluster(l, B, max_n, r));
   if (wi.occ) TRY(enqueue_wave_grids(l, *wi.occ, B, max_n));
-  return enqueue_wave_pack(l, B, max_n, mask);
+  return enqueue_wave_pack(l, B, max_n, mask, r);
 }
 
-// Enqueues one wave on lane l: input upload, all stages and enqueue_wave_back.  Returns without waiting for any of it.
-int enqueue_wave(Lane* l, const WaveInput& wi, int w0, int B, uint32_t mask) {
+// Enqueues one wave (largest frame: max_n points) on lane l along route r: input upload, all stages and
+// enqueue_wave_back.  Returns without waiting for any of it.  repeat: the wave ran before (a voxel decline); its
+// PointCloud2 payloads are staged already.
+int enqueue_wave(Lane* l, const WaveInput& wi, int w0, int B, int max_n, uint32_t mask, const WaveRoute& r, bool repeat) {
   pcop_handle* h = l->h;
   for (int s = 0; s < PCOP_N_STAGES; ++s) l->stage_used[s] = false;
   const float4* in;
   size_t stride;
   const int32_t* n = wi.n;
-  int max_n = 1;
-  for (int f = 0; f < B; ++f) max_n = std::max(max_n, (int)n[w0 + f]);
   {
     StageTimer t(l, PCOP_STAGE_H2D);
     memcpy(l->h_n_in, n + w0, sizeof(int) * B);  // (the lane's previous wave has been collected: the staging is free)
     PCOP_CUDA_TRY(cudaMemcpyAsync(l->cnt(CNT_IN), l->h_n_in, sizeof(int) * B, cudaMemcpyHostToDevice, l->stream));
     if (wi.pc2) {  // from the decode on, the wave is a host-input wave
-      TRY(enqueue_wave_decode(l, *wi.pc2, w0, B, max_n));
+      TRY(enqueue_wave_decode(l, *wi.pc2, w0, B, max_n, repeat));
       in = l->d_in;
       stride = h->cap;
     } else if (wi.on_device) {
@@ -645,76 +655,90 @@ int enqueue_wave(Lane* l, const WaveInput& wi, int w0, int B, uint32_t mask) {
     }
   }
   if (wi.occ) TRY(enqueue_wave_counts(l, *wi.occ, w0, B, in, stride, max_n));
-  TRY(run_wave_stages(l, B, in, stride, max_n));
+  TRY(run_wave_stages(l, B, in, stride, max_n, r));
   l->pending = true;
   l->pend_w0 = w0;
   l->pend_B = B;
   l->pend_max_n = max_n;
-  return enqueue_wave_back(l, wi, B, max_n, mask, l->expect_big_remaining);
+  l->route = r;
+  return enqueue_wave_back(l, wi, B, max_n, mask, r);
 }
 
+// Waits for the counts of the lane's wave in flight and corrects its route: each part of the wave a wrong guess left
+// undone runs again, then the lane's history takes in what the wave needed.  The repeats, in this order:
+//   - a frame the fused voxel path declined (a survivor with a NaN y or z: generic kernels; a bucket above the partition
+//     path's limit: LSD path; more groups than the reduce grid covered: worst-case grid) repeats the whole wave;
+//   - a plane-stage input too large for the resident tiers that ran repeats the wave from the plane stage on;
+//   - a remaining cloud too large for the fused clustering kernel repeats the back half with the generic kernels.
+int settle_wave(Lane* l, const WaveInput& wi, uint32_t mask) {
+  pcop_handle* h = l->h;
+  const pcop_params& p = h->params;
+  const int w0 = l->pend_w0, B = l->pend_B, max_n = l->pend_max_n;
+  const WaveRoute first = l->route;
+  WaveRoute r = first;
+  auto count = [&](int row, int f) { return l->h_counts[(size_t)row * h->maxB + f]; };
+  PCOP_CUDA_TRY(cudaEventSynchronize(l->ev_meta));
+  uint32_t vox_flags = 0u;
+  int max_groups = 0;
+  for (int f = 0; f < B && first.vox != WaveRoute::VOX_GENERIC; ++f) {
+    vox_flags |= l->h_vf_flags[f];
+    max_groups = std::max(max_groups, count(CNT_GROUPS, f));
+  }
+  if (vox_flags) {
+    r.vox = (vox_flags & 1u) ? WaveRoute::VOX_GENERIC : ((vox_flags & 2u) ? WaveRoute::VOX_LSD : WaveRoute::VOX_PARTITION);
+    r.vox_groups = l->vp_gstride - 1;
+    TRY(enqueue_wave(l, wi, w0, B, max_n, mask, r, /*repeat=*/true));
+    PCOP_CUDA_TRY(cudaEventSynchronize(l->ev_meta));
+    for (int f = 0; f < B && r.vox != WaveRoute::VOX_GENERIC; ++f)  // (the repeat's flags came back with its metadata)
+      if (l->h_vf_flags[f]) {
+        l->pending = false;
+        return fail(h, PCOP_ERR_INTERNAL, "the fused voxel path declined frame " + std::to_string(w0 + f) + " again on its repeat");
+      }
+  }
+  const bool plane_checked = p.enable_plane && h->plane_resident;
+  bool large = false, huge = false;
+  for (int f = 0; f < B && plane_checked; ++f) {  // (CNT_SOR = the plane stage's input size)
+    large = large || count(CNT_SOR, f) > plane_small_tier_max();
+    huge = huge || count(CNT_SOR, f) > plane_resident_max();
+  }
+  const bool small_tier_only = r.plane == WaveRoute::PLANE_SMALL && max_n > plane_small_tier_max();
+  if (r.plane != WaveRoute::PLANE_HOSTLOOP && (huge || (large && small_tier_only))) {
+    r.plane = huge ? WaveRoute::PLANE_HOSTLOOP : WaveRoute::PLANE_RESIDENT;
+    TRY(run_wave_plane(l, B, max_n, r));
+    TRY(enqueue_wave_back(l, wi, B, max_n, mask, r));
+    PCOP_CUDA_TRY(cudaEventSynchronize(l->ev_meta));
+  }
+  bool big = false;
+  for (int f = 0; f < B && p.enable_cluster; ++f) big = big || count(CNT_REM, f) > h->ece_small_max;
+  if (big && !r.cluster_generic && max_n > h->ece_small_max) {
+    r.cluster_generic = true;
+    TRY(enqueue_wave_back(l, wi, B, max_n, mask, r));
+    PCOP_CUDA_TRY(cudaEventSynchronize(l->ev_meta));
+  }
 
-// Waits for the lane's wave in flight, starts its payload copy and fills out[w0 .. w0 + B).  (Result pointers into
+  // history (from the first run: the group count of the frames, the voxel-path flags)
+  if (first.vox != WaveRoute::VOX_GENERIC) {
+    if (h->vplan.part_ok)  // the next wave's reduce grid: 1.25 x the largest frame seen, >= 64
+      l->vp_group_hint = std::min(l->vp_gstride - 1, std::max(64, max_groups + max_groups / 4 + 8));
+    if (l->vox_lsd_waves > 0) --l->vox_lsd_waves;
+    if (vox_flags & 2u) l->vox_lsd_waves = 64;  // dense buckets tend to come back: the next waves go straight to the LSD path
+  }
+  if (plane_checked) {
+    if (l->plane_hostloop_waves > 0) --l->plane_hostloop_waves;
+    if (huge) l->plane_hostloop_waves = 64;  // such frames tend to come back: host-looped kernels for the next waves
+    l->expect_large_plane = large;
+  }
+  if (p.enable_cluster) l->expect_big_remaining = big;
+  return PCOP_OK;
+}
+
+// Settles the lane's wave in flight, starts its payload copy and fills out[w0 .. w0 + B).  (Result pointers into
 // the pinned buffer are stored as offsets and fixed up when the call ends: the buffer may still grow.)
 int finish_wave(Lane* l, const WaveInput& wi, uint32_t mask, pcop_frame_result* out_all) {
   pcop_handle* h = l->h;
   if (!l->pending) return PCOP_OK;
+  TRY(settle_wave(l, wi, mask));
   const int w0 = l->pend_w0, B = l->pend_B;
-  PCOP_CUDA_TRY(cudaEventSynchronize(l->ev_meta));
-  if (l->wave_used_fused) {
-    uint32_t fl = 0u;
-    for (int f = 0; f < B; ++f) fl |= l->h_vf_flags[f];
-    if (h->vox_mode == 2 && l->vox_redo < 0) {  // size the next wave's reduce grid: 1.25 x the largest frame seen, >= 64
-      int mg = 0;
-      for (int f = 0; f < B; ++f) mg = std::max(mg, l->h_counts[(size_t)CNT_GROUPS * h->maxB + f]);
-      l->vp_group_hint = std::min(l->vp_gstride - 1, std::max(64, mg + mg / 4 + 8));
-    }
-    if (l->vox_lsd_waves > 0) --l->vox_lsd_waves;
-    if (fl & 2u) l->vox_lsd_waves = 64;  // dense buckets tend to come back: the next waves go straight to the LSD path
-    if (fl) {
-      // the fused voxel path declined a frame of this wave: a survivor with a NaN y or z (generic kernels), a bucket
-      // above the partition path's limit (LSD path), or more groups than the reduce grid covered (worst-case grid)
-      l->vox_redo = (fl & 1u) ? 0 : ((fl & 2u) ? 1 : 2);
-      l->vox_full_groups = true;
-      const int st = enqueue_wave(l, wi, w0, B, mask);
-      const bool fused_redo = l->vox_redo != 0;
-      l->vox_redo = -1;
-      l->vox_full_groups = false;
-      TRY(st);
-      PCOP_CUDA_TRY(cudaEventSynchronize(l->ev_meta));
-      for (int f = 0; f < B && fused_redo; ++f)  // (the repeat's flags came back with its metadata)
-        if (l->h_vf_flags[f]) {
-          l->pending = false;
-          return fail(h, PCOP_ERR_INTERNAL, "the fused voxel path declined frame " + std::to_string(w0 + f) + " again on its repeat");
-        }
-    }
-  }
-  if (h->params.enable_plane && h->plane_resident) {
-    bool large = false, huge = false;  // (CNT_SOR = the plane stage's input size)
-    for (int f = 0; f < B; ++f) {
-      const int s = l->h_counts[(size_t)CNT_SOR * h->maxB + f];
-      large = large || s > plane_small_tier_max();
-      huge = huge || s > plane_resident_max();
-    }
-    if (l->plane_hostloop_waves > 0) --l->plane_hostloop_waves;
-    if (huge) l->plane_hostloop_waves = 64;  // such frames tend to come back: host-looped kernels for the next waves
-    if (l->wave_plane_resident && (huge || (large && l->wave_plane_speculated))) {
-      // a frame too large for the tiers that ran: repeat the wave from the plane stage on
-      TRY(run_wave_plane(l, B, l->pend_max_n, true));
-      TRY(enqueue_wave_back(l, wi, B, l->pend_max_n, mask, l->expect_big_remaining));
-      PCOP_CUDA_TRY(cudaEventSynchronize(l->ev_meta));
-    }
-    l->expect_large_plane = large;
-  }
-  if (h->params.enable_cluster) {
-    bool big = false;
-    for (int f = 0; f < B; ++f) big = big || l->h_counts[(size_t)CNT_REM * h->maxB + f] > h->ece_small_max;
-    if (big && l->wave_cluster_speculated) {  // a remaining cloud too large for the fused kernel: generic clustering
-      TRY(enqueue_wave_back(l, wi, B, l->pend_max_n, mask, true));
-      PCOP_CUDA_TRY(cudaEventSynchronize(l->ev_meta));
-    }
-    l->expect_big_remaining = big;
-  }
   l->pending = false;
   pcop_frame_result* out = out_all + w0;
   const bool dev_results = (mask & PCOP_OUT_DEVICE) != 0;
@@ -945,7 +969,12 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
     const double th0 = h->trace ? trace_host_us() : 0.0;
     status = finish_wave(l, wi, mask, out);  // (the lane's previous wave, if any)
     const double th1 = h->trace ? trace_host_us() : 0.0;
-    if (status == PCOP_OK) status = enqueue_wave(l, wi, waves[w].first, waves[w].second, mask);
+    if (status == PCOP_OK) {  // (after the finish: the route follows the history the lane's previous wave left)
+      const int w0 = waves[w].first, B = waves[w].second;
+      int max_n = 1;
+      for (int f = w0; f < w0 + B; ++f) max_n = std::max(max_n, (int)n[f]);
+      status = enqueue_wave(l, wi, w0, B, max_n, mask, next_route(l, max_n), /*repeat=*/false);
+    }
     if (h->trace)
       fprintf(stderr, "[pcop trace]   host: wave %4d+%-4d lane %zu: finish of the lane's previous wave %7.0f .. %7.0f us, enqueue .. %7.0f us\n",
               waves[w].first, waves[w].second, w % lanes.size(), th0, th1, trace_host_us());

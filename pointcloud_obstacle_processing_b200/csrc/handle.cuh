@@ -94,6 +94,16 @@ struct WaveInput {
   const OccCall* occ;  // non-null: the grid product of every frame as well
 };
 
+// What one wave launches where the frame sizes decide the path.  The host does not know those sizes when it enqueues
+// the wave, so the first route is a guess from the lane's earlier waves (next_route, batch.cu); settle_wave checks it
+// against the wave's counts and repeats the part of the wave a wrong guess left undone.
+struct WaveRoute {
+  enum Vox { VOX_GENERIC, VOX_LSD, VOX_PARTITION } vox = VOX_GENERIC;  // crop + VoxelGrid: generic, fused LSD / partition
+  int vox_groups = 0;  // VOX_PARTITION: reduce groups per frame
+  enum Plane { PLANE_SMALL, PLANE_RESIDENT, PLANE_HOSTLOOP } plane = PLANE_SMALL;  // small tier, both resident tiers, host loop
+  bool cluster_generic = false;  // the generic clustering kernels run beside the fused small-cloud kernel
+};
+
 constexpr int PCOP_MIN_LANE_WAVE = 8;  // a call is split over the lanes only when every lane gets at least this many frames
 struct Lane;
 
@@ -101,8 +111,7 @@ struct Lane;
 
 struct pcop_handle {
   pcop_params params;
-  pcop::VoxFusedPlan vplan{};  // fused crop + voxel fast path (ok = 0: not applicable to these parameters)
-  int vox_mode = 0;            // 0 generic crop + voxel kernels, 1 fused LSD path, 2 fused partition path
+  pcop::VoxFusedPlan vplan{};  // fused crop + voxel paths (ok = 0: generic kernels; part_ok = 0: no partition path)
   int device = 0;
   int cap = 0;
   int maxB = 0;                // frames of one lane's wave buffers
@@ -207,6 +216,7 @@ struct Lane {
   bool pending = false;             // a wave is enqueued and not yet collected
   int pend_w0 = 0, pend_B = 0;
   int pend_max_n = 1;
+  WaveRoute route;                  // of the wave in flight
   std::vector<size_t> fixups;  // result-pointer slots of the running call (byte offsets into the caller's array)
   struct TraceRec {
     int w0, B;
@@ -216,23 +226,17 @@ struct Lane {
   std::vector<TraceRec> trace_recs;
   size_t trace_used = 0;
 
-  // speculation: what the lane's last waves saw decides which tiers its next wave launches
+  // history: what the lane's last waves needed decides the next wave's route (next_route, batch.cu)
   bool expect_big_remaining = false;  // the last collected wave had a remaining cloud above ece_small_max
   bool expect_large_plane = false;    // ... a plane-stage input above the small tier of the resident plane kernel
   int plane_hostloop_waves = 0;       // waves left that take the host-looped plane kernels (a frame was above the resident limit)
   int vox_lsd_waves = 0;              // waves left that take the LSD voxel path (the partition path declined a bucket)
-  bool wave_plane_resident = false;   // the wave in flight ran the resident plane path
-  bool wave_plane_speculated = false; // the wave in flight ran the small tier only
   const float4* plane_in = nullptr;   // plane-stage input of the wave in flight (for a repeat of the stage)
   size_t plane_stride = 0;
   const int* plane_n = nullptr;
-  bool wave_cluster_speculated = false;  // the wave in flight ran the fused clustering kernel only
   uint32_t* d_vf_flags = nullptr;  // [maxB]
   unsigned long long* d_vf_pair[2] = {nullptr, nullptr};
   uint32_t* h_vf_flags = nullptr;
-  int vox_redo = -1;               // >= 0 while a wave is repeated: the mode to take instead of vox_mode
-  bool vox_full_groups = false;    // ... with the worst-case reduce grid of the partition path
-  bool wave_used_fused = false;
   // partition voxel path (allocated and grown by apply_params while the plan allows the path)
   uint32_t* d_vp_hist = nullptr;
   uint32_t* d_vp_bstart = nullptr;
@@ -338,7 +342,7 @@ inline bool pc2_layout_ok(int point_step, int ox, int oy, int oz) {
 
 inline Ctx make_ctx(Lane* l, int B, int grid_cap = -1) {
   const int cap = l->h->cap;
-  return Ctx{l->stream, B, cap, &l->h->launches, &l->h->kt, (grid_cap > 0 && grid_cap < cap) ? grid_cap : cap, nullptr};
+  return Ctx{l->stream, B, cap, &l->h->launches, &l->h->kt, (grid_cap > 0 && grid_cap < cap) ? grid_cap : cap};
 }
 
 inline PlaneConst make_plane_const(const pcop_params& p) {

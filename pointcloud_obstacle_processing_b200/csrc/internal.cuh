@@ -33,16 +33,7 @@ struct Ctx {
   int64_t* launches;
   KernelTimers* kt;
   int grid_cap;  // points per frame the launch grids must cover (<= cap; the host lowers it when it knows a bound)
-  cudaEvent_t block_ev = nullptr;  // non-null: host waits sleep on this blocking-sync event instead of spinning
 };
-
-// host wait for everything queued on the stream: spin (cudaStreamSynchronize, lowest latency) or sleep on a
-// blocking-sync event (when several processes share few cores, spinning lane threads starve each other)
-inline cudaError_t stream_wait(cudaStream_t s, cudaEvent_t block_ev) {
-  if (!block_ev) return cudaStreamSynchronize(s);
-  const cudaError_t e = cudaEventRecord(block_ev, s);
-  return e != cudaSuccess ? e : cudaEventSynchronize(block_ev);
-}
 
 inline void count_launch(const Ctx& c, int n = 1) { *c.launches += n; }
 

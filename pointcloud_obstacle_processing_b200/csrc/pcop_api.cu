@@ -55,14 +55,13 @@ void fill_rng_table(uint32_t seed, int* out, int count) {
 
 // crop + VoxelGrid paths: the fused partition path when the plan allows it, else the fused LSD path, else the generic
 // kernels.  PCOP_VOXEL_FUSED=0 forces the generic kernels, =lsd the LSD path (the tests cover all three).
-VoxFusedPlan make_plan(const pcop_params& p, size_t max_points, int* mode) {
+VoxFusedPlan make_plan(const pcop_params& p, size_t max_points) {
   VoxFusedPlan pl = make_vox_fused_plan(p);
   vox_part_plan(pl, max_points);
   const char* s = getenv("PCOP_VOXEL_FUSED");
   if (s && s[0] == '0') pl.ok = 0;
   if (s && (s[0] == 'l' || s[0] == 'L')) pl.part_ok = 0;
   if (!pl.ok) pl.part_ok = 0;
-  *mode = pl.part_ok ? 2 : (pl.ok ? 1 : 0);
   return pl;
 }
 
@@ -263,10 +262,9 @@ int init_lane(Lane* l) {
 
 // Parameters of pcop_create and pcop_set_params (validated): every lane's buffers that depend on them are grown
 // first (never shrunk), so a failure leaves the handle with its previous parameters; then the RANSAC table (16 KB of
-// the seed's rnd() values), the crop + VoxelGrid plan and the lanes' partition-path stride and speculation state.
+// the seed's rnd() values), the crop + VoxelGrid plan and the lanes' partition-path stride and route history.
 int apply_params(pcop_handle* h, const pcop_params& p) {
-  int mode = 0;
-  const VoxFusedPlan plan = make_plan(p, (size_t)h->cap, &mode);
+  const VoxFusedPlan plan = make_plan(p, (size_t)h->cap);
   const int gstride = plan.part_ok ? vox_part_group_bound(plan, h->cap) + 1 : 0;
   const int B = h->maxB;
   for (auto& lp : h->lanes) {
@@ -295,8 +293,7 @@ int apply_params(pcop_handle* h, const pcop_params& p) {
   PCOP_CUDA_TRY(cudaMemcpy(h->d_rng, tbl.data(), sizeof(int) * RNG_TABLE, cudaMemcpyHostToDevice));
   h->params = p;
   h->vplan = plan;
-  h->vox_mode = mode;
-  for (auto& l : h->lanes) {
+  for (auto& l : h->lanes) {  // (route history: the countdowns and the group hint start over, the sizes of the last wave are kept)
     if (plan.part_ok) {
       l->vp_gstride = gstride;
       l->vp_group_hint = gstride - 1;

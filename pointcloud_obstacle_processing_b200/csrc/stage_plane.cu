@@ -1312,7 +1312,7 @@ static cudaError_t run_plane_hostloop(const Ctx& c, const PlaneArgs& a) {
   KL(c, "k_plane_init", k_plane_init<<<cdiv(c.B, 128), 128, 0, c.stream>>>(a.pf, a.n_in, a.pc.keep_fraction, a.n_active, a.n_in_copy, c.B));
   count_launch(c);
   cudaMemcpyAsync(a.h_n_active, a.n_active, 3 * sizeof(int), cudaMemcpyDeviceToHost, c.stream);
-  if ((e = stream_wait(c.stream, c.block_ev)) != cudaSuccess) return e;
+  if ((e = cudaStreamSynchronize(c.stream)) != cudaSuccess) return e;
   Ctx cc = c;
   while (*a.h_n_active > 0) {
     cc.grid_cap = max(1, min(c.grid_cap, a.h_n_active[1]));
@@ -1340,7 +1340,7 @@ static cudaError_t run_plane_hostloop(const Ctx& c, const PlaneArgs& a) {
     KL(c, "k_plane_update", k_plane_update<<<cdiv(c.B, 128), 128, 0, c.stream>>>(a.pf, a.n_tmp, a.pc.keep_fraction, a.n_active, a.warnings, c.B));
     count_launch(c, 9);
     cudaMemcpyAsync(a.h_n_active, a.n_active, 3 * sizeof(int), cudaMemcpyDeviceToHost, c.stream);
-    if ((e = stream_wait(c.stream, c.block_ev)) != cudaSuccess) return e;
+    if ((e = cudaStreamSynchronize(c.stream)) != cudaSuccess) return e;
   }
   return cudaGetLastError();
 }
