@@ -281,8 +281,7 @@ WaveRoute next_route(const Lane* l, int max_n) {
   } else if (h->vplan.ok) {
     r.vox = WaveRoute::VOX_LSD;
   }
-  if (!h->plane_resident || l->plane_hostloop_waves > 0) r.plane = WaveRoute::PLANE_HOSTLOOP;
-  else if (l->expect_large_plane) r.plane = WaveRoute::PLANE_RESIDENT;
+  r.plane_large = l->expect_large_plane;
   r.cluster_generic = l->expect_big_remaining || h->ece_small_max <= 0;  // (no fused kernel at all: run_cluster)
   return r;
 }
@@ -295,8 +294,7 @@ int run_wave_plane(Lane* l, int B, int max_n, const WaveRoute& r) {
   if (p.enable_plane) {
     PlaneArgs a = make_plane_args(l, l->plane_in, l->plane_stride, l->plane_n);
     a.n_in_copy = p.enable_sor ? nullptr : l->cnt(CNT_SOR);
-    a.resident = r.plane != WaveRoute::PLANE_HOSTLOOP;
-    a.large_tier = r.plane == WaveRoute::PLANE_RESIDENT;
+    a.large_tier = r.plane_large;
     if (!(effective_outputs(p) & PCOP_OUT_PLANE)) a.inlier_idx = nullptr;  // the inlier list is only written on request
     cudaError_t e = run_plane(c, a);
     if (e != cudaSuccess) return fail_cuda(l->h, e, "run_plane", __FILE__, __LINE__);
@@ -668,7 +666,7 @@ int enqueue_wave(Lane* l, const WaveInput& wi, int w0, int B, int max_n, uint32_
 // undone runs again, then the lane's history takes in what the wave needed.  The repeats, in this order:
 //   - a frame the fused voxel path declined (a survivor with a NaN y or z: generic kernels; a bucket above the partition
 //     path's limit: LSD path; more groups than the reduce grid covered: worst-case grid) repeats the whole wave;
-//   - a plane-stage input too large for the resident tiers that ran repeats the wave from the plane stage on;
+//   - a plane-stage input above the small plane tier, when only that tier ran, repeats the wave from the plane stage on;
 //   - a remaining cloud too large for the fused clustering kernel repeats the back half with the generic kernels.
 int settle_wave(Lane* l, const WaveInput& wi, uint32_t mask) {
   pcop_handle* h = l->h;
@@ -695,15 +693,11 @@ int settle_wave(Lane* l, const WaveInput& wi, uint32_t mask) {
         return fail(h, PCOP_ERR_INTERNAL, "the fused voxel path declined frame " + std::to_string(w0 + f) + " again on its repeat");
       }
   }
-  const bool plane_checked = p.enable_plane && h->plane_resident;
-  bool large = false, huge = false;
-  for (int f = 0; f < B && plane_checked; ++f) {  // (CNT_SOR = the plane stage's input size)
+  bool large = false;
+  for (int f = 0; f < B && p.enable_plane; ++f)  // (CNT_SOR = the plane stage's input size)
     large = large || count(CNT_SOR, f) > plane_small_tier_max();
-    huge = huge || count(CNT_SOR, f) > plane_resident_max();
-  }
-  const bool small_tier_only = r.plane == WaveRoute::PLANE_SMALL && max_n > plane_small_tier_max();
-  if (r.plane != WaveRoute::PLANE_HOSTLOOP && (huge || (large && small_tier_only))) {
-    r.plane = huge ? WaveRoute::PLANE_HOSTLOOP : WaveRoute::PLANE_RESIDENT;
+  if (large && !r.plane_large) {
+    r.plane_large = true;
     TRY(run_wave_plane(l, B, max_n, r));
     TRY(enqueue_wave_back(l, wi, B, max_n, mask, r));
     PCOP_CUDA_TRY(cudaEventSynchronize(l->ev_meta));
@@ -723,11 +717,7 @@ int settle_wave(Lane* l, const WaveInput& wi, uint32_t mask) {
     if (l->vox_lsd_waves > 0) --l->vox_lsd_waves;
     if (vox_flags & 2u) l->vox_lsd_waves = 64;  // dense buckets tend to come back: the next waves go straight to the LSD path
   }
-  if (plane_checked) {
-    if (l->plane_hostloop_waves > 0) --l->plane_hostloop_waves;
-    if (huge) l->plane_hostloop_waves = 64;  // such frames tend to come back: host-looped kernels for the next waves
-    l->expect_large_plane = large;
-  }
+  if (p.enable_plane) l->expect_large_plane = large;
   if (p.enable_cluster) l->expect_big_remaining = big;
   return PCOP_OK;
 }

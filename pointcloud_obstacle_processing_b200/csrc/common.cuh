@@ -106,16 +106,12 @@ struct PlaneFrame {  // state of the plane loop of one frame
   int n_passes;
   int n_hyp;         // hypotheses generated this pass
   int gen_end;       // generator stopped early: 0 no, 1 empty sample / skip limit, 2 rng table exhausted
-  int best;          // selected hypothesis or -1
-  int model_ok;      // selected + valid
-  int need_more;     // the adaptive-k replay ran past the hypotheses scored so far
   int n_inliers_last;
-  double log_prob;   // det_log(1 - probability) (frame-resident path: evaluated once per frame)
+  double log_prob;   // det_log(1 - probability), evaluated once per frame
   float4 coeff_sel;  // RANSAC winner
   float4 coeff_ref;  // after refinement
   float4 hyp[MAX_HYP];
   int hyp_valid[MAX_HYP];  // isModelValid
-  int counts[MAX_HYP];
   int pass_points[PCOP_MAX_PLANE_PASSES_RECORDED];
   int pass_inliers[PCOP_MAX_PLANE_PASSES_RECORDED];
   float4 pass_coeff[PCOP_MAX_PLANE_PASSES_RECORDED];

@@ -18,7 +18,6 @@ enum {  // rows of the per-frame count table (device: d_counts[row*maxB + f])
   CNT_REM,
   CNT_CLUS,
   CNT_CLPTS,
-  CNT_TMP,
   CNT_NINL,   // inliers of the last segment() call
   CNT_CLUS1,  // C + 1 (CSR offsets length)
   CNT_CELLS,  // occupied clique cells (ECE scratch)
@@ -100,7 +99,7 @@ struct WaveInput {
 struct WaveRoute {
   enum Vox { VOX_GENERIC, VOX_LSD, VOX_PARTITION } vox = VOX_GENERIC;  // crop + VoxelGrid: generic, fused LSD / partition
   int vox_groups = 0;  // VOX_PARTITION: reduce groups per frame
-  enum Plane { PLANE_SMALL, PLANE_RESIDENT, PLANE_HOSTLOOP } plane = PLANE_SMALL;  // small tier, both resident tiers, host loop
+  bool plane_large = false;  // the large plane tier runs beside the small one
   bool cluster_generic = false;  // the generic clustering kernels run beside the fused small-cloud kernel
 };
 
@@ -119,7 +118,6 @@ struct pcop_handle {
   int wave_frames = 0;         // frames per wave a batched call aims at (<= maxB; PCOP_WAVE_FRAMES at create)
   bool trace = false;          // PCOP_TRACE at create: per-wave device timeline of every call on stderr
   int ece_small_max = 0;       // ECE_SMALL_MAX or PCOP_ECE_SMALL_MAX (read at create)
-  int plane_resident = 1;      // 0: PCOP_PLANE_RESIDENT=0 at create (host-looped plane kernels)
   std::vector<std::unique_ptr<pcop::Lane>> lanes;  // batched calls deal their waves round-robin to the lanes
   std::string err;
   std::vector<void*> dev_allocs;
@@ -175,7 +173,6 @@ struct Lane {
   PlaneRecord* d_prec = nullptr;
   double* d_partial = nullptr;  // [maxB][chunks][10]
   double* d_thr = nullptr;
-  int* d_n_active = nullptr;
   int* d_pack_off = nullptr;  // [PK_N][maxB]
   PackMeta* d_meta = nullptr;
   unsigned char* d_pack = nullptr;  // packed results of the wave in flight (PCOP_OUT_DEVICE: of all waves of the call)
@@ -195,7 +192,6 @@ struct Lane {
   Pc2Frame* h_pc2 = nullptr;       // [maxB] pinned staging of the same (the batched PointCloud2 wave)
 
   // pinned host
-  int* h_n_active = nullptr;
   int* h_counts = nullptr;  // [CNT_ROWS][maxB]
   uint32_t* h_warnings = nullptr;
   PlaneRecord* h_prec = nullptr;
@@ -228,8 +224,7 @@ struct Lane {
 
   // history: what the lane's last waves needed decides the next wave's route (next_route, batch.cu)
   bool expect_big_remaining = false;  // the last collected wave had a remaining cloud above ece_small_max
-  bool expect_large_plane = false;    // ... a plane-stage input above the small tier of the resident plane kernel
-  int plane_hostloop_waves = 0;       // waves left that take the host-looped plane kernels (a frame was above the resident limit)
+  bool expect_large_plane = false;    // ... a plane-stage input above the small tier of the plane kernel
   int vox_lsd_waves = 0;              // waves left that take the LSD voxel path (the partition path declined a bucket)
   const float4* plane_in = nullptr;   // plane-stage input of the wave in flight (for a repeat of the stage)
   size_t plane_stride = 0;
@@ -372,12 +367,7 @@ inline PlaneArgs make_plane_args(Lane* l, const float4* in, size_t stride, const
   a.inlier_idx = l->d_inliers;
   a.pf = l->d_pf;
   a.partial = l->d_partial;
-  a.desc = l->d_desc;
-  a.n_tmp = l->cnt(CNT_TMP);
-  a.n_active = l->d_n_active;
-  a.h_n_active = l->h_n_active;
   a.rng = h->d_rng;
-  a.resident = h->plane_resident;
   a.pc = make_plane_const(h->params);
   a.warnings = l->d_warnings;
   a.out = l->d_rem;

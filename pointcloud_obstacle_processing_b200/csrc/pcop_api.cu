@@ -237,13 +237,11 @@ int init_lane(Lane* l) {
   TRY(dalloc(h, &l->d_prec, B));
   TRY(dalloc(h, &l->d_partial, (size_t)B * chunks * 10));
   TRY(dalloc(h, &l->d_thr, B));
-  TRY(dalloc(h, &l->d_n_active, 64));
   TRY(dalloc(h, &l->d_pack_off, (size_t)PK_N * B));
   TRY(dalloc(h, &l->d_meta, 1));
   TRY(dalloc(h, &l->d_pack_cursor, 1));
   TRY(dalloc(h, &l->d_pc2, B));
   TRY(halloc(h, &l->h_pc2, B));
-  TRY(halloc(h, &l->h_n_active, 16));
   TRY(halloc(h, &l->h_counts, (size_t)CNT_ROWS * B));
   TRY(halloc(h, &l->h_warnings, B));
   TRY(halloc(h, &l->h_prec, B));
@@ -293,13 +291,12 @@ int apply_params(pcop_handle* h, const pcop_params& p) {
   PCOP_CUDA_TRY(cudaMemcpy(h->d_rng, tbl.data(), sizeof(int) * RNG_TABLE, cudaMemcpyHostToDevice));
   h->params = p;
   h->vplan = plan;
-  for (auto& l : h->lanes) {  // (route history: the countdowns and the group hint start over, the sizes of the last wave are kept)
+  for (auto& l : h->lanes) {  // (route history: the LSD-path countdown and the group hint start over, the sizes of the last wave are kept)
     if (plan.part_ok) {
       l->vp_gstride = gstride;
       l->vp_group_hint = gstride - 1;
     }
     l->vox_lsd_waves = 0;
-    l->plane_hostloop_waves = 0;
   }
   return PCOP_OK;
 }
@@ -419,7 +416,6 @@ int pcop_create(const pcop_params* params, int device, size_t max_points, int ma
   h->wave_frames = std::min(wave_frames, lane_batch);
   h->trace = getenv("PCOP_TRACE") != nullptr;
   h->ece_small_max = ece_small_limit();
-  if (const char* s = getenv("PCOP_PLANE_RESIDENT")) h->plane_resident = (s[0] == '0') ? 0 : 1;  // (the tests cover both paths)
   const int st = [&] {  // everything the handle allocates, then the parameters
     TRY(validate_params(h, *params));
     PCOP_CUDA_TRY(cudaSetDevice(h->device));
@@ -909,7 +905,6 @@ int pcop_plane(pcop_handle* h, const float* xyzw, int32_t s, float* remaining_xy
   Ctx c = make_ctx(l, 1, s);
   PlaneArgs a = make_plane_args(l, l->d_in, h->cap, l->cnt(CNT_SOR));
   a.large_tier = 1;
-  if (s > plane_resident_max()) a.resident = 0;  // (the host knows the size here)
   cudaError_t e = run_plane(c, a);
   if (e != cudaSuccess) return fail_cuda(h, e, "run_plane", __FILE__, __LINE__);
   KL(c, "k_plane_record", k_plane_record<<<1, 32, 0, l->stream>>>(l->d_pf, l->d_prec, l->cnt(CNT_NINL), l->cnt(CNT_CLUS), l->cnt(CNT_CLUS1), 1, 1));

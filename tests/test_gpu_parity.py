@@ -35,18 +35,6 @@ def vox_path(request, monkeypatch):
     return request.param
 
 
-@pytest.fixture(params=["resident", "hostloop"])
-def plane_path(request, monkeypatch):
-    """The plane loop has two device paths: the frame-resident cluster kernel (one launch runs every pass) and the
-    host-looped kernels (the fallback for frames above 131072 points); PCOP_PLANE_RESIDENT=0 (read when the handle is
-    created) forces the latter."""
-    if request.param == "hostloop":
-        monkeypatch.setenv("PCOP_PLANE_RESIDENT", "0")
-    else:
-        monkeypatch.delenv("PCOP_PLANE_RESIDENT", raising=False)
-    return request.param
-
-
 def all_outputs(p):
     p = p.copy()
     p.outputs = abi.OUT_ALL
@@ -114,10 +102,12 @@ def test_stage_sor_with_non_finite_points(frames):
     assert_bits_equal(g_pts, o_pts, "sor points")
 
 
-@pytest.mark.parametrize("config", [1, 2, 3])
-def test_stage_plane(config, frames, plane_path):
+@pytest.mark.parametrize("config,index", [(1, 0), (2, 0), (2, 1), (3, 0), (3, 1), (4, 0)])
+def test_stage_plane(config, index):
+    """plane inputs of 8 684 (small tier), 56 424 and about 56 000, 129 789 (large tier), 132 404 (windows) and 999 976
+    points (windows, 13 passes)"""
     p = synth.params(config)
-    cloud, _ = O.crop(p, frames[config])
+    cloud, _ = O.crop(p, synth.frame(config, index))
     cloud, _, _ = O.voxel(p, cloud)
     with ObstacleProcessor(p, len(cloud)) as op:
         g = op.segment_plane_and_extract_indices(cloud)
@@ -445,22 +435,78 @@ def _planes_cloud(rng, n, fracs, noise=0.01):
 
 
 @pytest.mark.parametrize("n,fracs", [(30000, (0.35, 0.25, 0.15, 0.1)), (9000, (0.3, 0.2, 0.12, 0.1, 0.08)),
-                                     (100000, (0.4, 0.2, 0.15))])
-def test_plane_multi_pass(n, fracs, plane_path):
+                                     (100000, (0.4, 0.2, 0.15)), (66000, (0.35, 0.25, 0.15, 0.1)),
+                                     (150000, (0.4, 0.25, 0.15)), (1000000, (0.4, 0.2, 0.15))])
+def test_plane_multi_pass(n, fracs):
     """several passes inside one launch: the second and later passes generate their hypotheses in the kernel and
-    reload the cloud that the previous pass wrote"""
+    reload the cloud that the previous pass wrote (66 000 points: the large tier from the first pass on; 150 000 and
+    1 000 000: windows in the first passes)"""
     p = synth.params(2)
     rng = np.random.default_rng(77 + n)
     o = _compare_plane(p, _cloud(_planes_cloud(rng, n, fracs)))
     assert o["n_passes"] >= 3, o["n_passes"]
 
 
-def test_plane_frame_above_resident_capacity_takes_host_loop():
-    """more than 131072 points do not fit the cluster's shared memory: same result from the host-looped kernels"""
+def _collinear_cloud(rng, n, frac_line):
+    """a share of exactly collinear points ((p1-p0)/(p2-p0) has equal components) in a flat clutter: samples drawn from
+    the line fail isSampleGood and are redrawn"""
+    n_line = int(n * frac_line)
+    t = rng.integers(-2000, 2000, n_line).astype(np.float32) / 64.0
+    line = np.stack([t, t, t], axis=1)
+    rest = np.concatenate([rng.uniform(-30, 30, size=(n - n_line, 2)), rng.normal(size=(n - n_line, 1)) * 0.05], axis=1)
+    pts = np.concatenate([line, rest]).astype(np.float32)
+    return pts[rng.permutation(n)]
+
+
+@pytest.mark.parametrize("case", ["n131073", "n150000", "n300000", "collinear", "no_plane"])
+def test_plane_large_frames_in_windows(case):
+    """frames above 8 x 16384 points: each CTA of the large tier walks its part of the frame in windows of its slice.
+    131073 points: CTAs 0-6 own 18432 points (a full window and a 2048-point one), CTA 7 owns 2049 in one window;
+    300000 points: later passes reload windows that other CTAs wrote in the same launch; redraws of collinear samples;
+    a cloud whose RANSAC finds no plane (the loop breaks on its first pass)"""
     p = synth.params(2)
     rng = np.random.default_rng(5)
-    o = _compare_plane(p, _cloud(_planes_cloud(rng, 150000, (0.45, 0.3))))
-    assert o["n_passes"] >= 2
+    if case == "n131073":
+        pts, min_passes = _planes_cloud(rng, 131073, (0.45, 0.3)), 2
+    elif case == "n150000":
+        pts, min_passes = _planes_cloud(rng, 150000, (0.45, 0.3)), 2
+    elif case == "n300000":
+        pts, min_passes = _planes_cloud(rng, 300000, (0.4, 0.2, 0.15)), 3
+    elif case == "collinear":
+        pts, min_passes = _collinear_cloud(rng, 140000, 0.5), 0
+    else:  # a zero threshold: no point is closer than 0 to any plane, the loop breaks on its first pass
+        p.plane_segment_dist_thres = 0.0
+        pts, min_passes = rng.uniform(-50, 50, size=(140000, 3)).astype(np.float32), 0
+    o = _compare_plane(p, _cloud(pts))
+    assert o["n_passes"] >= min_passes, o["n_passes"]
+    if case == "no_plane":
+        assert o["n_passes"] == 0 and o["warnings"] & abi.WARN_PLANE_BREAK, o
+
+
+def test_plane_batch_with_large_and_windowed_frames():
+    """one wave through pcop_process_batch: a small-tier frame, a large-tier frame in one window per CTA, a frame in
+    several windows, an empty frame, and frames that need different numbers of passes"""
+    p = all_outputs(synth.params(2))
+    p.enable_crop = 0
+    p.enable_voxel = 0
+    rng = np.random.default_rng(23)
+    clouds = [_planes_cloud(rng, 20000, (0.8,)), _planes_cloud(rng, 100000, (0.35, 0.3, 0.2)),
+              _planes_cloud(rng, 200000, (0.4, 0.25, 0.15)), np.zeros((0, 3), np.float32),
+              _planes_cloud(rng, 150000, (0.5, 0.25))]
+    cap = max(len(c) for c in clouds)
+    batch = np.zeros((len(clouds), cap, 4), np.float32)
+    counts = np.array([len(c) for c in clouds], np.int32)
+    for f, c in enumerate(clouds):
+        batch[f, :len(c), :3] = c
+        batch[f, :len(c), 3] = 1.0
+    with ObstacleProcessor(p, cap, max_batch=len(clouds)) as op:
+        res = op.process_batch(batch, counts)
+    passes = []
+    for f in range(len(clouds)):
+        o = O.process(p, batch[f, :counts[f]])
+        compare_frames(res[f], o, p, f"frame{f}: ")
+        passes.append(o.n_plane_passes)
+    assert len(set(passes)) >= 3, passes
 
 
 def test_plane_batch_frames_with_different_pass_counts():
@@ -490,19 +536,15 @@ def test_plane_batch_frames_with_different_pass_counts():
     assert len(set(passes)) >= 3, passes
 
 
+@pytest.mark.parametrize("n", [6000, 100000])
 @pytest.mark.parametrize("frac_line", [0.5, 0.9, 1.0])
-def test_plane_collinear_samples_redrawn(frac_line, plane_path):
+def test_plane_collinear_samples_redrawn(frac_line, n):
     """samples that fail isSampleGood are redrawn (consuming random numbers): the hypothesis generator's parallel
-    fast path must hand such frames to the sequential replay; an all-collinear cloud exhausts the 1000 redraws"""
+    fast path must hand such frames to the sequential replay; an all-collinear cloud exhausts the 1000 redraws.
+    6 000 points: small tier; 100 000: large tier, where later passes generate in the kernel from the cloud it wrote"""
     p = synth.params(2)
     rng = np.random.default_rng(61)
-    n = 6000
-    n_line = int(n * frac_line)
-    t = rng.integers(-2000, 2000, n_line).astype(np.float32) / 64.0
-    line = np.stack([t, t, t], axis=1)  # exactly collinear: (p1-p0)/(p2-p0) has equal components
-    rest = np.concatenate([rng.uniform(-30, 30, size=(n - n_line, 2)), rng.normal(size=(n - n_line, 1)) * 0.05], axis=1)
-    pts = np.concatenate([line, rest]).astype(np.float32)
-    pts = pts[rng.permutation(n)]
+    pts = _collinear_cloud(rng, n, frac_line)
     o = _compare_plane(p, _cloud(pts))
     print("passes", o["n_passes"], "warnings", o["warnings"])
 
