@@ -18,6 +18,7 @@
  *   od.cpp:817-833  handle_shadow_casting per cluster (od.cpp:467-672) + obstacle marks   -> pcop_occupancy_shadows
  *   od.cpp:699-852  pipeline + occupancy grid of a batch of frames                        -> pcop_process_batch_occupancy
  *   od.cpp:688-696 + 699-852  the same for a batch of raw PointCloud2 messages with a pose each -> pcop_process_batch_pointcloud2
+ *   od.cpp:688-701 + 699-852  ... with accumulate_count messages (or several sensors) per frame -> pcop_process_batch_pointcloud2_windows
  *
  * Plain C: POD structs, raw pointers and sizes, integer status codes.  No C++
  * exceptions, PCL, ROS or torch types cross this boundary.
@@ -330,7 +331,7 @@ int pcop_process_batch_occupancy(pcop_handle* h, const float* xyzw, size_t frame
  * GPU inside the batched pipeline; nothing returns to the host per message.
  *   frames             [batch] message descriptors (host memory); layouts may differ from message to message.  A
  *                      message with n_points == 0 may have data == NULL.  Payloads may be host or device pointers
- *                      (classified per message).  Host payloads should be pinned (cudaHostAlloc): a copy from pageable
+ *                      (classified per allocation).  Host payloads should be pinned (cudaHostAlloc): a copy from pageable
  *                      memory holds the calling thread until it has been staged, once per message, so the lanes stop
  *                      overlapping.  Device payloads are read in place.
  *   transform16        [batch][16] row-major floats (host memory), message f's world <- sensor pose, applied with
@@ -360,6 +361,35 @@ typedef struct pcop_pointcloud2_frame {
 int pcop_process_batch_pointcloud2(pcop_handle* h, const pcop_pointcloud2_frame* frames, int32_t batch,
                                    const float* transform16, const float* world_to_sensor16,
                                    const float* sensor_to_world16, int8_t* grids, pcop_frame_result* out);
+
+/* ---- accumulation windows: one frame from several posed messages (od.cpp:688-701 per processing callback) ---------
+ * The node appends accumulate_count posed messages to passthrough_input_cloud and runs the pipeline on the
+ * concatenation; a rig with several sensors merges their messages into one cloud per time step the same way.
+ * pcop_process_batch_pointcloud2_windows takes a whole message stream with one pose per message and returns, in one
+ * call, what the node computes for every processing callback:
+ *   messages, n_messages   [n_messages] descriptors as in pcop_process_batch_pointcloud2 (layouts and memory kinds may
+ *                          differ from message to message; payloads are classified per allocation)
+ *   window_first           [batch + 1] (host memory): frame f is the world-frame concatenation of messages
+ *                          window_first[f] .. window_first[f + 1] - 1, in message order (an empty window is a frame of
+ *                          0 points)
+ *   transform16            [n_messages][16] or NULL: message m's world <- sensor pose (as pcop_process_batch_pointcloud2)
+ *   world_to_sensor16, sensor_to_world16, grids    [batch] poses and grids, as pcop_process_batch_pointcloud2
+ *   out                    [batch]
+ * out[f] equals, byte for byte, what pcop_accumulate_reset + pcop_accumulate_pointcloud2(message m, transform16 + 16 m)
+ * for every m of window f in order + pcop_process_accumulated return: n_input is the window's total and crop_kept_idx
+ * indexes the concatenation.  With grids, frame f's results and grid equal pcop_process_batch_occupancy(NULL, ..., batch
+ * 1, world_to_sensor16 + 16 f, sensor_to_world16 + 16 f) after the same accumulation.  PCOP_OUT_DEVICE, result pointer
+ * lifetime and the alternating pinned result buffers behave as in pcop_process_batch.  The accumulator is neither read
+ * nor changed.  pcop_process_batch_pointcloud2 is this call with windows of one message each.
+ * Errors (the handle stays usable): PCOP_ERR_BAD_PARAM for every message check of pcop_process_batch_pointcloud2, for
+ * window_first[0] != 0, a decreasing window_first, window_first[batch] != n_messages, or window_first = NULL with
+ * batch > 0; PCOP_ERR_CAPACITY for a window of more than max_points records or a grid above PCOP_OCC_BATCH_MAX_CELLS.
+ * batch = 0 does nothing.  Every lane of the handle keeps the decode descriptors of its largest wave's messages
+ * (allocated by the first call, grown, never shrunk); the decode is one launch per wave whatever its message count. */
+int pcop_process_batch_pointcloud2_windows(pcop_handle* h, const pcop_pointcloud2_frame* messages, int32_t n_messages,
+                                           const int32_t* window_first, int32_t batch, const float* transform16,
+                                           const float* world_to_sensor16, const float* sensor_to_world16,
+                                           int8_t* grids, pcop_frame_result* out);
 
 /* Copies `bytes` from a device result array (PCOP_OUT_DEVICE) to host memory, or device to device when dst is a device
  * pointer; synchronous. */

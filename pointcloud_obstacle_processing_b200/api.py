@@ -55,6 +55,7 @@ EXPORTS = [
     "pcop_download",
     "pcop_process_batch_occupancy",
     "pcop_process_batch_pointcloud2",
+    "pcop_process_batch_pointcloud2_windows",
 ]
 
 
@@ -113,6 +114,8 @@ def load_library():
     L.pcop_process_batch_occupancy.argtypes = [vp, vp, C.c_size_t, vp, i32, vp, vp, vp, C.POINTER(FrameResult)]
     L.pcop_process_batch_pointcloud2.argtypes = [vp, C.POINTER(PointCloud2Frame), i32, vp, vp, vp, vp,
                                                  C.POINTER(FrameResult)]
+    L.pcop_process_batch_pointcloud2_windows.argtypes = [vp, C.POINTER(PointCloud2Frame), i32, vp, i32, vp, vp, vp, vp,
+                                                         C.POINTER(FrameResult)]
     L.pcop_enable_kernel_timing.argtypes = [vp, C.c_int]
     L.pcop_kernel_timing_count.argtypes = [vp]
     L.pcop_kernel_timing_get.argtypes = [vp, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_double),
@@ -139,6 +142,51 @@ def params_code_defaults() -> Params:
     p = Params()
     load_library().pcop_params_init_code_defaults(C.byref(p))
     return p
+
+
+def node_windows(n_messages: int, accumulate_count: int):
+    """The processing callbacks of the reference node over a stream of n_messages messages (od.cpp:690-701): with
+    K = accumulate_count, messages j(K+1) .. j(K+1)+K-1 are converted, transformed and appended, and message j(K+1)+K
+    runs the pipeline on them without being added itself.  A trailing window that never sees its trigger message is not
+    processed; K = 0 gives one empty frame per message.
+    Returns (window_first int32 [J + 1] over the kept messages, kept int64 [J K]: the stream index of every kept
+    message, triggers int64 [J]: the stream index of each window's trigger message, during which the node looks up the
+    grid TFs, od.cpp:592, 570, 634) -- window_first and the kept messages are what process_batch_pointcloud2_windows
+    takes."""
+    n, k = int(n_messages), int(accumulate_count)
+    if n < 0 or k < 0:
+        raise ValueError("n_messages and accumulate_count must be >= 0")
+    J = n // (k + 1)
+    starts = np.arange(J, dtype=np.int64) * (k + 1)
+    kept = (starts[:, None] + np.arange(k, dtype=np.int64)[None, :]).reshape(-1)
+    return np.arange(J + 1, dtype=np.int32) * k, kept, starts + k
+
+
+def _pc2_descriptors(messages):
+    """PointCloud2Message sequence -> (host buffers to keep alive, PointCloud2Frame list)"""
+    keep, frames = [], []
+    for m in messages:
+        m = PointCloud2Message(*m)
+        if m.data is None:
+            buf = np.zeros(0, np.uint8)
+        elif isinstance(m.data, np.ndarray):
+            buf = np.ascontiguousarray(m.data.reshape(-1)).view(np.uint8)
+        else:
+            buf = np.frombuffer(m.data, np.uint8)
+        keep.append(buf)
+        frames.append(PointCloud2Frame(buf.ctypes.data if buf.size else None, m.n_points, m.point_step, m.off_x,
+                                       m.off_y, m.off_z, 1 if m.is_dense else 0))
+    return keep, frames
+
+
+def _mats(m, count, what):
+    """[count, 4, 4] float32 matrices (or None) -> (array kept alive, pointer)"""
+    if m is None:
+        return None, None
+    m = np.ascontiguousarray(m, np.float32).reshape(-1, 16)
+    if m.shape[0] != count:
+        raise ValueError(f"one {what} matrix per {'message' if what == 'transform' else 'frame'} ({count})")
+    return m, m.ctypes.data_as(C.c_void_p)
 
 
 def _f32(a):
@@ -271,16 +319,8 @@ class ObstacleProcessor:
         call)."""
         B = len(frames)
         arr = (PointCloud2Frame * max(B, 1))(*frames)
-
-        def mats(m, what):
-            if m is None:
-                return None, None
-            m = np.ascontiguousarray(m, np.float32).reshape(-1, 16)
-            if m.shape[0] != B:
-                raise ValueError(f"one {what} matrix per message ({B})")
-            return m, m.ctypes.data_as(C.c_void_p)
-        (t, tp), (ws, wsp), (sw, swp) = mats(transforms, "transform"), mats(world_to_sensor, "world_to_sensor"), \
-            mats(sensor_to_world, "sensor_to_world")
+        (t, tp), (ws, wsp), (sw, swp) = _mats(transforms, B, "transform"), _mats(world_to_sensor, B, "world_to_sensor"), \
+            _mats(sensor_to_world, B, "sensor_to_world")
         res = (FrameResult * max(B, 1))()
         self._check(self._lib.pcop_process_batch_pointcloud2(
             self._h, arr, B, tp, wsp, swp, None if grids_ptr is None else C.c_void_p(grids_ptr), res))
@@ -295,24 +335,54 @@ class ObstacleProcessor:
         Pageable payloads and grids hold the host per copy; for throughput pass pinned or device memory to
         process_batch_pointcloud2_raw."""
         self._host_results_only()
-        keep, frames = [], []
-        for m in messages:
-            m = PointCloud2Message(*m)
-            if m.data is None:
-                buf = np.zeros(0, np.uint8)
-            elif isinstance(m.data, np.ndarray):
-                buf = np.ascontiguousarray(m.data.reshape(-1)).view(np.uint8)
-            else:
-                buf = np.frombuffer(m.data, np.uint8)
-            keep.append(buf)
-            frames.append(PointCloud2Frame(buf.ctypes.data if buf.size else None, m.n_points, m.point_step, m.off_x,
-                                           m.off_y, m.off_z, 1 if m.is_dense else 0))
+        keep, frames = _pc2_descriptors(messages)
         g = None
         if grids:
             w, h = self.occupancy_dims()
             g = np.empty((len(frames), h, w), np.int8)
         res = self.process_batch_pointcloud2_raw(frames, transforms, world_to_sensor, sensor_to_world,
                                                  None if g is None else g.ctypes.data)
+        out = [Frame.from_c(r) for r in res]
+        return (out, g) if grids else out
+
+    # ---- accumulation windows: several posed messages per frame (od.cpp:688-701 per processing callback) ----------
+    def process_batch_pointcloud2_windows_raw(self, messages, window_first, transforms=None, world_to_sensor=None,
+                                              sensor_to_world=None, grids_ptr=None):
+        """pcop_process_batch_pointcloud2_windows.  messages: a sequence of PointCloud2Frame (data = host or device
+        address); window_first: int [B + 1], frame f = messages window_first[f] .. window_first[f + 1] - 1 concatenated.
+        transforms: [n_messages, 4, 4] float32 or None; world_to_sensor / sensor_to_world: [B, 4, 4] float32 or None;
+        grids_ptr: raw host or device address of [B, H, W] int8, or None.  Returns the ctypes result array (valid until
+        the next call)."""
+        M = len(messages)
+        first = np.ascontiguousarray(window_first, np.int32).reshape(-1)
+        if first.size < 1:
+            raise ValueError("window_first needs batch + 1 entries")
+        B = first.size - 1
+        arr = (PointCloud2Frame * max(M, 1))(*messages)
+        (t, tp), (ws, wsp), (sw, swp) = _mats(transforms, M, "transform"), _mats(world_to_sensor, B, "world_to_sensor"), \
+            _mats(sensor_to_world, B, "sensor_to_world")
+        res = (FrameResult * max(B, 1))()
+        self._check(self._lib.pcop_process_batch_pointcloud2_windows(
+            self._h, arr, M, first.ctypes.data_as(C.c_void_p), B, tp, wsp, swp,
+            None if grids_ptr is None else C.c_void_p(grids_ptr), res))
+        return res[:B] if B else []
+
+    def process_batch_pointcloud2_windows(self, messages, window_first, transforms=None, world_to_sensor=None,
+                                          sensor_to_world=None, grids=False):
+        """messages: a sequence of PointCloud2Message (host payloads), one pose each in transforms ([n_messages, 4, 4]
+        float32 world <- sensor, or None).  Frame f is the world-frame concatenation of messages window_first[f] ..
+        window_first[f + 1] - 1 -- what the node accumulates before a processing callback (node_windows() builds
+        window_first for an accumulate_count), or the messages of several sensors at one time step.  Returns the list
+        of Frame, or (frames, grids int8 [B, H, W]) with grids=True (world_to_sensor / sensor_to_world: [B, 4, 4], one
+        pair per frame)."""
+        self._host_results_only()
+        keep, frames = _pc2_descriptors(messages)
+        g = None
+        if grids:
+            w, h = self.occupancy_dims()
+            g = np.empty((len(window_first) - 1, h, w), np.int8)
+        res = self.process_batch_pointcloud2_windows_raw(frames, window_first, transforms, world_to_sensor,
+                                                         sensor_to_world, None if g is None else g.ctypes.data)
         out = [Frame.from_c(r) for r in res]
         return (out, g) if grids else out
 

@@ -36,29 +36,8 @@ __device__ __forceinline__ float pc2_load_f32(const unsigned char* p) {
 __device__ __forceinline__ float pc2_lane(const float4& v, int k) {  // (compares, not an indexed register array)
   return k == 0 ? v.x : (k == 1 ? v.y : (k == 2 ? v.z : v.w));
 }
-// One decode per message (pcop_accumulate_pointcloud2 / pcop_pointcloud2_to_xyz: one frame; the batched PointCloud2
-// wave: one frame per message).  blockIdx.y = frame, records along x.  Every per-frame quantity comes from the
-// descriptor table in device memory.  aligned = 1 (point_step % 16 == 0, 16-byte aligned base, x / y / z inside one
-// aligned 16-byte word of the record): one 16-byte load per record instead of three 4-byte (or twelve 1-byte) loads.
-__global__ void __launch_bounds__(256)
-    k_pc2_ingest(const Pc2Frame* __restrict__ frames, float4* __restrict__ out, size_t out_stride) {
-  const int f = blockIdx.y;
-  const int n = frames[f].n;
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const Pc2Frame& d = frames[f];
-  const unsigned char* rec = d.data + (size_t)i * (size_t)d.point_step;
-  float x, y, z;
-  if (d.aligned) {
-    const float4 v = __ldg(reinterpret_cast<const float4*>(rec + (d.off_x & ~15)));
-    x = pc2_lane(v, (d.off_x & 15) >> 2);
-    y = pc2_lane(v, (d.off_y & 15) >> 2);
-    z = pc2_lane(v, (d.off_z & 15) >> 2);
-  } else {
-    x = pc2_load_f32(rec + d.off_x);
-    y = pc2_load_f32(rec + d.off_y);
-    z = pc2_load_f32(rec + d.off_z);
-  }
+// the decoded point of one record (PCL's transform coefficients in float, no FMA)
+__device__ __forceinline__ float4 pc2_point(const Pc2Frame& d, float x, float y, float z) {
   float4 o = make_float4(x, y, z, 1.0f);
   const bool finite = fabsf(x) <= 3.402823466e+38f && fabsf(y) <= 3.402823466e+38f && fabsf(z) <= 3.402823466e+38f;
   if (d.apply_transform && (d.is_dense || finite)) {
@@ -67,10 +46,56 @@ __global__ void __launch_bounds__(256)
     o.y = fadd(fadd(fadd(fmul(t.m[4], x), fmul(t.m[5], y)), fmul(t.m[6], z)), t.m[7]);
     o.z = fadd(fadd(fadd(fmul(t.m[8], x), fmul(t.m[9], y)), fmul(t.m[10], z)), t.m[11]);
   }
-  out[(size_t)f * out_stride + i] = o;
+  return o;
+}
+// Every decode of the library (pcop_accumulate_pointcloud2 / pcop_pointcloud2_to_xyz: one message; the batched
+// PointCloud2 wave: every message of its windows).  A 1-D grid over record tiles of PC2_TILE records: message m owns
+// tiles tile0 .. tile0 + cdiv(n, PC2_TILE) - 1 (empty messages own none), so a block finds its message by a binary
+// search over tile0, and a tile never spans two messages.  Record i of message m goes to out[dst + i].  aligned = 1
+// (point_step % 16 == 0, 16-byte aligned base, x / y / z inside one aligned 16-byte word of the record): one 16-byte
+// load per record instead of three 4-byte (or twelve 1-byte) loads; a thread issues the loads of its PC2_ITEMS records
+// before it stores.
+__global__ void __launch_bounds__(PC2_THREADS)
+    k_pc2_ingest(const Pc2Frame* __restrict__ msgs, int n_msgs, float4* __restrict__ out) {
+  const int tile = blockIdx.x;
+  int lo = 0, hi = n_msgs - 1;  // the last message whose first tile is <= tile
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (msgs[mid].tile0 <= tile) lo = mid;
+    else hi = mid - 1;
+  }
+  const Pc2Frame& d = msgs[lo];
+  const int base = (tile - d.tile0) * PC2_TILE;
+  const int n = d.n - base;  // (> 0)
+  const unsigned char* rec0 = d.data + (size_t)base * (size_t)d.point_step;
+  float4* o = out + d.dst + base;
+  if (d.aligned) {
+    const int word = d.off_x & ~15, kx = (d.off_x & 15) >> 2, ky = (d.off_y & 15) >> 2, kz = (d.off_z & 15) >> 2;
+    float4 v[PC2_ITEMS];
+#pragma unroll
+    for (int k = 0; k < PC2_ITEMS; ++k) {
+      const int i = k * PC2_THREADS + threadIdx.x;
+      if (i < n) v[k] = __ldg(reinterpret_cast<const float4*>(rec0 + (size_t)i * (size_t)d.point_step + word));
+    }
+#pragma unroll
+    for (int k = 0; k < PC2_ITEMS; ++k) {
+      const int i = k * PC2_THREADS + threadIdx.x;
+      if (i < n) o[i] = pc2_point(d, pc2_lane(v[k], kx), pc2_lane(v[k], ky), pc2_lane(v[k], kz));
+    }
+  } else {
+#pragma unroll
+    for (int k = 0; k < PC2_ITEMS; ++k) {
+      const int i = k * PC2_THREADS + threadIdx.x;
+      if (i < n) {
+        const unsigned char* rec = rec0 + (size_t)i * (size_t)d.point_step;
+        o[i] = pc2_point(d, pc2_load_f32(rec + d.off_x), pc2_load_f32(rec + d.off_y), pc2_load_f32(rec + d.off_z));
+      }
+    }
+  }
 }
 
-// the descriptor of one message whose payload sits at `src` on the device (validated by the caller)
+// the descriptor of one message whose payload sits at `src` on the device (validated by the caller); its place in the
+// launch (dst, tile0) is set by the caller
 Pc2Frame make_pc2_frame(const unsigned char* src, int n, int point_step, int ox, int oy, int oz, const float* t16,
                         int is_dense) {
   Pc2Frame d{};
@@ -466,31 +491,47 @@ int run_wave_cluster(Lane* l, int B, int max_n, const WaveRoute& r) {
 
 size_t pc2_payload_bytes(const pcop_pointcloud2_frame& m) { return (size_t)m.n_points * (size_t)m.point_step; }
 
-// PointCloud2 wave, input half: the descriptors go up through the pinned staging (the lane's previous wave no longer
-// reads it), every host payload into the lane's raw staging at a 256-byte aligned offset, device payloads are read in
-// place; one k_pc2_ingest launch decodes (and transforms) every message into d_in.  A repeat of the wave (voxel
-// decline) decodes again from the same staging -- the plane stage has overwritten d_in, the staging is intact.
+// PointCloud2 wave, input half: the descriptors of every message of the wave's windows go up through the pinned staging
+// (the lane's previous wave no longer reads it), every host payload into the lane's raw staging at a 256-byte aligned
+// offset, device payloads are read in place; one k_pc2_ingest launch decodes (and transforms) every message into its
+// frame's slot of d_in, after the messages before it in its window.  A repeat of the wave (voxel decline) decodes again
+// from the same staging -- the plane stage has overwritten d_in, the staging is intact.
 int enqueue_wave_decode(Lane* l, const Pc2Call& pc, int w0, int B, int max_n, bool repeat) {
   pcop_handle* h = l->h;
   if (!repeat) {
+    const int m0 = pc.window_first[w0];
     size_t off = 0;
+    int tiles = 0;
     for (int f = 0; f < B; ++f) {
-      const pcop_pointcloud2_frame& m = pc.frames[w0 + f];
-      const size_t bytes = pc2_payload_bytes(m);
-      const unsigned char* src = m.data;
-      if (bytes > 0 && !pc.on_device[w0 + f]) {
-        PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_raw + off, m.data, bytes, cudaMemcpyHostToDevice, l->stream));
-        src = l->d_raw + off;
-        off += (bytes + 255) & ~(size_t)255;
+      size_t dst = (size_t)f * (size_t)h->cap;
+      for (int k = pc.window_first[w0 + f]; k < pc.window_first[w0 + f + 1]; ++k) {
+        const pcop_pointcloud2_frame& m = pc.msgs[k];
+        const size_t bytes = pc2_payload_bytes(m);
+        const unsigned char* src = m.data;
+        if (bytes > 0 && !pc.on_device[k]) {
+          PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_raw + off, m.data, bytes, cudaMemcpyHostToDevice, l->stream));
+          src = l->d_raw + off;
+          off += (bytes + 255) & ~(size_t)255;
+        }
+        Pc2Frame& d = l->h_pc2[k - m0];
+        d = make_pc2_frame(src, m.n_points, m.point_step, m.off_x, m.off_y, m.off_z,
+                           pc.transform16 ? pc.transform16 + (size_t)k * 16 : nullptr, m.is_dense);
+        d.dst = dst;
+        d.tile0 = tiles;
+        dst += (size_t)m.n_points;
+        tiles += cdiv(m.n_points, PC2_TILE);
       }
-      l->h_pc2[f] = make_pc2_frame(src, m.n_points, m.point_step, m.off_x, m.off_y, m.off_z,
-                                   pc.transform16 ? pc.transform16 + (size_t)(w0 + f) * 16 : nullptr, m.is_dense);
     }
-    PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_pc2, l->h_pc2, sizeof(Pc2Frame) * B, cudaMemcpyHostToDevice, l->stream));
+    l->pc2_msgs = pc.window_first[w0 + B] - m0;
+    l->pc2_tiles = tiles;
+    if (l->pc2_msgs > 0)
+      PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_pc2, l->h_pc2, sizeof(Pc2Frame) * l->pc2_msgs, cudaMemcpyHostToDevice, l->stream));
   }
-  Ctx c = make_ctx(l, B, max_n);
-  KL(c, "k_pc2_ingest", k_pc2_ingest<<<dim3(cdiv(max_n, 256), B), 256, 0, l->stream>>>(l->d_pc2, l->d_in, (size_t)h->cap));
-  count_launch(c);
+  if (l->pc2_tiles > 0) {  // (a wave of empty windows decodes nothing)
+    Ctx c = make_ctx(l, B, max_n);
+    KL(c, "k_pc2_ingest", k_pc2_ingest<<<l->pc2_tiles, PC2_THREADS, 0, l->stream>>>(l->d_pc2, l->pc2_msgs, l->d_in));
+    count_launch(c);
+  }
   return PCOP_OK;
 }
 
@@ -819,7 +860,9 @@ int finish_wave(Lane* l, const WaveInput& wi, uint32_t mask, pcop_frame_result* 
     // algorithmic bytes (SURVEY 8d)
     double b = 0.0;
     const pcop_params& p = h->params;
-    if (wi.pc2) b += (double)(wi.pc2->frames[w0 + f].point_step + 16) * r.n_input;  // the decode: payload in, PointXYZ out
+    if (wi.pc2)  // the decode: every message's payload in, PointXYZ out
+      for (int k = wi.pc2->window_first[w0 + f]; k < wi.pc2->window_first[w0 + f + 1]; ++k)
+        b += (double)(wi.pc2->msgs[k].point_step + 16) * wi.pc2->msgs[k].n_points;
     if (p.enable_crop) b += 16.0 * r.n_input + 20.0 * r.n_crop;
     if (p.enable_voxel) b += 16.0 * r.n_crop + 20.0 * r.n_voxel;
     if (p.enable_sor) b += 16.0 * r.n_voxel + 20.0 * r.n_sor;
@@ -917,13 +960,16 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
       w0 += B;
     }
   }
-  size_t raw_need = 0;  // PointCloud2 messages: host payload bytes of the largest wave, as staged (256-byte aligned)
+  // PointCloud2 messages: host payload bytes of the largest wave, as staged (256-byte aligned), and its message count
+  size_t raw_need = 0, pc2_need = 0;
   if (pc2)
     for (const auto& w : waves) {
       size_t bytes = 0;
-      for (int f = w.first; f < w.first + w.second; ++f)
-        if (!pc2->on_device[f]) bytes += (pc2_payload_bytes(pc2->frames[f]) + 255) & ~(size_t)255;
+      const int m0 = pc2->window_first[w.first], m1 = pc2->window_first[w.first + w.second];
+      for (int k = m0; k < m1; ++k)
+        if (!pc2->on_device[k]) bytes += (pc2_payload_bytes(pc2->msgs[k]) + 255) & ~(size_t)255;
       raw_need = std::max(raw_need, bytes);
+      pc2_need = std::max(pc2_need, (size_t)(m1 - m0));
     }
   h->launches = 0;
   h->alg_bytes = 0.0;
@@ -934,6 +980,7 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
   for (Lane* l : lanes) {
     if (occ && !waves.empty()) TRY(ensure_occ_scratch(l, (size_t)waves[0].second, (size_t)occ->g.cells));  // (the first wave is the largest)
     if (raw_need) TRY(ensure_raw(l, raw_need));
+    if (pc2_need) TRY(ensure_pc2(l, pc2_need));
     l->h_pack_used = 0;
     l->h_pack_sel ^= 1;
     l->h_pack = l->h_pack_buf[l->h_pack_sel];
@@ -1026,11 +1073,12 @@ int pc2_ingest(pcop_handle* h, const unsigned char* data, int32_t n, int32_t poi
     PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_raw, data, bytes, cudaMemcpyHostToDevice, l->stream));
     src = l->d_raw;
   }
-  // the batched decode with one frame; the descriptor goes up from pageable memory (staged before the call returns)
-  const Pc2Frame d = make_pc2_frame(src, n, point_step, ox, oy, oz, t16, is_dense);
+  // the batched decode with one message; the descriptor goes up from pageable memory (staged before the call returns)
+  TRY(ensure_pc2(l, 1));
+  const Pc2Frame d = make_pc2_frame(src, n, point_step, ox, oy, oz, t16, is_dense);  // (dst = 0, tile0 = 0)
   PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_pc2, &d, sizeof(d), cudaMemcpyHostToDevice, l->stream));
   Ctx c = make_ctx(l, 1, n);
-  KL(c, "k_pc2_ingest", k_pc2_ingest<<<dim3(cdiv(n, 256), 1), 256, 0, l->stream>>>(l->d_pc2, dst, (size_t)0));
+  KL(c, "k_pc2_ingest", k_pc2_ingest<<<cdiv(n, PC2_TILE), PC2_THREADS, 0, l->stream>>>(l->d_pc2, 1, dst));
   count_launch(c);
   if (src != data) PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));  // the caller may reuse its buffer
   return PCOP_OK;

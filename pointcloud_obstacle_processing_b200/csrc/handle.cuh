@@ -6,6 +6,8 @@
 #include <string>
 #include <vector>
 
+#include <cuda.h>  // (types of cuPointerGetAttributes only; see PayloadClassifier)
+
 #include "internal.cuh"
 
 namespace pcop {
@@ -63,10 +65,13 @@ struct PackMeta {  // device -> host in one copy
 
 struct Pc2Frame {  // decode descriptor of one PointCloud2 message (device memory, read by k_pc2_ingest)
   const unsigned char* data;  // payload on the device
+  size_t dst;                 // element offset of the message's first decoded point in the output
   int n, point_step, off_x, off_y, off_z;
   int is_dense, apply_transform, aligned;
+  int tile0;                  // the message's first record tile (PC2_TILE records each) in the launch
   Mat34 t;
 };
+constexpr int PC2_THREADS = 256, PC2_ITEMS = 4, PC2_TILE = PC2_THREADS * PC2_ITEMS;  // k_pc2_ingest
 
 // the grid product of a batched call (pcop_process_batch_occupancy, pcop_process_batch_pointcloud2 with grids)
 struct OccCall {
@@ -77,10 +82,11 @@ struct OccCall {
   bool grids_on_device;
 };
 
-// the messages of a pcop_process_batch_pointcloud2 call
+// the messages of a pcop_process_batch_pointcloud2_windows call
 struct Pc2Call {
-  const pcop_pointcloud2_frame* frames;
-  const float* transform16;       // [batch][16] or nullptr
+  const pcop_pointcloud2_frame* msgs;
+  const int32_t* window_first;    // [batch + 1]: frame f = messages window_first[f] .. window_first[f + 1] - 1
+  const float* transform16;       // [messages][16] or nullptr
   std::vector<char> on_device;    // per message: the payload is a device pointer (used in place)
 };
 
@@ -188,8 +194,10 @@ struct Lane {
   cudaEvent_t ev_grids_copied = nullptr;  // the last copy out of d_occ_grids
   unsigned char* d_raw = nullptr;  // staging of raw PointCloud2 payloads from host memory: one message, or the host
   size_t raw_cap = 0;              // messages of one wave at 256-byte aligned offsets (grown on demand)
-  Pc2Frame* d_pc2 = nullptr;       // [maxB] decode descriptors of k_pc2_ingest
-  Pc2Frame* h_pc2 = nullptr;       // [maxB] pinned staging of the same (the batched PointCloud2 wave)
+  Pc2Frame* d_pc2 = nullptr;       // decode descriptors of k_pc2_ingest: one per message of a wave
+  Pc2Frame* h_pc2 = nullptr;       // pinned staging of the same (the batched PointCloud2 wave)
+  size_t pc2_cap = 0;              // descriptors the two hold (grown on demand, never shrunk)
+  int pc2_msgs = 0, pc2_tiles = 0; // messages and record tiles of the wave in flight (a repeat decodes them again)
 
   // pinned host
   int* h_counts = nullptr;  // [CNT_ROWS][maxB]
@@ -321,6 +329,22 @@ inline int ensure_raw(Lane* l, size_t bytes) {
   return PCOP_OK;
 }
 
+// the PointCloud2 decode descriptors of lane l hold at least `msgs` messages (grown, never shrunk)
+inline int ensure_pc2(Lane* l, size_t msgs) {
+  pcop_handle* h = l->h;
+  if (msgs <= l->pc2_cap) return PCOP_OK;
+  PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
+  cudaFree(l->d_pc2);  // (not tracked in dev_allocs / host_allocs)
+  if (l->h_pc2) cudaFreeHost(l->h_pc2);
+  l->d_pc2 = nullptr;
+  l->h_pc2 = nullptr;
+  l->pc2_cap = 0;
+  PCOP_CUDA_TRY(cudaMalloc((void**)&l->d_pc2, sizeof(Pc2Frame) * msgs));
+  PCOP_CUDA_TRY(cudaHostAlloc((void**)&l->h_pc2, sizeof(Pc2Frame) * msgs, cudaHostAllocDefault));
+  l->pc2_cap = msgs;
+  return PCOP_OK;
+}
+
 inline bool is_device_pointer(const void* p) {
   cudaPointerAttributes at;
   if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
@@ -329,6 +353,50 @@ inline bool is_device_pointer(const void* p) {
   }
   return at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged;
 }
+
+// is_device_pointer for the many payloads of one call, one driver query per allocation: the query also returns the
+// allocation's address range, and a later pointer inside the last range takes that range's answer.  Memory the driver
+// does not know (pageable host memory) has no range and is queried per pointer.  (cuPointerGetAttributes comes through
+// cudaGetDriverEntryPoint: the library links the runtime only.)  Valid within one call: allocations may change between calls.
+struct PayloadClassifier {
+  uintptr_t lo = 0, hi = 0;
+  bool dev = false;
+
+  using GetAttributes = CUresult (*)(unsigned, CUpointer_attribute*, void**, CUdeviceptr);
+  static GetAttributes entry() {
+    static const GetAttributes fn = [] {
+      void* f = nullptr;
+      cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+      if (cudaGetDriverEntryPoint("cuPointerGetAttributes", &f, cudaEnableDefault, &q) != cudaSuccess ||
+          q != cudaDriverEntryPointSuccess) {
+        cudaGetLastError();
+        f = nullptr;
+      }
+      return reinterpret_cast<GetAttributes>(f);
+    }();
+    return fn;
+  }
+
+  bool operator()(const void* p) {
+    const uintptr_t a = reinterpret_cast<uintptr_t>(p);
+    if (a >= lo && a < hi) return dev;
+    const GetAttributes fn = entry();
+    unsigned type = 0, managed = 0;
+    CUdeviceptr start = 0;
+    size_t size = 0;
+    CUpointer_attribute at[4] = {CU_POINTER_ATTRIBUTE_MEMORY_TYPE, CU_POINTER_ATTRIBUTE_IS_MANAGED,
+                                 CU_POINTER_ATTRIBUTE_RANGE_START_ADDR, CU_POINTER_ATTRIBUTE_RANGE_SIZE};
+    void* data[4] = {&type, &managed, &start, &size};
+    if (!fn || fn(4, at, data, (CUdeviceptr)a) != CUDA_SUCCESS) return is_device_pointer(p);
+    const bool d = type == CU_MEMORYTYPE_DEVICE || type == CU_MEMORYTYPE_UNIFIED || managed != 0;
+    if (size > 0 && a >= (uintptr_t)start && a - (uintptr_t)start < size) {
+      lo = (uintptr_t)start;
+      hi = (uintptr_t)start + size;
+      dev = d;
+    }
+    return d;
+  }
+};
 
 inline bool pc2_layout_ok(int point_step, int ox, int oy, int oz) {
   return point_step >= 4 && ox >= 0 && oy >= 0 && oz >= 0 && ox <= point_step - 4 && oy <= point_step - 4 &&

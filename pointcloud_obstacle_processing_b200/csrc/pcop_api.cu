@@ -240,8 +240,6 @@ int init_lane(Lane* l) {
   TRY(dalloc(h, &l->d_pack_off, (size_t)PK_N * B));
   TRY(dalloc(h, &l->d_meta, 1));
   TRY(dalloc(h, &l->d_pack_cursor, 1));
-  TRY(dalloc(h, &l->d_pc2, B));
-  TRY(halloc(h, &l->h_pc2, B));
   TRY(halloc(h, &l->h_counts, (size_t)CNT_ROWS * B));
   TRY(halloc(h, &l->h_warnings, B));
   TRY(halloc(h, &l->h_prec, B));
@@ -312,6 +310,8 @@ pcop::Lane::~Lane() {
   cudaFree(d_occ_grids);
   cudaFree(d_vp_grec);
   cudaFree(d_vp_desc);
+  cudaFree(d_pc2);
+  if (h_pc2) cudaFreeHost(h_pc2);
   for (int i = 0; i < 2; ++i)
     if (h_pack_buf[i]) cudaFreeHost(h_pack_buf[i]);
   for (cudaEvent_t e : {ev_lane_done, ev_copied, ev_meta, ev_grids_copied})
@@ -518,34 +518,70 @@ int pcop_process_batch_occupancy(pcop_handle* h, const float* xyzw, size_t frame
   return st;
 }
 
+// pcop_process_batch_pointcloud2_windows, and pcop_process_batch_pointcloud2 with one message per window (`who` names
+// the entry point in error messages)
+static int pointcloud2_windows(pcop_handle* h, const char* who, const pcop_pointcloud2_frame* msgs, int32_t n_msgs,
+                               const int32_t* window_first, int32_t batch, const float* transform16,
+                               const float* world_to_sensor16, const float* sensor_to_world16, int8_t* grids,
+                               pcop_frame_result* out) {
+  const std::string w(who);
+  if (!out || batch < 0 || n_msgs < 0 || (!msgs && n_msgs > 0) || (!window_first && (batch > 0 || n_msgs > 0)) ||
+      (grids && (!world_to_sensor16 || !sensor_to_world16)))
+    return fail(h, PCOP_ERR_BAD_PARAM, w + ": null argument (grids need world_to_sensor16 and sensor_to_world16)");
+  if (window_first && (window_first[0] != 0 || window_first[batch] != n_msgs))
+    return fail(h, PCOP_ERR_BAD_PARAM, w + ": window_first must start at 0 and end at the message count");
+  for (int f = 0; f < batch; ++f)  // (then every window lies inside [0, n_msgs))
+    if (window_first[f + 1] < window_first[f])
+      return fail(h, PCOP_ERR_BAD_PARAM, w + ": window_first decreases at window " + std::to_string(f));
+  // window by window, message by message: with one message per window the checks run in the order of
+  // pcop_process_batch_pointcloud2's per-frame checks
+  std::vector<int32_t> n((size_t)batch + 1, 0);  // frame f = the concatenation of its window's messages
+  for (int f = 0; f < batch; ++f) {
+    long long total = 0;
+    for (int m = window_first[f]; m < window_first[f + 1]; ++m) {
+      const pcop_pointcloud2_frame& d = msgs[m];
+      if (d.n_points < 0 || (!d.data && d.n_points > 0))
+        return fail(h, PCOP_ERR_BAD_PARAM, w + ": message " + std::to_string(m) + ": bad count or NULL data");
+      if (!pc2_layout_ok(d.point_step, d.off_x, d.off_y, d.off_z))
+        return fail(h, PCOP_ERR_BAD_PARAM,
+                    w + ": message " + std::to_string(m) + ": PointCloud2 field offsets do not fit point_step");
+      total += d.n_points;
+    }
+    if (total > h->cap)
+      return fail(h, PCOP_ERR_CAPACITY, w + ": window " + std::to_string(f) + " holds " + std::to_string(total) +
+                                            " points, more than max_points");
+    n[f] = (int32_t)total;
+  }
+  OccCall oc{};
+  if (grids) TRY(occ_call_of(h, who, world_to_sensor16, sensor_to_world16, grids, &oc));
+  PCOP_CUDA_TRY(cudaSetDevice(h->device));
+  Pc2Call pc;
+  pc.msgs = msgs;
+  pc.window_first = window_first;
+  pc.transform16 = transform16;
+  pc.on_device.resize((size_t)n_msgs);
+  PayloadClassifier on_device;
+  for (int m = 0; m < n_msgs; ++m) pc.on_device[m] = msgs[m].n_points > 0 && on_device(msgs[m].data);
+  return process_impl(h, nullptr, (size_t)h->cap, n.data(), batch, out, grids ? &oc : nullptr, &pc);
+}
+
+int pcop_process_batch_pointcloud2_windows(pcop_handle* h, const pcop_pointcloud2_frame* messages, int32_t n_messages,
+                                           const int32_t* window_first, int32_t batch, const float* transform16,
+                                           const float* world_to_sensor16, const float* sensor_to_world16,
+                                           int8_t* grids, pcop_frame_result* out) {
+  if (!h) return fail(nullptr, PCOP_ERR_BAD_PARAM, "null handle");
+  return pointcloud2_windows(h, "pcop_process_batch_pointcloud2_windows", messages, n_messages, window_first, batch,
+                             transform16, world_to_sensor16, sensor_to_world16, grids, out);
+}
+
 int pcop_process_batch_pointcloud2(pcop_handle* h, const pcop_pointcloud2_frame* frames, int32_t batch,
                                    const float* transform16, const float* world_to_sensor16,
                                    const float* sensor_to_world16, int8_t* grids, pcop_frame_result* out) {
   if (!h) return fail(nullptr, PCOP_ERR_BAD_PARAM, "null handle");
-  if (!out || batch < 0 || (!frames && batch > 0) || (grids && (!world_to_sensor16 || !sensor_to_world16)))
-    return fail(h, PCOP_ERR_BAD_PARAM,
-                "pcop_process_batch_pointcloud2: null argument (grids need world_to_sensor16 and sensor_to_world16)");
-  Pc2Call pc;
-  pc.frames = frames;
-  pc.transform16 = transform16;
-  std::vector<int32_t> n((size_t)batch + 1, 0);
-  for (int f = 0; f < batch; ++f) {
-    const pcop_pointcloud2_frame& m = frames[f];
-    if (m.n_points < 0 || (!m.data && m.n_points > 0))
-      return fail(h, PCOP_ERR_BAD_PARAM, "pcop_process_batch_pointcloud2: frame " + std::to_string(f) + ": bad count or NULL data");
-    if (!pc2_layout_ok(m.point_step, m.off_x, m.off_y, m.off_z))
-      return fail(h, PCOP_ERR_BAD_PARAM,
-                  "pcop_process_batch_pointcloud2: frame " + std::to_string(f) + ": PointCloud2 field offsets do not fit point_step");
-    if (m.n_points > h->cap)
-      return fail(h, PCOP_ERR_CAPACITY, "pcop_process_batch_pointcloud2: frame " + std::to_string(f) + " has more points than max_points");
-    n[f] = m.n_points;
-  }
-  OccCall oc{};
-  if (grids) TRY(occ_call_of(h, "pcop_process_batch_pointcloud2", world_to_sensor16, sensor_to_world16, grids, &oc));
-  PCOP_CUDA_TRY(cudaSetDevice(h->device));
-  pc.on_device.resize((size_t)batch);
-  for (int f = 0; f < batch; ++f) pc.on_device[f] = frames[f].n_points > 0 && is_device_pointer(frames[f].data);
-  return process_impl(h, nullptr, (size_t)h->cap, n.data(), batch, out, grids ? &oc : nullptr, &pc);
+  std::vector<int32_t> first((size_t)std::max(batch, 0) + 1);
+  for (size_t f = 0; f < first.size(); ++f) first[f] = (int32_t)f;
+  return pointcloud2_windows(h, "pcop_process_batch_pointcloud2", frames, batch, first.data(), batch, transform16,
+                             world_to_sensor16, sensor_to_world16, grids, out);
 }
 
 int pcop_enable_kernel_timing(pcop_handle* h, int enable) {
