@@ -8,8 +8,9 @@
 // its payload copy with the exact size and refills the lane, so a wave's result copy and the host's
 // bookkeeping overlap the other lanes' kernels.  Requested outputs of all frames of a wave are packed
 // on the device into one contiguous buffer and come back in a single device->host copy.
-// Every buffer is allocated by pcop_create; the pinned result buffer only grows (a second call of the
-// same shape allocates nothing).
+// The wave buffers belong to the lanes (handle.cuh).  A call first grows the buffers its shape needs (grid scratch,
+// PointCloud2 staging and descriptors, pack buffer); the pinned result buffer grows while the call runs.  Neither
+// shrinks, so a second call of the same shape allocates nothing.
 #include <chrono>
 #include <cstdio>
 
@@ -275,22 +276,17 @@ void resolve_kernel_timers(pcop_handle* h) {
   k.used = 0;
 }
 
+// The pinned result buffer of the running call holds at least `need` bytes.  Unlike grow() it keeps its contents: the
+// call's earlier waves are in it.
 int ensure_host_pack(Lane* l, size_t need) {
-  if (need <= l->h_pack_cap) return PCOP_OK;
-  size_t ncap = std::max<size_t>(need, l->h_pack_cap * 2);
-  ncap = std::max<size_t>(ncap, 1 << 20);
-  unsigned char* q = nullptr;
-  cudaError_t e = cudaHostAlloc((void**)&q, ncap, cudaHostAllocMapped);
-  if (e != cudaSuccess) return fail_cuda(l->h, e, "cudaHostAlloc(pack)", __FILE__, __LINE__);
-  if (l->cstream) cudaStreamSynchronize(l->cstream);  // copies into the old buffer must have landed
-  if (l->h_pack) {
-    memcpy(q, l->h_pack, l->h_pack_cap);
-    cudaFreeHost(l->h_pack);
-  }
-  l->h_pack = q;
-  l->h_pack_cap = ncap;
-  l->h_pack_buf[l->h_pack_sel] = q;
-  l->h_pack_buf_cap[l->h_pack_sel] = ncap;
+  HostBuffer<unsigned char>& b = l->h_pack();
+  if (need <= b.size()) return PCOP_OK;
+  HostBuffer<unsigned char> q;
+  const cudaError_t e = q.allocate(std::max<size_t>({need, b.size() * 2, 1 << 20}));
+  if (e != cudaSuccess) return fail_cuda(l->h, e, "cudaHostAlloc: pinned result buffer", __FILE__, __LINE__);
+  cudaStreamSynchronize(l->cstream);  // copies into the old buffer must have landed
+  if (b.size()) memcpy(q, b, b.size());
+  b = std::move(q);
   return PCOP_OK;
 }
 
@@ -372,7 +368,7 @@ int run_wave_stages(Lane* l, int B, const float4* in, size_t stride, int max_n, 
     a.group_stride = l->vp_gstride;
     a.group_launch = r.vox_groups;
     a.flags = l->d_vf_flags;
-    a.warnings = (effective_outputs(p) & PCOP_OUT_CROP) ? nullptr : l->d_warnings;  // zeroed by k_vp_init
+    a.warnings = (effective_outputs(p) & PCOP_OUT_CROP) ? nullptr : l->d_warnings.get();  // zeroed by k_vp_init
     a.n_crop = l->cnt(CNT_CROP);
     a.out = l->d_vox;
     a.out_keys = l->d_vox_keys;
@@ -403,7 +399,7 @@ int run_wave_stages(Lane* l, int B, const float4* in, size_t stride, int max_n, 
     a.pair[1] = l->d_vf_pair[1];
     a.desc = l->d_desc;
     a.flags = l->d_vf_flags;
-    a.warnings = (effective_outputs(p) & PCOP_OUT_CROP) ? nullptr : l->d_warnings;  // zeroed by k_vf_init
+    a.warnings = (effective_outputs(p) & PCOP_OUT_CROP) ? nullptr : l->d_warnings.get();  // zeroed by k_vf_init
     a.n_crop = l->cnt(CNT_CROP);
     a.out = l->d_vox;
     a.out_keys = l->d_vox_keys;
@@ -545,8 +541,8 @@ int enqueue_wave_pack(Lane* l, int B, int max_n, uint32_t mask, const WaveRoute&
   const bool dev_results = (mask & PCOP_OUT_DEVICE) != 0;  // the arrays stay in d_pack (bump-allocated over the call)
   if (!dev_results && l->wave_seq >= 1) PCOP_CUDA_TRY(cudaStreamWaitEvent(l->stream, l->ev_copied, 0));  // d_pack is free again
   KL(c, "k_pack_scan", k_pack_scan<<<1, 320, 0, l->stream>>>(l->d_counts, h->maxB, B, mask, l->d_pack_off, l->d_meta, l->d_pf, l->d_prec,
-                                             h->params.enable_plane ? 1 : 0, dev_results ? l->d_pack_cursor : nullptr,
-                                             (unsigned long long)l->pack_cap));
+                                             h->params.enable_plane ? 1 : 0, dev_results ? l->d_pack_cursor.get() : nullptr,
+                                             (unsigned long long)l->d_pack.size()));
   count_launch(c);
   const void* srcs[PK_N] = {l->d_crop_kept, l->d_vox_keys, l->d_vox,     l->d_sor_kept, l->d_inliers,
                             l->d_rem,       l->d_rem_src,  l->d_offsets, l->d_indices,  l->d_obst};
@@ -781,7 +777,7 @@ int finish_wave(Lane* l, const WaveInput& wi, uint32_t mask, pcop_frame_result* 
   if (!dev_results) {
     // (when the buffer has to grow, grow it for all the waves this lane will see in the call: a pinned allocation
     // costs ~0.4 ms per MB, and every regrowth copies what is already there)
-    if (base_off + meta.total_bytes + 256 > l->h_pack_cap)
+    if (base_off + meta.total_bytes + 256 > l->h_pack().size())
       TRY(ensure_host_pack(l, base_off + (size_t)((double)(meta.total_bytes + 256) * 1.1 * std::max(1, l->call_lane_waves - l->wave_seq))));
     // payload copy on the copy stream (the pack kernels have finished: ev_meta follows them), in pieces: one large
     // device-to-host copy holds up the kernels of the other lanes for as long as it runs (measured: 6.4 ms per
@@ -789,7 +785,7 @@ int finish_wave(Lane* l, const WaveInput& wi, uint32_t mask, pcop_frame_result* 
     // 6.3 ms with 256 KB pieces -- the host thread becomes the limit -- and 5.3 ms with no copy at all)
     const size_t piece = (size_t)1 << 20;
     for (size_t o = 0; o < meta.total_bytes; o += piece)
-      PCOP_CUDA_TRY(cudaMemcpyAsync(l->h_pack + base_off + o, l->d_pack + o, std::min<size_t>(piece, meta.total_bytes - o),
+      PCOP_CUDA_TRY(cudaMemcpyAsync(l->h_pack() + base_off + o, l->d_pack + o, std::min<size_t>(piece, meta.total_bytes - o),
                                     cudaMemcpyDeviceToHost, l->cstream));
     PCOP_CUDA_TRY(cudaEventRecord(l->ev_copied, l->cstream));
     l->h_pack_used = base_off + meta.total_bytes;
@@ -797,7 +793,7 @@ int finish_wave(Lane* l, const WaveInput& wi, uint32_t mask, pcop_frame_result* 
   if (wi.occ) {  // the wave's grids, after its last repeat, on the copy stream beside the payload
     const size_t bytes = (size_t)B * (size_t)wi.occ->g.cells;
     int8_t* dst = wi.occ->grids + (size_t)w0 * (size_t)wi.occ->g.cells;
-    const unsigned char* src = reinterpret_cast<const unsigned char*>(l->d_occ_grids);
+    const unsigned char* src = reinterpret_cast<const unsigned char*>(l->d_occ_grids.get());
     if (wi.occ->grids_on_device) {
       PCOP_CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, l->cstream));
     } else {
@@ -896,28 +892,6 @@ static double trace_host_us() {
   return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - g_trace_t0).count();
 }
 
-// occupancy grid scratch of one lane for waves of `frames` frames of `cells` cells (grown, never shrunk)
-int ensure_occ_scratch(Lane* l, size_t frames, size_t cells) {
-  pcop_handle* h = l->h;
-  if (!l->d_occ_mats) {
-    TRY(dalloc(h, &l->d_occ_mats, 2 * (size_t)h->maxB));
-    TRY(halloc(h, &l->h_occ_mats, 2 * (size_t)h->maxB));
-  }
-  const size_t need = frames * cells;
-  if (need <= l->occ_scratch_cells) return PCOP_OK;
-  PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
-  PCOP_CUDA_TRY(cudaStreamSynchronize(l->cstream));
-  if (l->d_occ_counts) cudaFree(l->d_occ_counts);  // (not tracked in dev_allocs)
-  if (l->d_occ_grids) cudaFree(l->d_occ_grids);
-  l->d_occ_counts = nullptr;
-  l->d_occ_grids = nullptr;
-  l->occ_scratch_cells = 0;
-  PCOP_CUDA_TRY(cudaMalloc((void**)&l->d_occ_counts, sizeof(int) * need));
-  PCOP_CUDA_TRY(cudaMalloc((void**)&l->d_occ_grids, need));
-  l->occ_scratch_cells = need;
-  return PCOP_OK;
-}
-
 }  // namespace
 
 namespace pcop {
@@ -978,19 +952,24 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
   h->sort_pass_keys = 0;
   for (int s = 0; s < PCOP_N_STAGES; ++s) h->stage_us[s] = 0.f;
   for (Lane* l : lanes) {
-    if (occ && !waves.empty()) TRY(ensure_occ_scratch(l, (size_t)waves[0].second, (size_t)occ->g.cells));  // (the first wave is the largest)
-    if (raw_need) TRY(ensure_raw(l, raw_need));
-    if (pc2_need) TRY(ensure_pc2(l, pc2_need));
+    if (occ && !waves.empty()) {  // (the first wave is the largest)
+      const size_t cells = (size_t)waves[0].second * (size_t)occ->g.cells;
+      TRY(grow(l, l->d_occ_mats, 2 * (size_t)h->maxB));
+      TRY(grow(l, l->h_occ_mats, 2 * (size_t)h->maxB));
+      TRY(grow(l, l->d_occ_counts, cells));
+      TRY(grow(l, l->d_occ_grids, cells));
+    }
+    TRY(grow_raw(l, raw_need));
+    TRY(grow(l, l->d_pc2, pc2_need));
+    TRY(grow(l, l->h_pc2, pc2_need));
     l->h_pack_used = 0;
     l->h_pack_sel ^= 1;
-    l->h_pack = l->h_pack_buf[l->h_pack_sel];
-    l->h_pack_cap = l->h_pack_buf_cap[l->h_pack_sel];
     l->fixups.clear();
     l->wave_seq = 0;
     l->call_lane_waves = cdiv((int)waves.size(), (int)lanes.size());
     l->trace_used = 0;
     l->pending = false;
-    TRY(ensure_pack_capacity(l, mask));
+    TRY(grow(l, l->d_pack, pack_capacity_bytes(mask, h->maxB, h->cap)));
   }
   PCOP_CUDA_TRY(cudaEventRecord(h->ev_call[0], lanes[0]->stream));
   if (h->trace) g_trace_t0 = std::chrono::steady_clock::now();
@@ -1056,7 +1035,7 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
     for (size_t fx : l->fixups) {
       const void** slot = (const void**)((unsigned char*)out + fx);
       const size_t off = (size_t)(uintptr_t)(*slot) - 1;
-      *slot = l->h_pack + off;
+      *slot = l->h_pack() + off;
     }
   }
   return PCOP_OK;
@@ -1069,12 +1048,12 @@ int pc2_ingest(pcop_handle* h, const unsigned char* data, int32_t n, int32_t poi
   const size_t bytes = (size_t)n * (size_t)point_step;
   const unsigned char* src = data;
   if (!is_device_pointer(data)) {
-    TRY(ensure_raw(l, bytes));
+    TRY(grow_raw(l, bytes));
     PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_raw, data, bytes, cudaMemcpyHostToDevice, l->stream));
     src = l->d_raw;
   }
   // the batched decode with one message; the descriptor goes up from pageable memory (staged before the call returns)
-  TRY(ensure_pc2(l, 1));
+  TRY(grow(l, l->d_pc2, 1));
   const Pc2Frame d = make_pc2_frame(src, n, point_step, ox, oy, oz, t16, is_dense);  // (dst = 0, tile0 = 0)
   PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_pc2, &d, sizeof(d), cudaMemcpyHostToDevice, l->stream));
   Ctx c = make_ctx(l, 1, n);

@@ -1,9 +1,11 @@
 // The handle and its lanes (pcop_api.cu, batch.cu).  The handle holds the parameters, knobs, per-call counters and error
 // text once; a lane holds what one wave in flight needs and reaches the parameters through its handle.
 #pragma once
+#include <algorithm>
 #include <cmath>
 #include <memory>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include <cuda.h>  // (types of cuPointerGetAttributes only; see PayloadClassifier)
@@ -112,6 +114,67 @@ struct WaveRoute {
 constexpr int PCOP_MIN_LANE_WAVE = 8;  // a call is split over the lanes only when every lane gets at least this many frames
 struct Lane;
 
+// Owns n elements of T in device memory, or (Pinned) in pinned host memory mapped into the device's address space,
+// and frees them when it is destroyed.  It reads as a T*: the kernel argument structs and the other views hold plain
+// pointers into buffers that a lane or the handle owns.
+template <class T, bool Pinned = false>
+class Buffer {
+ public:
+  Buffer() = default;
+  Buffer(const Buffer&) = delete;
+  Buffer& operator=(const Buffer&) = delete;
+  Buffer(Buffer&& o) noexcept : p_(o.p_), n_(o.n_) {
+    o.p_ = nullptr;
+    o.n_ = 0;
+  }
+  Buffer& operator=(Buffer&& o) noexcept {
+    if (this != &o) {
+      reset();
+      std::swap(p_, o.p_);
+      std::swap(n_, o.n_);
+    }
+    return *this;
+  }
+  ~Buffer() { reset(); }
+
+  operator T*() const { return p_; }
+  T* get() const { return p_; }  // (for casts, which do not convert)
+  size_t size() const { return n_; }  // elements
+
+  void reset() {
+    if (p_) {
+      if constexpr (Pinned) cudaFreeHost(p_);
+      else cudaFree(p_);
+    }
+    p_ = nullptr;
+    n_ = 0;
+  }
+  // frees what the buffer holds, then allocates n elements (at least one); on failure the buffer is left empty
+  cudaError_t allocate(size_t n) {
+    reset();
+    void* q = nullptr;
+    const size_t bytes = std::max<size_t>(n, 1) * sizeof(T);
+    cudaError_t e;
+    if constexpr (Pinned) e = cudaHostAlloc(&q, bytes, cudaHostAllocMapped);
+    else e = cudaMalloc(&q, bytes);
+    if (e != cudaSuccess) return e;
+    p_ = static_cast<T*>(q);
+    n_ = n;
+    return cudaSuccess;
+  }
+  // allocate(n), the error recorded in h
+  int alloc(pcop_handle* h, size_t n) {
+    const cudaError_t e = allocate(n);
+    return e == cudaSuccess ? PCOP_OK : fail_cuda(h, e, Pinned ? "cudaHostAlloc" : "cudaMalloc", __FILE__, __LINE__);
+  }
+
+ private:
+  T* p_ = nullptr;
+  size_t n_ = 0;
+};
+template <class T>
+using HostBuffer = Buffer<T, true>;
+
 }  // namespace pcop
 
 struct pcop_handle {
@@ -126,15 +189,9 @@ struct pcop_handle {
   int ece_small_max = 0;       // ECE_SMALL_MAX or PCOP_ECE_SMALL_MAX (read at create)
   std::vector<std::unique_ptr<pcop::Lane>> lanes;  // batched calls deal their waves round-robin to the lanes
   std::string err;
-  std::vector<void*> dev_allocs;
-  std::vector<void*> host_allocs;
-  int* d_rng = nullptr;
-  float4* d_acc = nullptr;  // accumulated (world-frame) cloud, od.cpp:697
+  pcop::Buffer<int> d_rng;
+  pcop::Buffer<float4> d_acc;  // accumulated (world-frame) cloud, od.cpp:697
   int acc_count = 0;
-  unsigned char* d_occ = nullptr;  // occupancy grid scratch: int64 counts, int64 row averages, int8 cells
-  size_t occ_cap = 0;
-  unsigned char* d_shadow = nullptr;  // pcop_occupancy_shadows scratch: grid cells, CSR copy, records, warning word
-  size_t shadow_cap = 0;
 
   // per-call accounting (launch counts also accumulate over the single-frame calls until the next pcop_process* call)
   cudaEvent_t ev_call[2] = {nullptr, nullptr};
@@ -159,61 +216,61 @@ struct Lane {
   cudaEvent_t ev_stage[PCOP_N_STAGES][2] = {};
   bool stage_used[PCOP_N_STAGES] = {};
 
-  // device
-  float4 *d_in = nullptr, *d_crop = nullptr, *d_vox = nullptr, *d_sor = nullptr, *d_pbuf[2] = {nullptr, nullptr},
-         *d_rem = nullptr, *d_sorted = nullptr, *d_obst = nullptr;
-  int *d_crop_kept = nullptr, *d_run_start = nullptr, *d_sor_kept = nullptr, *d_psrc[2] = {nullptr, nullptr},
-      *d_rem_src = nullptr, *d_inliers = nullptr, *d_parent = nullptr, *d_csize = nullptr, *d_roots = nullptr,
-      *d_rank = nullptr, *d_indices = nullptr, *d_offsets = nullptr, *d_cell_start = nullptr;
-  uint32_t* d_cell_key = nullptr;
-  uint32_t* d_vox_keys = nullptr;
-  float* d_sor_dist = nullptr;
-  SortBufs sort{};
-  unsigned* d_desc = nullptr;
-  int* d_counts = nullptr;        // [CNT_ROWS][maxB]
-  uint32_t* d_warnings = nullptr; // [maxB]
-  MinMax* d_minmax = nullptr;
-  VoxelFrame* d_vf = nullptr;
-  EceFrame* d_ef = nullptr;
-  PlaneFrame* d_pf = nullptr;
-  PlaneRecord* d_prec = nullptr;
-  double* d_partial = nullptr;  // [maxB][chunks][10]
-  double* d_thr = nullptr;
-  int* d_pack_off = nullptr;  // [PK_N][maxB]
-  PackMeta* d_meta = nullptr;
-  unsigned char* d_pack = nullptr;  // packed results of the wave in flight (PCOP_OUT_DEVICE: of all waves of the call)
-  size_t pack_cap = 0;
-  unsigned long long* d_pack_cursor = nullptr;  // PCOP_OUT_DEVICE: bytes of d_pack used by the call so far
+  // device: [maxB * cap] wave arrays and per-frame records, allocated by pcop_create
+  Buffer<float4> d_in, d_crop, d_vox, d_sor, d_rem, d_sorted, d_obst;
+  float4* d_pbuf[2] = {nullptr, nullptr};  // (overlays, see init_lane)
+  Buffer<int> d_crop_kept, d_run_start, d_sor_kept, d_psrc[2], d_rem_src, d_inliers, d_parent, d_csize, d_roots, d_rank,
+      d_indices, d_offsets, d_cell_start;
+  Buffer<uint32_t> d_cell_key, d_vox_keys;
+  Buffer<float> d_sor_dist;
+  Buffer<uint32_t> d_sort_key[2], d_sort_val[2], d_sort_hist, d_sort_desc, d_sort_maxkey;
+  Buffer<int> d_sort_npass;
+  Buffer<unsigned long long> d_sort_stats;
+  SortBufs sort{};  // views of the d_sort_* buffers
+  Buffer<unsigned> d_desc;
+  Buffer<int> d_counts;        // [CNT_ROWS][maxB]
+  Buffer<uint32_t> d_warnings; // [maxB]
+  Buffer<MinMax> d_minmax;
+  Buffer<VoxelFrame> d_vf;
+  Buffer<EceFrame> d_ef;
+  Buffer<PlaneFrame> d_pf;
+  Buffer<PlaneRecord> d_prec;
+  Buffer<double> d_partial;  // [maxB][chunks][10]
+  Buffer<double> d_thr;
+  Buffer<int> d_pack_off;  // [PK_N][maxB]
+  Buffer<PackMeta> d_meta;
+  Buffer<unsigned long long> d_pack_cursor;  // PCOP_OUT_DEVICE: bytes of d_pack used by the call so far
+  // from here on, buffers that grow (grow(), never shrunk) with the parameters or with the calls the lane has run
+  Buffer<unsigned char> d_pack;  // packed results of the wave in flight (PCOP_OUT_DEVICE: of all waves of the call)
   // pcop_process_batch_occupancy (allocated by the first such call; counts / grids grow with W x H and with the
   // largest wave the lane has run)
-  int* d_occ_counts = nullptr;       // [wave frames][cells] int32
-  signed char* d_occ_grids = nullptr;  // [wave frames][cells]
-  size_t occ_scratch_cells = 0;      // frames x cells the two arrays hold
-  Mat34* d_occ_mats = nullptr;       // [maxB][2] world_to_sensor, sensor_to_world
-  Mat34* h_occ_mats = nullptr;       // pinned staging of the same
+  Buffer<int> d_occ_counts;          // [wave frames][cells] int32
+  Buffer<signed char> d_occ_grids;   // [wave frames][cells]
+  Buffer<Mat34> d_occ_mats;          // [maxB][2] world_to_sensor, sensor_to_world
+  HostBuffer<Mat34> h_occ_mats;      // pinned staging of the same
   cudaEvent_t ev_grids_copied = nullptr;  // the last copy out of d_occ_grids
-  unsigned char* d_raw = nullptr;  // staging of raw PointCloud2 payloads from host memory: one message, or the host
-  size_t raw_cap = 0;              // messages of one wave at 256-byte aligned offsets (grown on demand)
-  Pc2Frame* d_pc2 = nullptr;       // decode descriptors of k_pc2_ingest: one per message of a wave
-  Pc2Frame* h_pc2 = nullptr;       // pinned staging of the same (the batched PointCloud2 wave)
-  size_t pc2_cap = 0;              // descriptors the two hold (grown on demand, never shrunk)
+  Buffer<unsigned char> d_raw;  // staging of raw PointCloud2 payloads from host memory: one message, or the host
+                                // messages of one wave at 256-byte aligned offsets (a quarter more slack when it grows)
+  Buffer<Pc2Frame> d_pc2;       // decode descriptors of k_pc2_ingest: one per message of a wave
+  HostBuffer<Pc2Frame> h_pc2;   // pinned staging of the same (the batched PointCloud2 wave)
   int pc2_msgs = 0, pc2_tiles = 0; // messages and record tiles of the wave in flight (a repeat decodes them again)
+  // single-frame occupancy calls (lane 0): pcop_occupancy_grid's int64 counts, int64 row averages and int8 cells;
+  // pcop_occupancy_shadows' grid cells, CSR copy, records and warning word
+  Buffer<unsigned char> d_occ, d_shadow;
 
   // pinned host
-  int* h_counts = nullptr;  // [CNT_ROWS][maxB]
-  uint32_t* h_warnings = nullptr;
-  PlaneRecord* h_prec = nullptr;
-  PackMeta* h_meta = nullptr;
-  int* h_n_in = nullptr;  // staging for the per-frame input sizes
-  unsigned long long* h_stats = nullptr;
+  HostBuffer<int> h_counts;  // [CNT_ROWS][maxB]
+  HostBuffer<uint32_t> h_warnings;
+  HostBuffer<PlaneRecord> h_prec;
+  HostBuffer<PackMeta> h_meta;
+  HostBuffer<int> h_n_in;  // staging for the per-frame input sizes
+  HostBuffer<unsigned long long> h_stats;
   // pinned result buffers: two per lane, used by alternate calls, so the pointers a call returns stay valid while the
   // NEXT call runs (a consumer may still be reading them, e.g. the multi-GPU result gather)
-  unsigned char* h_pack_buf[2] = {nullptr, nullptr};
-  size_t h_pack_buf_cap[2] = {0, 0};
+  HostBuffer<unsigned char> h_pack_buf[2];
   int h_pack_sel = 0;
-  unsigned char* h_pack = nullptr;  // = h_pack_buf[h_pack_sel]
-  size_t h_pack_cap = 0;
   size_t h_pack_used = 0;  // of the running call
+  HostBuffer<unsigned char>& h_pack() { return h_pack_buf[h_pack_sel]; }  // the running call's
 
   int wave_seq = 0;                 // waves of the running call seen by this lane
   int call_lane_waves = 1;          // waves of the running call dealt to this lane
@@ -237,17 +294,14 @@ struct Lane {
   const float4* plane_in = nullptr;   // plane-stage input of the wave in flight (for a repeat of the stage)
   size_t plane_stride = 0;
   const int* plane_n = nullptr;
-  uint32_t* d_vf_flags = nullptr;  // [maxB]
-  unsigned long long* d_vf_pair[2] = {nullptr, nullptr};
-  uint32_t* h_vf_flags = nullptr;
+  Buffer<uint32_t> d_vf_flags;  // [maxB]
+  unsigned long long* d_vf_pair[2] = {nullptr, nullptr};  // (overlays, see init_lane)
+  HostBuffer<uint32_t> h_vf_flags;
   // partition voxel path (allocated and grown by apply_params while the plan allows the path)
-  uint32_t* d_vp_hist = nullptr;
-  uint32_t* d_vp_bstart = nullptr;
-  uint32_t* d_vp_nstart = nullptr;
-  unsigned short* d_vp_ne = nullptr;
-  uint2* d_vp_grec = nullptr;
-  unsigned* d_vp_desc = nullptr;
-  int vp_gcap = 0;                 // groups per frame d_vp_grec / d_vp_desc hold
+  Buffer<uint32_t> d_vp_hist, d_vp_bstart, d_vp_nstart;
+  Buffer<unsigned short> d_vp_ne;
+  Buffer<uint2> d_vp_grec;         // [maxB][vp_gstride]
+  Buffer<unsigned> d_vp_desc;      // [maxB][vp_gstride]
   int vp_gstride = 0;              // worst-case groups per frame + 1
   int vp_group_hint = 0;           // groups per frame the next wave's reduce grid covers (adapts to the frames seen)
 
@@ -264,23 +318,15 @@ int fail(pcop_handle* h, int code, const std::string& msg);
     if (_s != PCOP_OK) return _s;   \
   } while (0)
 
-template <class T>
-int dalloc(pcop_handle* h, T** p, size_t n) {
-  void* q = nullptr;
-  cudaError_t e = cudaMalloc(&q, std::max<size_t>(n, 1) * sizeof(T));
-  if (e != cudaSuccess) return fail_cuda(h, e, "cudaMalloc", __FILE__, __LINE__);
-  h->dev_allocs.push_back(q);
-  *p = (T*)q;
-  return PCOP_OK;
-}
-template <class T>
-int halloc(pcop_handle* h, T** p, size_t n) {
-  void* q = nullptr;
-  cudaError_t e = cudaHostAlloc(&q, std::max<size_t>(n, 1) * sizeof(T), cudaHostAllocMapped);
-  if (e != cudaSuccess) return fail_cuda(h, e, "cudaHostAlloc", __FILE__, __LINE__);
-  h->host_allocs.push_back(q);
-  *p = (T*)q;
-  return PCOP_OK;
+// The one way a lane's buffer grows: when b holds fewer than n elements, wait for the lane's kernels and copies (they
+// may still use the old allocation), free it and allocate exactly n.  On failure b is left empty.
+template <class T, bool Pinned>
+int grow(Lane* l, Buffer<T, Pinned>& b, size_t n) {
+  if (n <= b.size()) return PCOP_OK;
+  pcop_handle* h = l->h;
+  PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
+  PCOP_CUDA_TRY(cudaStreamSynchronize(l->cstream));
+  return b.alloc(h, n);
 }
 
 inline uint32_t effective_outputs(const pcop_params& p) {
@@ -302,47 +348,9 @@ inline size_t pack_capacity_bytes(uint32_t mask, int B, int cap) {
   return (bytes + 256 + 255) & ~(size_t)255;
 }
 
-inline int ensure_pack_capacity(Lane* l, uint32_t mask) {
-  pcop_handle* h = l->h;
-  const size_t need = pack_capacity_bytes(mask, h->maxB, h->cap);
-  if (need <= l->pack_cap) return PCOP_OK;
-  if (l->cstream) cudaStreamSynchronize(l->cstream);
-  if (l->d_pack) cudaFree(l->d_pack);  // not tracked in dev_allocs
-  l->d_pack = nullptr;
-  l->pack_cap = 0;
-  cudaError_t e = cudaMalloc((void**)&l->d_pack, need);
-  if (e != cudaSuccess) return fail_cuda(h, e, "cudaMalloc(pack)", __FILE__, __LINE__);
-  l->pack_cap = need;
-  return PCOP_OK;
-}
-
-// the raw PointCloud2 staging of lane l holds at least `bytes` (grown by a quarter more, never shrunk)
-inline int ensure_raw(Lane* l, size_t bytes) {
-  pcop_handle* h = l->h;
-  if (bytes <= l->raw_cap) return PCOP_OK;
-  PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
-  if (l->d_raw) cudaFree(l->d_raw);  // (not tracked in dev_allocs)
-  l->d_raw = nullptr;
-  l->raw_cap = 0;
-  PCOP_CUDA_TRY(cudaMalloc((void**)&l->d_raw, bytes + bytes / 4 + 256));
-  l->raw_cap = bytes + bytes / 4 + 256;
-  return PCOP_OK;
-}
-
-// the PointCloud2 decode descriptors of lane l hold at least `msgs` messages (grown, never shrunk)
-inline int ensure_pc2(Lane* l, size_t msgs) {
-  pcop_handle* h = l->h;
-  if (msgs <= l->pc2_cap) return PCOP_OK;
-  PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
-  cudaFree(l->d_pc2);  // (not tracked in dev_allocs / host_allocs)
-  if (l->h_pc2) cudaFreeHost(l->h_pc2);
-  l->d_pc2 = nullptr;
-  l->h_pc2 = nullptr;
-  l->pc2_cap = 0;
-  PCOP_CUDA_TRY(cudaMalloc((void**)&l->d_pc2, sizeof(Pc2Frame) * msgs));
-  PCOP_CUDA_TRY(cudaHostAlloc((void**)&l->h_pc2, sizeof(Pc2Frame) * msgs, cudaHostAllocDefault));
-  l->pc2_cap = msgs;
-  return PCOP_OK;
+// the raw PointCloud2 staging of lane l holds at least `bytes` (when it grows, by a quarter more)
+inline int grow_raw(Lane* l, size_t bytes) {
+  return bytes <= l->d_raw.size() ? PCOP_OK : grow(l, l->d_raw, bytes + bytes / 4 + 256);
 }
 
 inline bool is_device_pointer(const void* p) {

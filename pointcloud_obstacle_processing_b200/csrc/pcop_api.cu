@@ -1,7 +1,9 @@
 // C ABI of the library (include/pcop.h): handle creation and parameters, the single-frame and stage-isolated entry
 // points.  The batched calls run in the wave scheduler (batch.cu).
-// Every buffer is allocated by pcop_create (pcop_set_params may grow the partition voxel path's); the pinned result
-// buffer only grows (a second call of the same shape allocates nothing).
+// Memory: every allocation is a Buffer (handle.cuh) owned by a lane, or by the handle for the accumulated cloud and the
+// RANSAC table, and is freed with its owner.  pcop_create allocates the wave buffers; the buffers that depend on the
+// parameters or on a call's shape grow through grow() and never shrink (a second call of the same shape allocates
+// nothing).
 #include <cstdio>
 #include <cstdlib>
 
@@ -180,71 +182,53 @@ int init_lane(Lane* l) {
   const int B = h->maxB;
   const int chunks = cdiv(h->cap, TS_CHUNK);
   const int tiles = cdiv(h->cap, CT_TILE);
-  TRY(dalloc(h, &l->d_in, BC));
-  TRY(dalloc(h, &l->d_crop, BC));
-  TRY(dalloc(h, &l->d_vox, BC));
-  TRY(dalloc(h, &l->d_sor, BC));
+  for (Buffer<float4>* b : {&l->d_in, &l->d_crop, &l->d_vox, &l->d_sor, &l->d_rem, &l->d_sorted, &l->d_obst})
+    TRY(b->alloc(h, BC));
   // plane ping-pong clouds (only frames that need a second pass touch them): the cropped cloud and the input staging
   // are dead by then (the fused voxel path gathers from the caller's / staged input before the plane stage starts)
   l->d_pbuf[0] = l->d_crop;
   l->d_pbuf[1] = l->d_in;
-  TRY(dalloc(h, &l->d_rem, BC));
-  TRY(dalloc(h, &l->d_sorted, BC));
-  TRY(dalloc(h, &l->d_obst, BC));
-  TRY(dalloc(h, &l->d_crop_kept, BC));
-  TRY(dalloc(h, &l->d_run_start, BC));
-  TRY(dalloc(h, &l->d_sor_kept, BC));
-  TRY(dalloc(h, &l->d_psrc[0], BC));
-  TRY(dalloc(h, &l->d_psrc[1], BC));
-  TRY(dalloc(h, &l->d_rem_src, BC));
-  TRY(dalloc(h, &l->d_inliers, BC));
-  TRY(dalloc(h, &l->d_parent, BC));
-  TRY(dalloc(h, &l->d_csize, BC));
-  TRY(dalloc(h, &l->d_roots, BC));
-  TRY(dalloc(h, &l->d_rank, BC));
-  TRY(dalloc(h, &l->d_indices, BC));
-  TRY(dalloc(h, &l->d_cell_start, BC));
-  TRY(dalloc(h, &l->d_cell_key, BC));
-  TRY(dalloc(h, &l->d_offsets, BC + B));
-  TRY(dalloc(h, &l->d_vox_keys, BC));
-  TRY(dalloc(h, &l->d_sor_dist, BC));
-  TRY(dalloc(h, &l->sort.key[0], BC));
-  TRY(dalloc(h, &l->sort.key[1], BC));
-  TRY(dalloc(h, &l->sort.val[0], BC));
-  TRY(dalloc(h, &l->sort.val[1], BC));
-  TRY(dalloc(h, &l->sort.hist, std::max((size_t)B * RS_MAX_PASSES * RS_BINS, vox_fused_hist_elems(B))));
-  {
-    unsigned char* d = nullptr;
-    TRY(dalloc(h, &d, std::max(sort_desc_bytes(B, h->cap), vox_fused_desc_bytes(B, h->cap))));
-    l->sort.desc = (uint32_t*)d;
-  }
-  TRY(dalloc(h, &l->d_vf_flags, B));
+  for (Buffer<int>* b : {&l->d_crop_kept, &l->d_run_start, &l->d_sor_kept, &l->d_psrc[0], &l->d_psrc[1], &l->d_rem_src,
+                         &l->d_inliers, &l->d_parent, &l->d_csize, &l->d_roots, &l->d_rank, &l->d_indices,
+                         &l->d_cell_start})
+    TRY(b->alloc(h, BC));
+  TRY(l->d_cell_key.alloc(h, BC));
+  TRY(l->d_offsets.alloc(h, BC + B));
+  TRY(l->d_vox_keys.alloc(h, BC));
+  TRY(l->d_sor_dist.alloc(h, BC));
+  for (Buffer<uint32_t>* b : {&l->d_sort_key[0], &l->d_sort_key[1], &l->d_sort_val[0], &l->d_sort_val[1]})
+    TRY(b->alloc(h, BC));
+  TRY(l->d_sort_hist.alloc(h, std::max((size_t)B * RS_MAX_PASSES * RS_BINS, vox_fused_hist_elems(B))));
+  TRY(l->d_sort_desc.alloc(h, std::max(sort_desc_bytes(B, h->cap), vox_fused_desc_bytes(B, h->cap)) / sizeof(uint32_t)));
+  TRY(l->d_vf_flags.alloc(h, B));
   // (key, index) pairs of the fused voxel path: they overlay the search-grid point list of SOR / clustering
-  l->d_vf_pair[0] = reinterpret_cast<unsigned long long*>(l->d_sorted);
-  l->d_vf_pair[1] = reinterpret_cast<unsigned long long*>(l->d_sorted) + BC;
-  TRY(halloc(h, &l->h_vf_flags, B));
-  TRY(dalloc(h, &l->sort.maxkey, B));
-  TRY(dalloc(h, &l->sort.npass, B));
-  TRY(dalloc(h, &l->sort.stats, 1));
-  TRY(halloc(h, &l->h_stats, 1));
-  TRY(dalloc(h, &l->d_desc, (size_t)B * tiles));
-  TRY(dalloc(h, &l->d_counts, (size_t)CNT_ROWS * B));
-  TRY(dalloc(h, &l->d_warnings, B));
-  TRY(dalloc(h, &l->d_minmax, B));
-  TRY(dalloc(h, &l->d_vf, B));
-  TRY(dalloc(h, &l->d_ef, B));
-  TRY(dalloc(h, &l->d_pf, B));
-  TRY(dalloc(h, &l->d_prec, B));
-  TRY(dalloc(h, &l->d_partial, (size_t)B * chunks * 10));
-  TRY(dalloc(h, &l->d_thr, B));
-  TRY(dalloc(h, &l->d_pack_off, (size_t)PK_N * B));
-  TRY(dalloc(h, &l->d_meta, 1));
-  TRY(dalloc(h, &l->d_pack_cursor, 1));
-  TRY(halloc(h, &l->h_counts, (size_t)CNT_ROWS * B));
-  TRY(halloc(h, &l->h_warnings, B));
-  TRY(halloc(h, &l->h_prec, B));
-  TRY(halloc(h, &l->h_meta, 1));
-  TRY(halloc(h, &l->h_n_in, (size_t)B + 16));
+  l->d_vf_pair[0] = reinterpret_cast<unsigned long long*>(l->d_sorted.get());
+  l->d_vf_pair[1] = l->d_vf_pair[0] + BC;
+  TRY(l->h_vf_flags.alloc(h, B));
+  TRY(l->d_sort_maxkey.alloc(h, B));
+  TRY(l->d_sort_npass.alloc(h, B));
+  TRY(l->d_sort_stats.alloc(h, 1));
+  l->sort = SortBufs{{l->d_sort_key[0], l->d_sort_key[1]}, {l->d_sort_val[0], l->d_sort_val[1]}, l->d_sort_hist,
+                     l->d_sort_desc, l->d_sort_maxkey, l->d_sort_npass, l->d_sort_stats};
+  TRY(l->h_stats.alloc(h, 1));
+  TRY(l->d_desc.alloc(h, (size_t)B * tiles));
+  TRY(l->d_counts.alloc(h, (size_t)CNT_ROWS * B));
+  TRY(l->d_warnings.alloc(h, B));
+  TRY(l->d_minmax.alloc(h, B));
+  TRY(l->d_vf.alloc(h, B));
+  TRY(l->d_ef.alloc(h, B));
+  TRY(l->d_pf.alloc(h, B));
+  TRY(l->d_prec.alloc(h, B));
+  TRY(l->d_partial.alloc(h, (size_t)B * chunks * 10));
+  TRY(l->d_thr.alloc(h, B));
+  TRY(l->d_pack_off.alloc(h, (size_t)PK_N * B));
+  TRY(l->d_meta.alloc(h, 1));
+  TRY(l->d_pack_cursor.alloc(h, 1));
+  TRY(l->h_counts.alloc(h, (size_t)CNT_ROWS * B));
+  TRY(l->h_warnings.alloc(h, B));
+  TRY(l->h_prec.alloc(h, B));
+  TRY(l->h_meta.alloc(h, 1));
+  TRY(l->h_n_in.alloc(h, (size_t)B + 16));
   PCOP_CUDA_TRY(cudaMemset(l->d_counts, 0, sizeof(int) * CNT_ROWS * B));
   PCOP_CUDA_TRY(cudaMemset(l->d_pf, 0, sizeof(PlaneFrame) * B));
   for (int s = 0; s < PCOP_N_STAGES; ++s)
@@ -265,24 +249,15 @@ int apply_params(pcop_handle* h, const pcop_params& p) {
   const int B = h->maxB;
   for (auto& lp : h->lanes) {
     Lane* l = lp.get();
-    if (plan.part_ok && !l->d_vp_ne) {
-      TRY(dalloc(h, &l->d_vp_hist, vox_part_hist_elems(B)));
-      TRY(dalloc(h, &l->d_vp_bstart, vox_part_chunk_start_elems(B)));
-      TRY(dalloc(h, &l->d_vp_nstart, vox_part_start_elems(B)));
-      TRY(dalloc(h, &l->d_vp_ne, vox_part_bucket_elems(B)));
+    if (plan.part_ok) {
+      TRY(grow(l, l->d_vp_hist, vox_part_hist_elems(B)));
+      TRY(grow(l, l->d_vp_bstart, vox_part_chunk_start_elems(B)));
+      TRY(grow(l, l->d_vp_nstart, vox_part_start_elems(B)));
+      TRY(grow(l, l->d_vp_ne, vox_part_bucket_elems(B)));
+      TRY(grow(l, l->d_vp_grec, (size_t)B * gstride));
+      TRY(grow(l, l->d_vp_desc, (size_t)B * gstride));
     }
-    if (gstride > l->vp_gcap) {
-      PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
-      cudaFree(l->d_vp_grec);  // (not tracked in dev_allocs)
-      cudaFree(l->d_vp_desc);
-      l->d_vp_grec = nullptr;
-      l->d_vp_desc = nullptr;
-      l->vp_gcap = 0;
-      PCOP_CUDA_TRY(cudaMalloc((void**)&l->d_vp_grec, sizeof(uint2) * B * gstride));
-      PCOP_CUDA_TRY(cudaMalloc((void**)&l->d_vp_desc, sizeof(unsigned) * B * gstride));
-      l->vp_gcap = gstride;
-    }
-    TRY(ensure_pack_capacity(l, effective_outputs(p)));
+    TRY(grow(l, l->d_pack, pack_capacity_bytes(effective_outputs(p), B, h->cap)));
   }
   std::vector<int> tbl(RNG_TABLE);
   fill_rng_table(p.ransac_seed, tbl.data(), RNG_TABLE);
@@ -301,19 +276,9 @@ int apply_params(pcop_handle* h, const pcop_params& p) {
 
 }  // namespace
 
-pcop::Lane::~Lane() {
+pcop::Lane::~Lane() {  // (the buffers free themselves once the streams are idle)
   if (stream) cudaStreamSynchronize(stream);
   if (cstream) cudaStreamSynchronize(cstream);
-  cudaFree(d_pack);  // (the buffers that grow are not tracked in dev_allocs)
-  cudaFree(d_raw);
-  cudaFree(d_occ_counts);
-  cudaFree(d_occ_grids);
-  cudaFree(d_vp_grec);
-  cudaFree(d_vp_desc);
-  cudaFree(d_pc2);
-  if (h_pc2) cudaFreeHost(h_pc2);
-  for (int i = 0; i < 2; ++i)
-    if (h_pack_buf[i]) cudaFreeHost(h_pack_buf[i]);
   for (cudaEvent_t e : {ev_lane_done, ev_copied, ev_meta, ev_grids_copied})
     if (e) cudaEventDestroy(e);
   for (const TraceRec& r : trace_recs)  // (PCOP_TRACE)
@@ -419,8 +384,8 @@ int pcop_create(const pcop_params* params, int device, size_t max_points, int ma
   const int st = [&] {  // everything the handle allocates, then the parameters
     TRY(validate_params(h, *params));
     PCOP_CUDA_TRY(cudaSetDevice(h->device));
-    TRY(dalloc(h, &h->d_acc, (size_t)h->cap));
-    TRY(dalloc(h, &h->d_rng, RNG_TABLE));
+    TRY(h->d_acc.alloc(h, (size_t)h->cap));
+    TRY(h->d_rng.alloc(h, RNG_TABLE));
     for (int i = 0; i < 2; ++i) PCOP_CUDA_TRY(cudaEventCreate(&h->ev_call[i]));
     for (int i = 0; i < n_lanes; ++i) {
       h->lanes.emplace_back(new Lane{h});
@@ -441,10 +406,6 @@ void pcop_destroy(pcop_handle* h) {
   if (!h) return;
   cudaSetDevice(h->device);
   h->lanes.clear();  // (every lane waits for its streams first)
-  for (void* p : h->dev_allocs) cudaFree(p);
-  for (void* p : h->host_allocs) cudaFreeHost(p);
-  if (h->d_occ) cudaFree(h->d_occ);
-  if (h->d_shadow) cudaFree(h->d_shadow);
   if (h->kt.ev) {
     for (int i = 0; i < 2 * KernelTimers::MAX_SLOTS; ++i) cudaEventDestroy(h->kt.ev[i]);
     delete[] h->kt.ev;
@@ -513,7 +474,7 @@ int pcop_process_batch_occupancy(pcop_handle* h, const float* xyzw, size_t frame
   if (xyzw) return process_impl(h, xyzw, frame_stride_points, n, batch, out, &oc);
   // the accumulated cloud, consumed by this run (od.cpp:701), as pcop_process_accumulated
   const int32_t acc_n = h->acc_count;
-  const int st = process_impl(h, reinterpret_cast<const float*>(h->d_acc), (size_t)(acc_n > 0 ? acc_n : 1), &acc_n, 1, out, &oc);
+  const int st = process_impl(h, reinterpret_cast<const float*>(h->d_acc.get()), (size_t)(acc_n > 0 ? acc_n : 1), &acc_n, 1, out, &oc);
   h->acc_count = 0;
   return st;
 }
@@ -666,7 +627,7 @@ int pcop_process_accumulated(pcop_handle* h, pcop_frame_result* out) {
   if (!h || !out) return fail(h, PCOP_ERR_BAD_PARAM, "null argument");
   const int32_t n = h->acc_count;
   // od.cpp:701: current_frame_count = 0; the accumulator is consumed by this run
-  const int st = process_impl(h, reinterpret_cast<const float*>(h->d_acc), (size_t)(n > 0 ? n : 1), &n, 1, out);
+  const int st = process_impl(h, reinterpret_cast<const float*>(h->d_acc.get()), (size_t)(n > 0 ? n : 1), &n, 1, out);
   h->acc_count = 0;
   return st;
 }
@@ -723,7 +684,7 @@ int pcop_cloud_to_pointcloud2(pcop_handle* h, const float* xyzw, int32_t n, int3
   unsigned char* dst = out_data;
   const bool out_on_device = is_device_pointer(out_data);
   if (!out_on_device) {  // staged through the raw-payload buffer of the ingest path
-    TRY(ensure_raw(l, bytes));
+    TRY(grow_raw(l, bytes));
     dst = l->d_raw;
   }
   Ctx c = make_ctx(l, 1, n);
@@ -759,18 +720,10 @@ int pcop_occupancy_grid(pcop_handle* h, const float* xyzw, int32_t n, int8_t* gr
     TRY(device_cloud(h, xyzw, n, &src));
   }
   const size_t cells = (size_t)g.cells;
-  const size_t need = cells * 8 + (size_t)H * 8 + cells;
-  if (need > h->occ_cap) {
-    PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
-    if (h->d_occ) cudaFree(h->d_occ);
-    h->d_occ = nullptr;
-    h->occ_cap = 0;
-    PCOP_CUDA_TRY(cudaMalloc((void**)&h->d_occ, need + 256));
-    h->occ_cap = need;
-  }
-  unsigned long long* d_counts = reinterpret_cast<unsigned long long*>(h->d_occ);
-  long long* d_avg = reinterpret_cast<long long*>(h->d_occ + cells * 8);
-  signed char* d_grid = reinterpret_cast<signed char*>(h->d_occ + cells * 8 + (size_t)H * 8);
+  TRY(grow(l, l->d_occ, cells * 8 + (size_t)H * 8 + cells + 256));
+  unsigned long long* d_counts = reinterpret_cast<unsigned long long*>(l->d_occ.get());
+  long long* d_avg = reinterpret_cast<long long*>(l->d_occ + cells * 8);
+  signed char* d_grid = reinterpret_cast<signed char*>(l->d_occ + cells * 8 + (size_t)H * 8);
   Ctx c = make_ctx(l, 1, n);
   PCOP_CUDA_TRY(cudaMemsetAsync(d_counts, 0, cells * 8, l->stream));
   run_occ_count(c, src, n, g, d_counts);
@@ -810,15 +763,8 @@ int pcop_occupancy_shadows(pcop_handle* h, const float* remaining_xyzw, int32_t 
   const size_t off_ints = (cells + 15) & ~(size_t)15;
   const size_t need = off_ints + ((size_t)n_clusters + 1 + (size_t)L + 6 * (size_t)n_clusters + 3) * sizeof(int32_t) +
                       2 * sizeof(Mat34);
-  if (need > h->shadow_cap) {
-    PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
-    if (h->d_shadow) cudaFree(h->d_shadow);
-    h->d_shadow = nullptr;
-    h->shadow_cap = 0;
-    PCOP_CUDA_TRY(cudaMalloc((void**)&h->d_shadow, need + 256));
-    h->shadow_cap = need;
-  }
-  int32_t* d_off = reinterpret_cast<int32_t*>(h->d_shadow + off_ints);
+  TRY(grow(l, l->d_shadow, need + 256));
+  int32_t* d_off = reinterpret_cast<int32_t*>(l->d_shadow + off_ints);
   int32_t* d_idx = d_off + n_clusters + 1;
   int32_t* d_rec = d_idx + L;
   uint32_t* d_warn = reinterpret_cast<uint32_t*>(d_rec + 6 * (size_t)n_clusters);
@@ -861,8 +807,8 @@ int pcop_occupancy_shadows(pcop_handle* h, const float* remaining_xyzw, int32_t 
   const bool grid_on_device = is_device_pointer(grid_data);
   a.grid = reinterpret_cast<signed char*>(grid_data);
   if (!grid_on_device) {
-    PCOP_CUDA_TRY(cudaMemcpyAsync(h->d_shadow, grid_data, cells, cudaMemcpyHostToDevice, l->stream));
-    a.grid = reinterpret_cast<signed char*>(h->d_shadow);
+    PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_shadow, grid_data, cells, cudaMemcpyHostToDevice, l->stream));
+    a.grid = reinterpret_cast<signed char*>(l->d_shadow.get());
   }
   a.records = shadow_records ? d_rec : nullptr;
   a.warnings = d_warn;
