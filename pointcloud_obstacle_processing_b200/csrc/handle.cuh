@@ -218,7 +218,6 @@ struct Lane {
 
   // device: [maxB * cap] wave arrays and per-frame records, allocated by pcop_create
   Buffer<float4> d_in, d_crop, d_vox, d_sor, d_rem, d_sorted, d_obst;
-  float4* d_pbuf[2] = {nullptr, nullptr};  // (overlays, see init_lane)
   Buffer<int> d_crop_kept, d_run_start, d_sor_kept, d_psrc[2], d_rem_src, d_inliers, d_parent, d_csize, d_roots, d_rank,
       d_indices, d_offsets, d_cell_start;
   Buffer<uint32_t> d_cell_key, d_vox_keys;
@@ -436,8 +435,13 @@ inline PlaneArgs make_plane_args(Lane* l, const float4* in, size_t stride, const
   a.in = in;
   a.in_stride = stride;
   a.n_in = n_in;
-  a.buf[0] = l->d_pbuf[0];
-  a.buf[1] = l->d_pbuf[1];
+  // plane ping-pong clouds (only frames that need a second pass touch them): buffers the chain has no use for by then,
+  // and never the stage input, which pass 0 reads while it writes buf[0] and which a repeat of the stage reads again.
+  // The cropped cloud and the input staging are dead once the plane stage starts (the fused voxel path gathers from
+  // the caller's / staged input before it) unless the stage reads them: then the SOR output (SOR off) and the voxel
+  // output (crop, voxel and SOR off) take their place.
+  a.buf[0] = (in == l->d_crop) ? l->d_sor : l->d_crop;
+  a.buf[1] = (in == l->d_in) ? l->d_vox : l->d_in;
   a.src[0] = l->d_psrc[0];
   a.src[1] = l->d_psrc[1];
   a.inlier_idx = l->d_inliers;

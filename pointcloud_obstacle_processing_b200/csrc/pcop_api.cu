@@ -184,10 +184,6 @@ int init_lane(Lane* l) {
   const int tiles = cdiv(h->cap, CT_TILE);
   for (Buffer<float4>* b : {&l->d_in, &l->d_crop, &l->d_vox, &l->d_sor, &l->d_rem, &l->d_sorted, &l->d_obst})
     TRY(b->alloc(h, BC));
-  // plane ping-pong clouds (only frames that need a second pass touch them): the cropped cloud and the input staging
-  // are dead by then (the fused voxel path gathers from the caller's / staged input before the plane stage starts)
-  l->d_pbuf[0] = l->d_crop;
-  l->d_pbuf[1] = l->d_in;
   for (Buffer<int>* b : {&l->d_crop_kept, &l->d_run_start, &l->d_sor_kept, &l->d_psrc[0], &l->d_psrc[1], &l->d_rem_src,
                          &l->d_inliers, &l->d_parent, &l->d_csize, &l->d_roots, &l->d_rank, &l->d_indices,
                          &l->d_cell_start})

@@ -293,6 +293,9 @@ __device__ __forceinline__ bool plane_select_replay(const PlaneConst& pc, double
   int best = -2147483647;
   int sel = -1;
   double k = 1.0;
+  // PCL's loop also stops after max_skip = 10 * max_iterations samples that fail computeModelCoefficients.  A good
+  // sample never fails it, so that limit decides only max_iterations = 0: the loop never runs and no model is found.
+  if (pc.max_iterations == 0) nh = 0;
   for (int h = 0; h < nh; ++h) {
     if (!((double)h < k)) break;
     if (h >= navail) return true;

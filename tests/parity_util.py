@@ -65,3 +65,17 @@ def compare_frames(g, o, params, what=""):
         assert_bits_equal(g.cluster_indices, o.cluster_indices, what + "cluster_indices")
     if g.obstacles is not None:
         assert_close(g.obstacles, o.obstacles, what + "obstacles")
+
+
+def compare_plane(g, o, what=""):
+    """two segment_plane_and_extract_indices results (dicts of pcop_plane's outputs): counts and indices bit-exact,
+    the remaining cloud bit-exact, coefficients within REL_TOL"""
+    assert g["n_passes"] == o["n_passes"], f"{what}n_passes: {g['n_passes']} vs {o['n_passes']}"
+    assert_bits_equal(g["pass_points"], o["pass_points"], what + "pass_points")
+    assert_bits_equal(g["pass_inliers"], o["pass_inliers"], what + "pass_inliers")
+    assert_close(g["pass_coeff"], o["pass_coeff"], what + "pass_coeff")
+    assert_close(g["last_coeff"], o["last_coeff"], what + "last_coeff")
+    assert_bits_equal(g["inliers"], o["inliers"], what + "last inliers")
+    assert_bits_equal(g["src"], o["src"], what + "remaining src idx")
+    assert_bits_equal(g["remaining"], o["remaining"], what + "remaining cloud")
+    assert g["warnings"] == o["warnings"], f"{what}warnings: {g['warnings']} vs {o['warnings']}"

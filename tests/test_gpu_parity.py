@@ -3,7 +3,7 @@ import numpy as np
 import pytest
 
 import oracle_lib as O
-from parity_util import assert_bits_equal, assert_close, compare_frames
+from parity_util import assert_bits_equal, assert_close, compare_frames, compare_plane
 from pointcloud_obstacle_processing_b200 import ObstacleProcessor, synth
 from pointcloud_obstacle_processing_b200 import _ctypes_abi as abi
 
@@ -69,7 +69,8 @@ def test_stage_voxel(config, frames):
     assert_bits_equal(g_pts, o_pts, "voxel centroids")
 
 
-@pytest.mark.parametrize("mean_k", [15, 1, 31, 40])  # (the warp-per-point kernel holds up to 32 neighbours; 40 takes the serial one)
+@pytest.mark.parametrize("mean_k", [15, 1, 31, 32, 40, 63])  # (the warp-per-point kernel holds up to 32 neighbours: 32 is the
+# first value the serial one takes; 63 neighbours + the point itself fill its SOR_MAX_K = 64 array)
 def test_stage_sor(frames, mean_k):
     p = synth.params(1)
     p.statistical_outlier_meanK = mean_k
@@ -404,14 +405,7 @@ def _compare_plane(p, cloud):
     with ObstacleProcessor(p, len(cloud)) as op:
         g = op.segment_plane_and_extract_indices(cloud)
     o = O.plane(p, cloud)
-    assert g["n_passes"] == o["n_passes"]
-    assert_bits_equal(g["pass_points"], o["pass_points"], "pass_points")
-    assert_bits_equal(g["pass_inliers"], o["pass_inliers"], "pass_inliers")
-    assert_close(g["pass_coeff"], o["pass_coeff"], "pass_coeff")
-    assert_bits_equal(g["inliers"], o["inliers"], "last inliers")
-    assert_bits_equal(g["src"], o["src"], "remaining src idx")
-    assert_bits_equal(g["remaining"], o["remaining"], "remaining cloud")
-    assert g["warnings"] == o["warnings"]
+    compare_plane(g, o)
     return o
 
 
