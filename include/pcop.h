@@ -19,6 +19,8 @@
  *   od.cpp:699-852  pipeline + occupancy grid of a batch of frames                        -> pcop_process_batch_occupancy
  *   od.cpp:688-696 + 699-852  the same for a batch of raw PointCloud2 messages with a pose each -> pcop_process_batch_pointcloud2
  *   od.cpp:688-701 + 699-852  ... with accumulate_count messages (or several sensors) per frame -> pcop_process_batch_pointcloud2_windows
+ *   depth_image_proc (kinect2_bridge) + od.cpp:688-701 + 699-852 from depth images   -> pcop_process_batch_depth_windows
+ *                                                                                    / pcop_accumulate_depth_image
  *
  * Plain C: POD structs, raw pointers and sizes, integer status codes.  No C++
  * exceptions, PCL, ROS or torch types cross this boundary.
@@ -390,6 +392,51 @@ int pcop_process_batch_pointcloud2_windows(pcop_handle* h, const pcop_pointcloud
                                            const int32_t* window_first, int32_t batch, const float* transform16,
                                            const float* world_to_sensor16, const float* sensor_to_world16,
                                            int8_t* grids, pcop_frame_result* out);
+
+/* ---- depth images: the cloud of a depth camera built on the GPU from its sensor_msgs/Image + CameraInfo -------------
+ * A Kinect-style driver publishes a depth image (16UC1 millimetres or 32FC1 metres) and its CameraInfo; the node's
+ * `points` topic is the XYZRGB PointCloud2 that depth_image_proc builds from them on the host, 16x the bytes of the
+ * image.  These calls take the image instead and build the same cloud in the decode kernel of the batched pipeline:
+ * pixel (u, v) is point v * width + u; a pixel without a return (16UC1 0, 32FC1 non-finite) is a NaN point, otherwise
+ *   x = ((float)u - (float)cx) * depth * (float)(unit / fx),  y likewise with v, cy, fy,  z = depth * 0.001f (16UC1) or depth
+ * with unit = (double)0.001f (16UC1) or 1.0, each float op rounded in turn (depth_image_proc's convert<T>), and the
+ * padding float 1.0f.  The cloud is not dense: with a pose, NaN points are copied untransformed.  The decoded points
+ * equal, byte for byte, what the PointCloud2 calls decode from the point_step-32 XYZRGB message depth_image_proc
+ * publishes for the image, with is_dense = 0; colour does not enter PointXYZ, so the colour image is not an input.
+ * Little-endian images only; depth_image_proc's range_max substitution and ROI / binning corrections are not applied
+ * (pass the model's values). */
+enum {
+  PCOP_DEPTH_16UC1 = 1, /* "16UC1" and "mono16": uint16 millimetres, 0 = no return */
+  PCOP_DEPTH_32FC1 = 2  /* "32FC1": float metres, non-finite = no return           */
+};
+typedef struct pcop_depth_image {
+  const unsigned char* data;   /* sensor_msgs/Image.data: host or device pointer                       */
+  int32_t width, height;       /* Image.width / height                                                  */
+  int32_t step;                /* Image.step, bytes per row                                             */
+  int32_t encoding;            /* PCOP_DEPTH_*                                                          */
+  double fx, fy, cx, cy;       /* image_geometry::PinholeCameraModel fx() fy() cx() cy() (CameraInfo.P) */
+} pcop_depth_image;
+/* pcop_process_batch_depth_windows is pcop_process_batch_pointcloud2_windows with depth images in place of messages:
+ * frame f is the world-frame concatenation of images window_first[f] .. window_first[f + 1] - 1, out[f] and its grid
+ * equal pcop_accumulate_reset + pcop_accumulate_depth_image per image + pcop_process_accumulated (with grids:
+ * pcop_process_batch_occupancy(NULL, ...)), and PCOP_OUT_DEVICE, result pointer lifetime, the alternating pinned result
+ * buffers, payload memory kinds and the accumulator behave as there.  Windows of one image replay images one per frame.
+ * pcop_accumulate_depth_image appends one posed image to the accumulator (the live callback's path, in place of
+ * pcop_accumulate_pointcloud2); pcop_depth_image_to_xyz is the stage-isolated decode (no transform), out_xyzw
+ * [width * height][4].
+ * Errors (the handle stays usable), checked in the order of pcop_process_batch_pointcloud2_windows: PCOP_ERR_BAD_PARAM
+ * for a negative width or height, NULL data with pixels, an unknown encoding, step < width * sizeof(T) or step not a
+ * multiple of sizeof(T), fx or fy zero or non-finite, cx or cy non-finite, and every window_first / matrix check of
+ * pcop_process_batch_pointcloud2_windows; PCOP_ERR_CAPACITY for a window (accumulated cloud, image) of more than
+ * max_points pixels or a grid above PCOP_OCC_BATCH_MAX_CELLS.  An image of 0 pixels may have data == NULL.
+ * pcop_stage_times_us counts the upload and the decode as PCOP_STAGE_H2D; pcop_last_algorithmic_bytes counts
+ * (sizeof(T) + 16) bytes per pixel for the decode; the decode is one launch per wave. */
+int pcop_process_batch_depth_windows(pcop_handle* h, const pcop_depth_image* images, int32_t n_images,
+                                     const int32_t* window_first, int32_t batch, const float* transform16,
+                                     const float* world_to_sensor16, const float* sensor_to_world16, int8_t* grids,
+                                     pcop_frame_result* out);
+int pcop_accumulate_depth_image(pcop_handle* h, const pcop_depth_image* image, const float* transform16, int32_t* total);
+int pcop_depth_image_to_xyz(pcop_handle* h, const pcop_depth_image* image, float* out_xyzw);
 
 /* Copies `bytes` from a device result array (PCOP_OUT_DEVICE) to host memory, or device to device when dst is a device
  * pointer; synchronous. */

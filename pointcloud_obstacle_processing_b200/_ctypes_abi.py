@@ -48,6 +48,17 @@ class PointCloud2Frame(C.Structure):
     ]
 
 
+DEPTH_16UC1, DEPTH_32FC1 = 1, 2  # PCOP_DEPTH_*
+
+
+class DepthImageC(C.Structure):
+    """pcop_depth_image: one sensor_msgs/Image depth image + its pinhole model (data = host or device address)."""
+    _fields_ = [
+        ("data", C.c_void_p), ("width", C.c_int32), ("height", C.c_int32), ("step", C.c_int32),
+        ("encoding", C.c_int32), ("fx", C.c_double), ("fy", C.c_double), ("cx", C.c_double), ("cy", C.c_double),
+    ]
+
+
 class FrameResult(C.Structure):
     """pcop_frame_result."""
     _fields_ = [

@@ -19,7 +19,7 @@ import os
 import numpy as np
 
 from . import _ctypes_abi as abi
-from ._ctypes_abi import FrameResult, Params, PointCloud2Frame
+from ._ctypes_abi import DepthImageC, FrameResult, Params, PointCloud2Frame
 from .result import Frame
 
 
@@ -28,6 +28,52 @@ class PointCloud2Message(collections.namedtuple("PointCloud2Message",
                                                 defaults=(False,))):
     """The fields of a sensor_msgs/PointCloud2 message that the decode reads: data (bytes or uint8 array, host),
     n_points = width * height, point_step and the byte offsets of the FLOAT32 fields x, y, z."""
+
+
+# sensor_msgs/Image encodings of a depth image -> PCOP_DEPTH_*
+DEPTH_ENCODINGS = {"16UC1": abi.DEPTH_16UC1, "mono16": abi.DEPTH_16UC1, "32FC1": abi.DEPTH_32FC1}
+
+
+class DepthImage(collections.namedtuple("DepthImage", "data width height step encoding fx fy cx cy")):
+    """A depth image (sensor_msgs/Image) and the pinhole model of its CameraInfo: data (bytes or numpy array, host),
+    width, height, step (bytes per row), encoding (PCOP_DEPTH_* or a key of DEPTH_ENCODINGS), and
+    image_geometry::PinholeCameraModel's fx, fy, cx, cy."""
+
+    @classmethod
+    def from_array(cls, depth, fx, fy, cx, cy):
+        """a [H, W] uint16 (16UC1 millimetres) or float32 (32FC1 metres) array, rows possibly padded (step = the
+        array's row stride); its pixels must be contiguous along a row"""
+        depth = np.asarray(depth)
+        enc = {np.dtype(np.uint16): abi.DEPTH_16UC1, np.dtype(np.float32): abi.DEPTH_32FC1}.get(depth.dtype)
+        if enc is None or depth.ndim != 2:
+            raise ValueError("depth image must be a [H, W] uint16 or float32 array")
+        if depth.shape[1] > 1 and depth.strides[1] != depth.itemsize:
+            raise ValueError("the pixels of a row must be contiguous")
+        H, W = depth.shape
+        step = depth.strides[0] if H > 1 else W * depth.itemsize
+        return cls(depth, W, H, int(step), enc, float(fx), float(fy), float(cx), float(cy))
+
+
+def _depth_descriptors(images):
+    """DepthImage sequence -> (host buffers to keep alive, DepthImageC list)"""
+    keep, descs = [], []
+    for im in images:
+        im = DepthImage(*im)
+        enc = DEPTH_ENCODINGS[im.encoding] if isinstance(im.encoding, str) else int(im.encoding)
+        if im.data is None:
+            ptr, buf = None, None
+        elif isinstance(im.data, np.ndarray):
+            buf = im.data
+            if not (buf.flags.c_contiguous or (buf.ndim == 2 and buf.strides[1] == buf.itemsize and buf.strides[0] > 0)):
+                buf = np.ascontiguousarray(buf)
+            ptr = buf.ctypes.data if buf.size else None
+        else:
+            buf = np.frombuffer(im.data, np.uint8)
+            ptr = buf.ctypes.data if buf.size else None
+        keep.append(buf)
+        descs.append(DepthImageC(ptr, im.width, im.height, im.step, enc, im.fx, im.fy, im.cx, im.cy))
+    return keep, descs
+
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpcop.so")
@@ -56,6 +102,9 @@ EXPORTS = [
     "pcop_process_batch_occupancy",
     "pcop_process_batch_pointcloud2",
     "pcop_process_batch_pointcloud2_windows",
+    "pcop_process_batch_depth_windows",
+    "pcop_accumulate_depth_image",
+    "pcop_depth_image_to_xyz",
 ]
 
 
@@ -116,6 +165,10 @@ def load_library():
                                                  C.POINTER(FrameResult)]
     L.pcop_process_batch_pointcloud2_windows.argtypes = [vp, C.POINTER(PointCloud2Frame), i32, vp, i32, vp, vp, vp, vp,
                                                          C.POINTER(FrameResult)]
+    L.pcop_process_batch_depth_windows.argtypes = [vp, C.POINTER(DepthImageC), i32, vp, i32, vp, vp, vp, vp,
+                                                   C.POINTER(FrameResult)]
+    L.pcop_accumulate_depth_image.argtypes = [vp, C.POINTER(DepthImageC), vp, vp]
+    L.pcop_depth_image_to_xyz.argtypes = [vp, C.POINTER(DepthImageC), vp]
     L.pcop_enable_kernel_timing.argtypes = [vp, C.c_int]
     L.pcop_kernel_timing_count.argtypes = [vp]
     L.pcop_kernel_timing_get.argtypes = [vp, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_double),
@@ -385,6 +438,61 @@ class ObstacleProcessor:
                                                          sensor_to_world, None if g is None else g.ctypes.data)
         out = [Frame.from_c(r) for r in res]
         return (out, g) if grids else out
+
+    # ---- depth images: the depth camera's cloud built on the device (depth_image_proc + od.cpp:688-701) ----------
+    def process_batch_depth_windows_raw(self, images, window_first, transforms=None, world_to_sensor=None,
+                                        sensor_to_world=None, grids_ptr=None):
+        """pcop_process_batch_depth_windows.  images: a sequence of DepthImageC (data = host or device address); the
+        other arguments and the result as process_batch_pointcloud2_windows_raw."""
+        M = len(images)
+        first = np.ascontiguousarray(window_first, np.int32).reshape(-1)
+        if first.size < 1:
+            raise ValueError("window_first needs batch + 1 entries")
+        B = first.size - 1
+        arr = (DepthImageC * max(M, 1))(*images)
+        (t, tp), (ws, wsp), (sw, swp) = _mats(transforms, M, "transform"), _mats(world_to_sensor, B, "world_to_sensor"), \
+            _mats(sensor_to_world, B, "sensor_to_world")
+        res = (FrameResult * max(B, 1))()
+        self._check(self._lib.pcop_process_batch_depth_windows(
+            self._h, arr, M, first.ctypes.data_as(C.c_void_p), B, tp, wsp, swp,
+            None if grids_ptr is None else C.c_void_p(grids_ptr), res))
+        return res[:B] if B else []
+
+    def process_batch_depth_windows(self, images, window_first, transforms=None, world_to_sensor=None,
+                                    sensor_to_world=None, grids=False):
+        """images: a sequence of DepthImage (host payloads), one pose each in transforms ([n_images, 4, 4] float32
+        world <- camera, or None).  Frame f is the world-frame concatenation of the clouds of images window_first[f] ..
+        window_first[f + 1] - 1, each the cloud depth_image_proc builds from the image.  Returns the list of Frame, or
+        (frames, grids int8 [B, H, W]) with grids=True, as process_batch_pointcloud2_windows."""
+        self._host_results_only()
+        keep, descs = _depth_descriptors(images)
+        g = None
+        if grids:
+            w, h = self.occupancy_dims()
+            g = np.empty((len(window_first) - 1, h, w), np.int8)
+        res = self.process_batch_depth_windows_raw(descs, window_first, transforms, world_to_sensor, sensor_to_world,
+                                                   None if g is None else g.ctypes.data)
+        out = [Frame.from_c(r) for r in res]
+        return (out, g) if grids else out
+
+    def accumulate_depth_image(self, image, transform=None) -> int:
+        """the cloud of one DepthImage (depth_image_proc), world transform (is_dense = false) and append, on the
+        device; returns the accumulated point count"""
+        keep, (d,) = _depth_descriptors([image])
+        t = None if transform is None else np.ascontiguousarray(transform, dtype=np.float32).reshape(16)
+        total = C.c_int32()
+        self._check(self._lib.pcop_accumulate_depth_image(self._h, C.byref(d),
+                                                          None if t is None else t.ctypes.data_as(C.c_void_p),
+                                                          C.byref(total)))
+        return total.value
+
+    def depth_image_to_xyz(self, image):
+        """the stage-isolated decode of one DepthImage (no transform): float32 [width * height, 4]"""
+        keep, (d,) = _depth_descriptors([image])
+        n = d.width * d.height
+        out = np.empty((max(n, 1), 4), np.float32)
+        self._check(self._lib.pcop_depth_image_to_xyz(self._h, C.byref(d), out.ctypes.data_as(C.c_void_p)))
+        return out[:n].copy()
 
     # ---- accumulator ingest (od.cpp:691-698) ------------------------------------------
     def accumulate(self, cloud, transform=None, is_dense=False) -> int:

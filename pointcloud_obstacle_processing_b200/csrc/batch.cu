@@ -49,6 +49,16 @@ __device__ __forceinline__ float4 pc2_point(const Pc2Frame& d, float x, float y,
   }
   return o;
 }
+// the message that owns record tile `tile` of a decode launch: the last one whose first tile is <= tile
+__device__ __forceinline__ const Pc2Frame& tile_msg(const Pc2Frame* __restrict__ msgs, int n_msgs, int tile) {
+  int lo = 0, hi = n_msgs - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (msgs[mid].tile0 <= tile) lo = mid;
+    else hi = mid - 1;
+  }
+  return msgs[lo];
+}
 // Every decode of the library (pcop_accumulate_pointcloud2 / pcop_pointcloud2_to_xyz: one message; the batched
 // PointCloud2 wave: every message of its windows).  A 1-D grid over record tiles of PC2_TILE records: message m owns
 // tiles tile0 .. tile0 + cdiv(n, PC2_TILE) - 1 (empty messages own none), so a block finds its message by a binary
@@ -59,13 +69,7 @@ __device__ __forceinline__ float4 pc2_point(const Pc2Frame& d, float x, float y,
 __global__ void __launch_bounds__(PC2_THREADS)
     k_pc2_ingest(const Pc2Frame* __restrict__ msgs, int n_msgs, float4* __restrict__ out) {
   const int tile = blockIdx.x;
-  int lo = 0, hi = n_msgs - 1;  // the last message whose first tile is <= tile
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (msgs[mid].tile0 <= tile) lo = mid;
-    else hi = mid - 1;
-  }
-  const Pc2Frame& d = msgs[lo];
+  const Pc2Frame& d = tile_msg(msgs, n_msgs, tile);
   const int base = (tile - d.tile0) * PC2_TILE;
   const int n = d.n - base;  // (> 0)
   const unsigned char* rec0 = d.data + (size_t)base * (size_t)d.point_step;
@@ -95,6 +99,74 @@ __global__ void __launch_bounds__(PC2_THREADS)
   }
 }
 
+// sensor_msgs/Image (16UC1 millimetres or 32FC1 metres) + pinhole model -> pcl::PointXYZ, as depth_image_proc's
+// convert<T> builds its cloud [+ world transform]: pixel (u, v) is point v * width + u; a pixel without a return (0, or
+// non-finite) is a NaN point, otherwise x = ((float)u - center_x) * depth * kx, y likewise with v, each op rounded to
+// float, z = depth * 0.001f (16UC1) or depth (32FC1); padding float 1.0f.  The cloud is not dense: NaN points stay
+// untransformed (pc2_point).
+__device__ __forceinline__ float depth_load(const Pc2Frame& d, const unsigned char* p) {  // one pixel, any alignment
+  if (d.encoding != PCOP_DEPTH_16UC1) return pc2_load_f32(p);
+  if ((reinterpret_cast<uintptr_t>(p) & 1u) == 0u) return (float)__ldg(reinterpret_cast<const unsigned short*>(p));
+  return (float)((uint32_t)p[0] | ((uint32_t)p[1] << 8));
+}
+__device__ __forceinline__ float4 depth_point(const Pc2Frame& d, int u, int v, float depth) {
+  const bool u16 = d.encoding == PCOP_DEPTH_16UC1;
+  if (u16 ? depth == 0.0f : !(fabsf(depth) <= 3.402823466e+38f)) {
+    const float q = __int_as_float(0x7fc00000);
+    return pc2_point(d, q, q, q);
+  }
+  return pc2_point(d, fmul(fmul(fsub((float)u, d.center_x), depth), d.kx), fmul(fmul(fsub((float)v, d.center_y), depth), d.ky),
+                   u16 ? fmul(depth, 0.001f) : depth);
+}
+// The depth-image decode, in the launch shape of k_pc2_ingest: a 1-D grid over tiles of PC2_TILE pixels (row-major
+// over the image), the image found by tile_msg, pixel i of image m to out[dst + i].  aligned = 1 (width a multiple of
+// the pixels of one 16-byte load, step % 16 == 0, 16-byte aligned base): the tile's pixels come in with 16-byte loads
+// along the rows (8 of 16UC1, 4 of 32FC1; a load never spans two rows) into shared memory, and every thread then
+// stores its PC2_ITEMS points, so the stores of a warp stay contiguous; otherwise every thread loads its own pixels.
+__global__ void __launch_bounds__(PC2_THREADS)
+    k_depth_ingest(const Pc2Frame* __restrict__ msgs, int n_msgs, float4* __restrict__ out) {
+  __shared__ __align__(16) float s_depth[PC2_TILE];
+  const int tile = blockIdx.x;
+  const Pc2Frame& d = tile_msg(msgs, n_msgs, tile);
+  const int base = (tile - d.tile0) * PC2_TILE;
+  const int n = min(d.n - base, PC2_TILE);  // (> 0; with aligned, a multiple of the pixels per load)
+  const int bpp = d.encoding == PCOP_DEPTH_16UC1 ? 2 : 4;
+  float4* o = out + d.dst + base;
+  if (d.aligned) {
+    const int per = 16 / bpp;
+    for (int i = threadIdx.x * per; i < n; i += PC2_THREADS * per) {
+      const int p = base + i, v = p / d.width, u = p - v * d.width;
+      const uint4 q = __ldg(reinterpret_cast<const uint4*>(d.data + (size_t)v * (size_t)d.step + (size_t)u * bpp));
+      if (bpp == 2) {  // (little-endian: the first pixel of a word is its low half)
+        *reinterpret_cast<float4*>(&s_depth[i]) =
+            make_float4((float)(q.x & 0xffffu), (float)(q.x >> 16), (float)(q.y & 0xffffu), (float)(q.y >> 16));
+        *reinterpret_cast<float4*>(&s_depth[i + 4]) =
+            make_float4((float)(q.z & 0xffffu), (float)(q.z >> 16), (float)(q.w & 0xffffu), (float)(q.w >> 16));
+      } else {
+        *reinterpret_cast<float4*>(&s_depth[i]) =
+            make_float4(__uint_as_float(q.x), __uint_as_float(q.y), __uint_as_float(q.z), __uint_as_float(q.w));
+      }
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int k = 0; k < PC2_ITEMS; ++k) {
+    const int i = k * PC2_THREADS + threadIdx.x;
+    if (i < n) {
+      const int p = base + i, v = p / d.width, u = p - v * d.width;
+      const float depth = d.aligned ? s_depth[i] : depth_load(d, d.data + (size_t)v * (size_t)d.step + (size_t)u * bpp);
+      o[i] = depth_point(d, u, v, depth);
+    }
+  }
+}
+
+void set_pose(Pc2Frame& d, const float* t16, int is_dense) {
+  d.is_dense = is_dense ? 1 : 0;
+  d.apply_transform = t16 ? 1 : 0;
+  const float ident[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};
+  memcpy(d.t.m, t16 ? t16 : ident, sizeof(d.t.m));
+}
+
 // the descriptor of one message whose payload sits at `src` on the device (validated by the caller); its place in the
 // launch (dst, tile0) is set by the caller
 Pc2Frame make_pc2_frame(const unsigned char* src, int n, int point_step, int ox, int oy, int oz, const float* t16,
@@ -106,13 +178,31 @@ Pc2Frame make_pc2_frame(const unsigned char* src, int n, int point_step, int ox,
   d.off_x = ox;
   d.off_y = oy;
   d.off_z = oz;
-  d.is_dense = is_dense ? 1 : 0;
-  d.apply_transform = t16 ? 1 : 0;
-  const float ident[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};
-  memcpy(d.t.m, t16 ? t16 : ident, sizeof(d.t.m));
+  set_pose(d, t16, is_dense);
   const bool word4 = (ox & 3) == 0 && (oy & 3) == 0 && (oz & 3) == 0;
   const bool one_word = (ox >> 4) == (oy >> 4) && (ox >> 4) == (oz >> 4);
   d.aligned = (point_step % 16 == 0 && (reinterpret_cast<uintptr_t>(src) & 15u) == 0u && word4 && one_word) ? 1 : 0;
+  return d;
+}
+
+// the same for a depth image; the back-projection constants as depth_image_proc computes them on the host
+// (image_geometry's fx() .. cy() are doubles, DepthTraits<T>::toMeters(T(1)) a float widened to double)
+Pc2Frame make_depth_frame(const unsigned char* src, const pcop_depth_image& im, const float* t16) {
+  Pc2Frame d{};
+  d.data = src;
+  d.n = im.width * im.height;
+  d.width = im.width;
+  d.step = im.step;
+  d.encoding = im.encoding;
+  set_pose(d, t16, /*is_dense=*/0);  // (depth_image_proc publishes is_dense = false)
+  const bool u16 = im.encoding == PCOP_DEPTH_16UC1;
+  const double unit = u16 ? (double)0.001f : 1.0;
+  d.center_x = (float)im.cx;
+  d.center_y = (float)im.cy;
+  d.kx = (float)(unit / im.fx);
+  d.ky = (float)(unit / im.fy);
+  const int per = 16 / depth_pixel_bytes(im.encoding);
+  d.aligned = (im.width % per == 0 && im.step % 16 == 0 && (reinterpret_cast<uintptr_t>(src) & 15u) == 0u) ? 1 : 0;
   return d;
 }
 
@@ -485,12 +575,10 @@ int run_wave_cluster(Lane* l, int B, int max_n, const WaveRoute& r) {
   return PCOP_OK;
 }
 
-size_t pc2_payload_bytes(const pcop_pointcloud2_frame& m) { return (size_t)m.n_points * (size_t)m.point_step; }
-
-// PointCloud2 wave, input half: the descriptors of every message of the wave's windows go up through the pinned staging
-// (the lane's previous wave no longer reads it), every host payload into the lane's raw staging at a 256-byte aligned
-// offset, device payloads are read in place; one k_pc2_ingest launch decodes (and transforms) every message into its
-// frame's slot of d_in, after the messages before it in its window.  A repeat of the wave (voxel decline) decodes again
+// PointCloud2 / depth-image wave, input half: the descriptors of every message of the wave's windows go up through the
+// pinned staging (the lane's previous wave no longer reads it), every host payload into the lane's raw staging at a
+// 256-byte aligned offset, device payloads are read in place; one k_pc2_ingest (k_depth_ingest) launch decodes (and
+// transforms) every message into its frame's slot of d_in, after the messages before it in its window.  A repeat of the wave (voxel decline) decodes again
 // from the same staging -- the plane stage has overwritten d_in, the staging is intact.
 int enqueue_wave_decode(Lane* l, const Pc2Call& pc, int w0, int B, int max_n, bool repeat) {
   pcop_handle* h = l->h;
@@ -501,21 +589,25 @@ int enqueue_wave_decode(Lane* l, const Pc2Call& pc, int w0, int B, int max_n, bo
     for (int f = 0; f < B; ++f) {
       size_t dst = (size_t)f * (size_t)h->cap;
       for (int k = pc.window_first[w0 + f]; k < pc.window_first[w0 + f + 1]; ++k) {
-        const pcop_pointcloud2_frame& m = pc.msgs[k];
-        const size_t bytes = pc2_payload_bytes(m);
-        const unsigned char* src = m.data;
+        const size_t bytes = pc.payload_bytes(k);
+        const unsigned char* src = pc.data(k);
         if (bytes > 0 && !pc.on_device[k]) {
-          PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_raw + off, m.data, bytes, cudaMemcpyHostToDevice, l->stream));
+          PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_raw + off, src, bytes, cudaMemcpyHostToDevice, l->stream));
           src = l->d_raw + off;
           off += (bytes + 255) & ~(size_t)255;
         }
+        const float* t16 = pc.transform16 ? pc.transform16 + (size_t)k * 16 : nullptr;
         Pc2Frame& d = l->h_pc2[k - m0];
-        d = make_pc2_frame(src, m.n_points, m.point_step, m.off_x, m.off_y, m.off_z,
-                           pc.transform16 ? pc.transform16 + (size_t)k * 16 : nullptr, m.is_dense);
+        if (pc.images) {
+          d = make_depth_frame(src, pc.images[k], t16);
+        } else {
+          const pcop_pointcloud2_frame& m = pc.msgs[k];
+          d = make_pc2_frame(src, m.n_points, m.point_step, m.off_x, m.off_y, m.off_z, t16, m.is_dense);
+        }
         d.dst = dst;
         d.tile0 = tiles;
-        dst += (size_t)m.n_points;
-        tiles += cdiv(m.n_points, PC2_TILE);
+        dst += (size_t)d.n;
+        tiles += cdiv(d.n, PC2_TILE);
       }
     }
     l->pc2_msgs = pc.window_first[w0 + B] - m0;
@@ -525,7 +617,10 @@ int enqueue_wave_decode(Lane* l, const Pc2Call& pc, int w0, int B, int max_n, bo
   }
   if (l->pc2_tiles > 0) {  // (a wave of empty windows decodes nothing)
     Ctx c = make_ctx(l, B, max_n);
-    KL(c, "k_pc2_ingest", k_pc2_ingest<<<l->pc2_tiles, PC2_THREADS, 0, l->stream>>>(l->d_pc2, l->pc2_msgs, l->d_in));
+    if (pc.images)
+      KL(c, "k_depth_ingest", k_depth_ingest<<<l->pc2_tiles, PC2_THREADS, 0, l->stream>>>(l->d_pc2, l->pc2_msgs, l->d_in));
+    else
+      KL(c, "k_pc2_ingest", k_pc2_ingest<<<l->pc2_tiles, PC2_THREADS, 0, l->stream>>>(l->d_pc2, l->pc2_msgs, l->d_in));
     count_launch(c);
   }
   return PCOP_OK;
@@ -857,8 +952,7 @@ int finish_wave(Lane* l, const WaveInput& wi, uint32_t mask, pcop_frame_result* 
     double b = 0.0;
     const pcop_params& p = h->params;
     if (wi.pc2)  // the decode: every message's payload in, PointXYZ out
-      for (int k = wi.pc2->window_first[w0 + f]; k < wi.pc2->window_first[w0 + f + 1]; ++k)
-        b += (double)(wi.pc2->msgs[k].point_step + 16) * wi.pc2->msgs[k].n_points;
+      for (int k = wi.pc2->window_first[w0 + f]; k < wi.pc2->window_first[w0 + f + 1]; ++k) b += wi.pc2->decode_bytes(k);
     if (p.enable_crop) b += 16.0 * r.n_input + 20.0 * r.n_crop;
     if (p.enable_voxel) b += 16.0 * r.n_crop + 20.0 * r.n_voxel;
     if (p.enable_sor) b += 16.0 * r.n_voxel + 20.0 * r.n_sor;
@@ -934,14 +1028,14 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
       w0 += B;
     }
   }
-  // PointCloud2 messages: host payload bytes of the largest wave, as staged (256-byte aligned), and its message count
+  // PointCloud2 messages / depth images: host payload bytes of the largest wave, as staged (256-byte aligned), and its message count
   size_t raw_need = 0, pc2_need = 0;
   if (pc2)
     for (const auto& w : waves) {
       size_t bytes = 0;
       const int m0 = pc2->window_first[w.first], m1 = pc2->window_first[w.first + w.second];
       for (int k = m0; k < m1; ++k)
-        if (!pc2->on_device[k]) bytes += (pc2_payload_bytes(pc2->msgs[k]) + 255) & ~(size_t)255;
+        if (!pc2->on_device[k]) bytes += (pc2->payload_bytes(k) + 255) & ~(size_t)255;
       raw_need = std::max(raw_need, bytes);
       pc2_need = std::max(pc2_need, (size_t)(m1 - m0));
     }
@@ -1041,26 +1135,40 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
   return PCOP_OK;
 }
 
-int pc2_ingest(pcop_handle* h, const unsigned char* data, int32_t n, int32_t point_step, int32_t ox, int32_t oy,
-               int32_t oz, const float* t16, int is_dense, float4* dst) {
-  if (!pc2_layout_ok(point_step, ox, oy, oz)) return fail(h, PCOP_ERR_BAD_PARAM, "PointCloud2 field offsets do not fit point_step");
+// one message into dst (lane 0): a host payload is staged through d_raw, the descriptor goes up from pageable memory
+// (staged before the call returns), and the batched decode runs with one descriptor
+template <class MakeFrame>
+static int ingest_one(pcop_handle* h, const unsigned char* data, size_t bytes, bool depth, MakeFrame make, float4* dst) {
   Lane* l = h->lanes[0].get();
-  const size_t bytes = (size_t)n * (size_t)point_step;
   const unsigned char* src = data;
   if (!is_device_pointer(data)) {
     TRY(grow_raw(l, bytes));
     PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_raw, data, bytes, cudaMemcpyHostToDevice, l->stream));
     src = l->d_raw;
   }
-  // the batched decode with one message; the descriptor goes up from pageable memory (staged before the call returns)
   TRY(grow(l, l->d_pc2, 1));
-  const Pc2Frame d = make_pc2_frame(src, n, point_step, ox, oy, oz, t16, is_dense);  // (dst = 0, tile0 = 0)
+  const Pc2Frame d = make(src);  // (dst = 0, tile0 = 0)
   PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_pc2, &d, sizeof(d), cudaMemcpyHostToDevice, l->stream));
-  Ctx c = make_ctx(l, 1, n);
-  KL(c, "k_pc2_ingest", k_pc2_ingest<<<cdiv(n, PC2_TILE), PC2_THREADS, 0, l->stream>>>(l->d_pc2, 1, dst));
+  Ctx c = make_ctx(l, 1, d.n);
+  if (depth)
+    KL(c, "k_depth_ingest", k_depth_ingest<<<cdiv(d.n, PC2_TILE), PC2_THREADS, 0, l->stream>>>(l->d_pc2, 1, dst));
+  else
+    KL(c, "k_pc2_ingest", k_pc2_ingest<<<cdiv(d.n, PC2_TILE), PC2_THREADS, 0, l->stream>>>(l->d_pc2, 1, dst));
   count_launch(c);
   if (src != data) PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));  // the caller may reuse its buffer
   return PCOP_OK;
+}
+
+int pc2_ingest(pcop_handle* h, const unsigned char* data, int32_t n, int32_t point_step, int32_t ox, int32_t oy,
+               int32_t oz, const float* t16, int is_dense, float4* dst) {
+  if (!pc2_layout_ok(point_step, ox, oy, oz)) return fail(h, PCOP_ERR_BAD_PARAM, "PointCloud2 field offsets do not fit point_step");
+  return ingest_one(h, data, (size_t)n * (size_t)point_step, false,
+                    [&](const unsigned char* src) { return make_pc2_frame(src, n, point_step, ox, oy, oz, t16, is_dense); }, dst);
+}
+
+int depth_ingest(pcop_handle* h, const pcop_depth_image& im, const float* t16, float4* dst) {
+  return ingest_one(h, im.data, (size_t)im.step * (size_t)im.height, true,
+                    [&](const unsigned char* src) { return make_depth_frame(src, im, t16); }, dst);
 }
 
 }  // namespace pcop

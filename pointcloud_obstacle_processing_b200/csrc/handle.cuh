@@ -65,15 +65,20 @@ struct PackMeta {  // device -> host in one copy
   int overflow;     // the wave's arrays do not fit the pack buffer (nothing was packed)
 };
 
-struct Pc2Frame {  // decode descriptor of one PointCloud2 message (device memory, read by k_pc2_ingest)
+// decode descriptor of one message (device memory): a PointCloud2 message, read by k_pc2_ingest, or a depth image,
+// read by k_depth_ingest (n = width * height pixels; point_step and the field offsets unused)
+struct Pc2Frame {
   const unsigned char* data;  // payload on the device
   size_t dst;                 // element offset of the message's first decoded point in the output
   int n, point_step, off_x, off_y, off_z;
-  int is_dense, apply_transform, aligned;
+  int is_dense, apply_transform, aligned;  // depth image: aligned = 16-byte loads along its rows
   int tile0;                  // the message's first record tile (PC2_TILE records each) in the launch
   Mat34 t;
+  // depth image only: Image.width, Image.step, PCOP_DEPTH_*, and the back-projection constants of depth_image_proc
+  int width, step, encoding;
+  float center_x, center_y, kx, ky;
 };
-constexpr int PC2_THREADS = 256, PC2_ITEMS = 4, PC2_TILE = PC2_THREADS * PC2_ITEMS;  // k_pc2_ingest
+constexpr int PC2_THREADS = 256, PC2_ITEMS = 4, PC2_TILE = PC2_THREADS * PC2_ITEMS;  // k_pc2_ingest, k_depth_ingest
 
 // the grid product of a batched call (pcop_process_batch_occupancy, pcop_process_batch_pointcloud2 with grids)
 struct OccCall {
@@ -84,12 +89,26 @@ struct OccCall {
   bool grids_on_device;
 };
 
-// the messages of a pcop_process_batch_pointcloud2_windows call
+inline int depth_pixel_bytes(int encoding) { return encoding == PCOP_DEPTH_16UC1 ? 2 : 4; }
+
+// the messages of a pcop_process_batch_pointcloud2_windows call, or the images of a pcop_process_batch_depth_windows call
 struct Pc2Call {
   const pcop_pointcloud2_frame* msgs;
+  const pcop_depth_image* images = nullptr;  // non-null: the messages are depth images (msgs unused)
   const int32_t* window_first;    // [batch + 1]: frame f = messages window_first[f] .. window_first[f + 1] - 1
   const float* transform16;       // [messages][16] or nullptr
   std::vector<char> on_device;    // per message: the payload is a device pointer (used in place)
+
+  int points(int k) const { return images ? images[k].width * images[k].height : msgs[k].n_points; }
+  const unsigned char* data(int k) const { return images ? images[k].data : msgs[k].data; }
+  size_t payload_bytes(int k) const {  // (an image of 0 pixels uploads nothing, whatever its step)
+    if (!images) return (size_t)msgs[k].n_points * (size_t)msgs[k].point_step;
+    return points(k) > 0 ? (size_t)images[k].step * (size_t)images[k].height : 0;
+  }
+  double decode_bytes(int k) const {  // algorithmic bytes of the decode: the payload's records in, PointXYZ out
+    const int in = images ? depth_pixel_bytes(images[k].encoding) : msgs[k].point_step;
+    return (double)(in + 16) * points(k);
+  }
 };
 
 struct WaveInput {
@@ -584,6 +603,7 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
                  pcop_frame_result* out, const OccCall* occ = nullptr, const Pc2Call* pc2 = nullptr);
 int pc2_ingest(pcop_handle* h, const unsigned char* data, int32_t n, int32_t point_step, int32_t ox, int32_t oy,
                int32_t oz, const float* t16, int is_dense, float4* dst);
+int depth_ingest(pcop_handle* h, const pcop_depth_image& im, const float* t16, float4* dst);  // (validated image)
 __global__ void k_zero_u32(uint32_t* p, int n);  // batch.cu; upload_single zeroes one frame's warning word with it
 
 }  // namespace pcop

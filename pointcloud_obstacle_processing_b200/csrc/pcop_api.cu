@@ -475,14 +475,29 @@ int pcop_process_batch_occupancy(pcop_handle* h, const float* xyzw, size_t frame
   return st;
 }
 
-// pcop_process_batch_pointcloud2_windows, and pcop_process_batch_pointcloud2 with one message per window (`who` names
-// the entry point in error messages)
-static int pointcloud2_windows(pcop_handle* h, const char* who, const pcop_pointcloud2_frame* msgs, int32_t n_msgs,
-                               const int32_t* window_first, int32_t batch, const float* transform16,
-                               const float* world_to_sensor16, const float* sensor_to_world16, int8_t* grids,
-                               pcop_frame_result* out) {
+// the checks of one depth image ("" when it is well formed)
+static std::string depth_image_error(const pcop_depth_image& im) {
+  if (im.width < 0 || im.height < 0) return "negative width or height";
+  if (!im.data && (long long)im.width * im.height > 0) return "NULL data with pixels";
+  if (im.encoding != PCOP_DEPTH_16UC1 && im.encoding != PCOP_DEPTH_32FC1) return "unknown encoding";
+  const int bpp = depth_pixel_bytes(im.encoding);
+  if ((long long)im.step < (long long)im.width * bpp || im.step % bpp != 0)
+    return "step below width * sizeof(T) or not a multiple of sizeof(T)";
+  if (!std::isfinite(im.fx) || !std::isfinite(im.fy) || im.fx == 0.0 || im.fy == 0.0 || !std::isfinite(im.cx) ||
+      !std::isfinite(im.cy))
+    return "fx / fy zero or non-finite, or cx / cy non-finite";
+  return "";
+}
+
+// pcop_process_batch_pointcloud2_windows, pcop_process_batch_pointcloud2 with one message per window, and
+// pcop_process_batch_depth_windows (pc.images set: the messages are depth images); `who` names the entry point in
+// error messages
+static int windows_call(pcop_handle* h, const char* who, Pc2Call& pc, int32_t n_msgs, int32_t batch,
+                        const float* world_to_sensor16, const float* sensor_to_world16, int8_t* grids,
+                        pcop_frame_result* out) {
   const std::string w(who);
-  if (!out || batch < 0 || n_msgs < 0 || (!msgs && n_msgs > 0) || (!window_first && (batch > 0 || n_msgs > 0)) ||
+  const int32_t* window_first = pc.window_first;
+  if (!out || batch < 0 || n_msgs < 0 || (!pc.msgs && !pc.images && n_msgs > 0) || (!window_first && (batch > 0 || n_msgs > 0)) ||
       (grids && (!world_to_sensor16 || !sensor_to_world16)))
     return fail(h, PCOP_ERR_BAD_PARAM, w + ": null argument (grids need world_to_sensor16 and sensor_to_world16)");
   if (window_first && (window_first[0] != 0 || window_first[batch] != n_msgs))
@@ -496,7 +511,14 @@ static int pointcloud2_windows(pcop_handle* h, const char* who, const pcop_point
   for (int f = 0; f < batch; ++f) {
     long long total = 0;
     for (int m = window_first[f]; m < window_first[f + 1]; ++m) {
-      const pcop_pointcloud2_frame& d = msgs[m];
+      if (pc.images) {
+        const pcop_depth_image& im = pc.images[m];
+        const std::string e = depth_image_error(im);
+        if (!e.empty()) return fail(h, PCOP_ERR_BAD_PARAM, w + ": image " + std::to_string(m) + ": " + e);
+        total += (long long)im.width * im.height;
+        continue;
+      }
+      const pcop_pointcloud2_frame& d = pc.msgs[m];
       if (d.n_points < 0 || (!d.data && d.n_points > 0))
         return fail(h, PCOP_ERR_BAD_PARAM, w + ": message " + std::to_string(m) + ": bad count or NULL data");
       if (!pc2_layout_ok(d.point_step, d.off_x, d.off_y, d.off_z))
@@ -512,14 +534,21 @@ static int pointcloud2_windows(pcop_handle* h, const char* who, const pcop_point
   OccCall oc{};
   if (grids) TRY(occ_call_of(h, who, world_to_sensor16, sensor_to_world16, grids, &oc));
   PCOP_CUDA_TRY(cudaSetDevice(h->device));
+  pc.on_device.resize((size_t)n_msgs);
+  PayloadClassifier on_device;
+  for (int m = 0; m < n_msgs; ++m) pc.on_device[m] = pc.points(m) > 0 && on_device(pc.data(m));
+  return process_impl(h, nullptr, (size_t)h->cap, n.data(), batch, out, grids ? &oc : nullptr, &pc);
+}
+
+static int pointcloud2_windows(pcop_handle* h, const char* who, const pcop_pointcloud2_frame* msgs, int32_t n_msgs,
+                               const int32_t* window_first, int32_t batch, const float* transform16,
+                               const float* world_to_sensor16, const float* sensor_to_world16, int8_t* grids,
+                               pcop_frame_result* out) {
   Pc2Call pc;
   pc.msgs = msgs;
   pc.window_first = window_first;
   pc.transform16 = transform16;
-  pc.on_device.resize((size_t)n_msgs);
-  PayloadClassifier on_device;
-  for (int m = 0; m < n_msgs; ++m) pc.on_device[m] = msgs[m].n_points > 0 && on_device(msgs[m].data);
-  return process_impl(h, nullptr, (size_t)h->cap, n.data(), batch, out, grids ? &oc : nullptr, &pc);
+  return windows_call(h, who, pc, n_msgs, batch, world_to_sensor16, sensor_to_world16, grids, out);
 }
 
 int pcop_process_batch_pointcloud2_windows(pcop_handle* h, const pcop_pointcloud2_frame* messages, int32_t n_messages,
@@ -539,6 +568,20 @@ int pcop_process_batch_pointcloud2(pcop_handle* h, const pcop_pointcloud2_frame*
   for (size_t f = 0; f < first.size(); ++f) first[f] = (int32_t)f;
   return pointcloud2_windows(h, "pcop_process_batch_pointcloud2", frames, batch, first.data(), batch, transform16,
                              world_to_sensor16, sensor_to_world16, grids, out);
+}
+
+int pcop_process_batch_depth_windows(pcop_handle* h, const pcop_depth_image* images, int32_t n_images,
+                                     const int32_t* window_first, int32_t batch, const float* transform16,
+                                     const float* world_to_sensor16, const float* sensor_to_world16, int8_t* grids,
+                                     pcop_frame_result* out) {
+  if (!h) return fail(nullptr, PCOP_ERR_BAD_PARAM, "null handle");
+  Pc2Call pc;
+  pc.msgs = nullptr;
+  pc.images = images;
+  pc.window_first = window_first;
+  pc.transform16 = transform16;
+  return windows_call(h, "pcop_process_batch_depth_windows", pc, n_images, batch, world_to_sensor16, sensor_to_world16,
+                      grids, out);
 }
 
 int pcop_enable_kernel_timing(pcop_handle* h, int enable) {
@@ -661,6 +704,34 @@ int pcop_pointcloud2_to_xyz(pcop_handle* h, const unsigned char* data, int32_t n
   Lane* l = h->lanes[0].get();
   TRY(pc2_ingest(h, data, n_points, point_step, off_x, off_y, off_z, nullptr, 1, l->d_crop));
   TRY(download(h, out_xyzw, l->d_crop, (size_t)n_points * 16));
+  PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
+  return PCOP_OK;
+}
+
+int pcop_accumulate_depth_image(pcop_handle* h, const pcop_depth_image* image, const float* transform16, int32_t* total) {
+  if (!h || !image) return fail(h, PCOP_ERR_BAD_PARAM, "pcop_accumulate_depth_image: null argument");
+  const std::string e = depth_image_error(*image);
+  if (!e.empty()) return fail(h, PCOP_ERR_BAD_PARAM, "pcop_accumulate_depth_image: " + e);
+  const long long n = (long long)image->width * image->height;
+  if (h->acc_count + n > h->cap) return fail(h, PCOP_ERR_CAPACITY, "accumulated cloud exceeds max_points");
+  PCOP_CUDA_TRY(cudaSetDevice(h->device));
+  if (n > 0) TRY(depth_ingest(h, *image, transform16, h->d_acc + h->acc_count));
+  h->acc_count += (int32_t)n;
+  if (total) *total = h->acc_count;
+  return PCOP_OK;
+}
+
+int pcop_depth_image_to_xyz(pcop_handle* h, const pcop_depth_image* image, float* out_xyzw) {
+  if (!h || !image || !out_xyzw) return fail(h, PCOP_ERR_BAD_PARAM, "null argument");
+  const std::string e = depth_image_error(*image);
+  if (!e.empty()) return fail(h, PCOP_ERR_BAD_PARAM, "pcop_depth_image_to_xyz: " + e);
+  const long long n = (long long)image->width * image->height;
+  if (n > h->cap) return fail(h, PCOP_ERR_CAPACITY, "image has more pixels than max_points");
+  PCOP_CUDA_TRY(cudaSetDevice(h->device));
+  if (n == 0) return PCOP_OK;
+  Lane* l = h->lanes[0].get();
+  TRY(depth_ingest(h, *image, nullptr, l->d_crop));
+  TRY(download(h, out_xyzw, l->d_crop, (size_t)n * 16));
   PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
   return PCOP_OK;
 }

@@ -25,6 +25,8 @@ def _load():
         lib.pcop_synth_frame.argtypes = [C.c_int, C.c_int, C.c_void_p]
         lib.pcop_synth_params.restype = C.c_int
         lib.pcop_synth_params.argtypes = [C.c_int, C.POINTER(Params)]
+        lib.pcop_synth_depth_camera.restype = None
+        lib.pcop_synth_depth_camera.argtypes = [C.c_int, C.c_int, C.c_int] + [C.c_double] * 4 + [C.c_void_p]
         _lib = lib
     return _lib
 
@@ -60,4 +62,13 @@ def frames(config: int, first: int, count: int, out: np.ndarray = None, threads:
     threads = threads or min(32, os.cpu_count() or 1)
     with ThreadPoolExecutor(max_workers=threads) as ex:
         list(ex.map(lambda k: frame(config, first + k, out[k]), range(count)))
+    return out
+
+
+def depth_camera_frame(index: int, width: int, height: int, fx: float, fy: float, cx: float, cy: float) -> np.ndarray:
+    """Config 3's scene of frame `index` seen by another pinhole camera: float32 [height * width, 4] in the camera
+    frame, point v * width + u = pixel (u, v), NaN where the camera has no return.  The 640 x 480 camera at fx = fy =
+    525, cx = 319.5, cy = 239.5 gives frame(3, index)."""
+    out = np.empty((width * height, 4), dtype=np.float32)
+    _load().pcop_synth_depth_camera(index, width, height, fx, fy, cx, cy, out.ctypes.data_as(C.c_void_p))
     return out

@@ -211,7 +211,8 @@ void gen_hdl64(uint64_t seed, float* out) {
 }
 
 // config 3: organized 640x480 depth image, camera frame (x right, y down, z forward)
-void gen_depth(uint64_t seed, float* out) {
+// config 3's scene seen by a pinhole camera of W x H pixels: point v * W + u is pixel (u, v) in the camera frame
+void gen_depth_camera(uint64_t seed, int W, int H, double fx, double fy, double cx, double cy, float* out) {
   Rng rng(seed);
   // build the scene in a z-up world, camera at the origin looking along world +x:
   //   cam z = world x, cam x = -world y, cam y = -world z
@@ -227,11 +228,10 @@ void gen_depth(uint64_t seed, float* out) {
     else
       sc.spheres.push_back({{wx, wy, -1.0 + sz / 2}, sz / 2});
   }
-  const double fx = 525.0, fy = 525.0, cx = 319.5, cy = 239.5;
   const double o[3] = {0.0, 0.0, 0.0};
   int i = 0;
-  for (int v = 0; v < 480; ++v)
-    for (int u = 0; u < 640; ++u, ++i) {
+  for (int v = 0; v < H; ++v)
+    for (int u = 0; u < W; ++u, ++i) {
       const double xc = ((double)u - cx) / fx, yc = ((double)v - cy) / fy;  // cam ray (xc, yc, 1)
       const double dw[3] = {1.0, -xc, -yc};                                 // world dir, un-normalised
       const double nrm = std::sqrt(dw[0] * dw[0] + dw[1] * dw[1] + dw[2] * dw[2]);
@@ -252,6 +252,8 @@ void gen_depth(uint64_t seed, float* out) {
       put(out, i, xc * z, yc * z, z);
     }
 }
+
+void gen_depth(uint64_t seed, float* out) { gen_depth_camera(seed, 640, 480, 525.0, 525.0, 319.5, 239.5, out); }
 
 // config 4: adversarial 1 M points: 3 dense blobs + a 50 k-point snake + 50 k noise
 void gen_adversarial(uint64_t seed, float* out, int n) {
@@ -351,6 +353,11 @@ int32_t pcop_synth_frame(int config, int frame, float* out) {
     default: return -1;
   }
   return pcop_synth_points(config);
+}
+
+// config 3's scene of frame `frame` through another pinhole camera (W x H points into out[W * H * 4])
+void pcop_synth_depth_camera(int frame, int W, int H, double fx, double fy, double cx, double cy, float* out) {
+  gen_depth_camera(pcop_synth_seed(3, frame), W, H, fx, fy, cx, cy, out);
 }
 
 // the parameter set each config runs with (SURVEY 8d table)
