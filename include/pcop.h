@@ -79,6 +79,9 @@ enum {
   PCOP_OUT_OBSTACLES = 64, /* obstacles                                   */
   PCOP_OUT_DEFAULT = 16 | 32 | 64,
   PCOP_OUT_ALL = 127,
+  /* per-cluster box and ground-plane convex hull (pcop_last_footprints below).  Not part of PCOP_OUT_ALL, so
+   * publish_point_clouds does not switch it on; dropped when clustering is off.  (Releases before it ignored bit 128.) */
+  PCOP_OUT_FOOTPRINTS = 128,
   /* Modifier: leave the requested arrays in device memory.  The pcop_frame_result pointers are then DEVICE pointers
    * (valid until the next pcop_process* call on the handle; counts, warnings and the plane record are still host
    * values) for a consumer that lives on the GPU: the next GPU stage, a peer-to-peer / NCCL transfer,
@@ -437,6 +440,47 @@ int pcop_process_batch_depth_windows(pcop_handle* h, const pcop_depth_image* ima
                                      pcop_frame_result* out);
 int pcop_accumulate_depth_image(pcop_handle* h, const pcop_depth_image* image, const float* transform16, int32_t* total);
 int pcop_depth_image_to_xyz(pcop_handle* h, const pcop_depth_image* image, float* out_xyzw);
+
+/* ---- obstacle footprints: per-cluster bounding box and ground-plane convex hull (PCOP_OUT_FOOTPRINTS) ---------------
+ * A planner wants an obstacle's footprint on the ground plane (a polygon for costmap_converter / TEB obstacle messages or
+ * geometry_msgs/PolygonStamped, a box for BoundingBoxArray-style consumers), not the bounding sphere of `obstacles`.  With
+ * PCOP_OUT_FOOTPRINTS in pcop_params.outputs every pcop_process* call also computes, on the GPU inside the wave, for
+ * every cluster c of a frame, over its members remaining_cloud[cluster_indices[cluster_offsets[c] .. cluster_offsets[c+1]-1]]:
+ *   boxes[c]   float[8] = {min_x, min_y, min_z, 0, max_x, max_y, max_z, 0}, minima and maxima in IEEE totalOrder
+ *              (-0 < +0; bit-exact, order-independent).  A singleton's box is its member's coordinates copied, NaN / Inf
+ *              included (only a singleton can hold a non-finite point: clustering gives such a point no neighbours, so it
+ *              appears only with euc_min_cluster_size = 1).  An empty cluster (pcop_cluster_footprints only) has a box of
+ *              zeros and no hull vertices.
+ *   hull       the 2-D convex hull of the members projected along z (x, y; the occupancy grid's plane): its strictly
+ *              extreme points (a point on an edge is not a vertex), counter-clockwise seen from +z, starting at the
+ *              lexicographically smallest (x, then y) vertex.  Members with equal (x, y) (float ==, so -0 == +0) count once,
+ *              as the smallest remaining-cloud index among them.  All members at one point: 1 vertex; all collinear: 2
+ *              vertices, the lexicographic minimum first.  Orientations use Shewchuk's filtered orient2d with its exact
+ *              fallback, so the hull is exact and unique.  hull_offsets[C + 1] is a CSR over hull_indices[H], which hold
+ *              remaining-cloud indices (the index space of cluster_indices): resolving them needs PCOP_OUT_REMAINING.
+ * No oriented or minimum-area box and no concave hull; convex_hull_alpha stays accepted and ignored.
+ * pcop_last_footprints returns frame `frame` of the last pcop_process* call; its pointers live as long as that frame's
+ * pcop_frame_result pointers (alternating pinned buffers included) and are device pointers with PCOP_OUT_DEVICE.  Without
+ * the bit: PCOP_OK, NULL pointers and n_hull_vertices = 0.  PCOP_ERR_BAD_PARAM for NULL out, a frame outside the last
+ * call, or after a call that failed.
+ * pcop_cluster_footprints is the stage-isolated computation (host pointers in and out, as pcop_centroid_radius):
+ * boxes[c][8], hull_offsets[c + 1], hull_indices with room for cluster_offsets[c] entries, *n_hull = H.  PCOP_ERR_BAD_PARAM
+ * for NULL pointers, c < 0, cluster_offsets[0] != 0, decreasing offsets, cluster_offsets[c] > p or an index outside [0, p);
+ * PCOP_ERR_CAPACITY for p or c above max_points.
+ * The kernels count as PCOP_STAGE_CENTROID; pcop_last_d2h_bytes includes the three arrays; pcop_last_algorithmic_bytes
+ * adds 4 (C + 1) + 20 L bytes read and 32 C + 4 (C + 1) + 4 H written per frame.  Memory: every lane of the handle keeps
+ * 48 bytes per point of capacity and per frame of its waves (max_points x wave frames; boxes 32, hull sizes, offsets,
+ * staging and indices 4 each), allocated by the first call that asks for footprints, never by pcop_create. */
+typedef struct pcop_frame_footprints {
+  int32_t n_clusters, n_hull_vertices;
+  const float* boxes;           /* [C][8]                               */
+  const int32_t* hull_offsets;  /* [C+1]                                */
+  const int32_t* hull_indices;  /* [H] index into remaining_cloud       */
+} pcop_frame_footprints;
+int pcop_last_footprints(const pcop_handle* h, int32_t frame, pcop_frame_footprints* out);
+int pcop_cluster_footprints(pcop_handle* h, const float* xyzw, int32_t p, const int32_t* cluster_offsets,
+                            const int32_t* cluster_indices, int32_t c, float* boxes, int32_t* hull_offsets,
+                            int32_t* hull_indices, int32_t* n_hull);
 
 /* Copies `bytes` from a device result array (PCOP_OUT_DEVICE) to host memory, or device to device when dst is a device
  * pointer; synchronous. */

@@ -9,6 +9,7 @@ WARN_SHADOW_DEGENERATE = 16
 OCC_BATCH_MAX_CELLS = 1 << 20  # PCOP_OCC_BATCH_MAX_CELLS
 OUT_CROP, OUT_VOXEL, OUT_SOR, OUT_PLANE, OUT_REMAINING, OUT_CLUSTERS, OUT_OBSTACLES = 1, 2, 4, 8, 16, 32, 64
 OUT_DEFAULT, OUT_ALL = 16 | 32 | 64, 127
+OUT_FOOTPRINTS = 128  # per-cluster box + ground-plane convex hull (pcop_last_footprints); not part of OUT_ALL
 OUT_DEVICE = 256  # modifier: result arrays stay in device memory (pointers are device pointers)
 STAGE_NAMES = ["h2d", "crop", "voxel", "sor", "plane", "cluster", "centroid", "d2h"]
 
@@ -79,4 +80,14 @@ class FrameResult(C.Structure):
         ("cluster_offsets", C.POINTER(C.c_int32)),
         ("cluster_indices", C.POINTER(C.c_int32)),
         ("obstacles", C.POINTER(C.c_float)),
+    ]
+
+
+class FrameFootprints(C.Structure):
+    """pcop_frame_footprints: boxes [C][8], hull CSR over remaining-cloud indices."""
+    _fields_ = [
+        ("n_clusters", C.c_int32), ("n_hull_vertices", C.c_int32),
+        ("boxes", C.POINTER(C.c_float)),
+        ("hull_offsets", C.POINTER(C.c_int32)),
+        ("hull_indices", C.POINTER(C.c_int32)),
     ]

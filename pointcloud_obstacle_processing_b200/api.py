@@ -19,7 +19,7 @@ import os
 import numpy as np
 
 from . import _ctypes_abi as abi
-from ._ctypes_abi import DepthImageC, FrameResult, Params, PointCloud2Frame
+from ._ctypes_abi import DepthImageC, FrameFootprints, FrameResult, Params, PointCloud2Frame
 from .result import Frame
 
 
@@ -105,6 +105,8 @@ EXPORTS = [
     "pcop_process_batch_depth_windows",
     "pcop_accumulate_depth_image",
     "pcop_depth_image_to_xyz",
+    "pcop_last_footprints",
+    "pcop_cluster_footprints",
 ]
 
 
@@ -179,6 +181,8 @@ def load_library():
     L.pcop_plane.argtypes = [vp, vp, i32, vp, vp, pi32, pi32, vp, vp, vp, vp, vp, pi32, pu32]
     L.pcop_cluster.argtypes = [vp, vp, i32, vp, vp, pi32, pi32]
     L.pcop_centroid_radius.argtypes = [vp, vp, i32, vp, vp, i32, vp]
+    L.pcop_last_footprints.argtypes = [vp, i32, C.POINTER(FrameFootprints)]
+    L.pcop_cluster_footprints.argtypes = [vp, vp, i32, vp, vp, i32, vp, vp, vp, pi32]
     _lib = L
     return L
 
@@ -293,12 +297,22 @@ class ObstacleProcessor:
             raise ValueError("outputs | OUT_DEVICE leaves the result arrays on the GPU: call process_batch_raw() and "
                              "read them with download() / copy_device()")
 
+    def last_footprints(self, frame: int) -> FrameFootprints:
+        """pcop_last_footprints: frame `frame` of the last pcop_process* call (device pointers with OUT_DEVICE)"""
+        fp = FrameFootprints()
+        self._check(self._lib.pcop_last_footprints(self._h, frame, C.byref(fp)))
+        return fp
+
+    def _frames(self, res):
+        """Frames of the last call's host results, with their footprints"""
+        return [Frame.from_c(r).set_footprints(self.last_footprints(f)) for f, r in enumerate(res)]
+
     def process(self, cloud) -> Frame:
         self._host_results_only()
         cloud = _f32(cloud)
         r = FrameResult()
         self._check(self._lib.pcop_process(self._h, cloud.ctypes.data_as(C.c_void_p), cloud.shape[0], C.byref(r)))
-        return Frame.from_c(r)
+        return self._frames([r])[0]
 
     def process_batch_raw(self, ptr: int, frame_stride_points: int, counts: np.ndarray):
         """Frames at a raw host or device address; returns the ctypes result array (valid until the next call)."""
@@ -316,7 +330,7 @@ class ObstacleProcessor:
         if counts is None:
             counts = np.full(clouds.shape[0], clouds.shape[1], np.int32)
         res = self.process_batch_raw(clouds.ctypes.data, clouds.shape[1], counts)
-        return [Frame.from_c(r) for r in res]
+        return self._frames(res)
 
     # ---- pipeline + occupancy grid (the node's published product) --------------------------
     def occupancy_dims(self):
@@ -361,7 +375,7 @@ class ObstacleProcessor:
             ptr, stride = clouds.ctypes.data, clouds.shape[1]
         grids = np.empty((len(counts), h, w), np.int8)
         res = self.process_batch_occupancy_raw(ptr, stride, counts, world_to_sensor, sensor_to_world, grids.ctypes.data)
-        return [Frame.from_c(r) for r in res], grids
+        return self._frames(res), grids
 
     # ---- raw PointCloud2 messages, one pose each (od.cpp:688-696 + 699-852 per message) ------------------
     def process_batch_pointcloud2_raw(self, frames, transforms=None, world_to_sensor=None, sensor_to_world=None,
@@ -395,7 +409,7 @@ class ObstacleProcessor:
             g = np.empty((len(frames), h, w), np.int8)
         res = self.process_batch_pointcloud2_raw(frames, transforms, world_to_sensor, sensor_to_world,
                                                  None if g is None else g.ctypes.data)
-        out = [Frame.from_c(r) for r in res]
+        out = self._frames(res)
         return (out, g) if grids else out
 
     # ---- accumulation windows: several posed messages per frame (od.cpp:688-701 per processing callback) ----------
@@ -436,7 +450,7 @@ class ObstacleProcessor:
             g = np.empty((len(window_first) - 1, h, w), np.int8)
         res = self.process_batch_pointcloud2_windows_raw(frames, window_first, transforms, world_to_sensor,
                                                          sensor_to_world, None if g is None else g.ctypes.data)
-        out = [Frame.from_c(r) for r in res]
+        out = self._frames(res)
         return (out, g) if grids else out
 
     # ---- depth images: the depth camera's cloud built on the device (depth_image_proc + od.cpp:688-701) ----------
@@ -472,7 +486,7 @@ class ObstacleProcessor:
             g = np.empty((len(window_first) - 1, h, w), np.int8)
         res = self.process_batch_depth_windows_raw(descs, window_first, transforms, world_to_sensor, sensor_to_world,
                                                    None if g is None else g.ctypes.data)
-        out = [Frame.from_c(r) for r in res]
+        out = self._frames(res)
         return (out, g) if grids else out
 
     def accumulate_depth_image(self, image, transform=None) -> int:
@@ -594,7 +608,7 @@ class ObstacleProcessor:
         self._host_results_only()
         r = FrameResult()
         self._check(self._lib.pcop_process_accumulated(self._h, C.byref(r)))
-        return Frame.from_c(r)
+        return self._frames([r])[0]
 
     def transform(self, cloud, transform, is_dense=False):
         cloud = _f32(cloud)
@@ -730,3 +744,20 @@ class ObstacleProcessor:
                                                    indices.ctypes.data_as(C.c_void_p), c,
                                                    out.ctypes.data_as(C.c_void_p)))
         return out[:c].copy()
+
+    def cluster_footprints(self, cloud, offsets, indices):
+        """pcop_cluster_footprints: every cluster's box and ground-plane convex hull, stage-isolated.  Returns (boxes
+        float32 [C, 8], hull_offsets int32 [C + 1], hull_indices int32 [H])."""
+        cloud = _f32(cloud) if len(cloud) else np.zeros((0, 4), np.float32)
+        offsets = np.ascontiguousarray(offsets, np.int32)
+        indices = np.ascontiguousarray(indices, np.int32)
+        c = len(offsets) - 1
+        boxes = np.zeros((max(c, 1), 8), np.float32)
+        hoff = np.zeros(c + 1, np.int32)
+        hidx = np.zeros(max(len(indices), 1), np.int32)
+        n = C.c_int32()
+        self._check(self._lib.pcop_cluster_footprints(
+            self._h, cloud.ctypes.data_as(C.c_void_p), cloud.shape[0], offsets.ctypes.data_as(C.c_void_p),
+            (indices if len(indices) else hidx).ctypes.data_as(C.c_void_p), c, boxes.ctypes.data_as(C.c_void_p),
+            hoff.ctypes.data_as(C.c_void_p), hidx.ctypes.data_as(C.c_void_p), C.byref(n)))
+        return boxes[:c].copy(), hoff, hidx[:n.value].copy()

@@ -236,11 +236,13 @@ __global__ void k_pack_scan(int* __restrict__ counts, int maxB, int B, uint32_t 
                      counts + (size_t)CNT_CLUS1 * maxB, plane_enabled, f);
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int kPkCountD[PK_N] = {CNT_CROP, CNT_VOX, CNT_VOX, CNT_SOR, CNT_NINL, CNT_REM, CNT_REM, CNT_CLUS1, CNT_CLPTS, CNT_CLUS};
-  const uint32_t kPkMaskD[PK_N] = {PCOP_OUT_CROP,     PCOP_OUT_VOXEL,     PCOP_OUT_VOXEL,     PCOP_OUT_SOR,
-                                   PCOP_OUT_PLANE,    PCOP_OUT_REMAINING, PCOP_OUT_REMAINING, PCOP_OUT_CLUSTERS,
-                                   PCOP_OUT_CLUSTERS, PCOP_OUT_OBSTACLES};
-  const int kPkElemD[PK_N] = {4, 4, 16, 4, 4, 16, 4, 4, 4, 16};
+  const int kPkCountD[PK_N] = {CNT_CROP,  CNT_VOX,   CNT_VOX,  CNT_SOR,  CNT_NINL,  CNT_REM, CNT_REM,
+                               CNT_CLUS1, CNT_CLPTS, CNT_CLUS, CNT_CLUS, CNT_CLUS1, CNT_HULL};
+  const uint32_t kPkMaskD[PK_N] = {PCOP_OUT_CROP,     PCOP_OUT_VOXEL,      PCOP_OUT_VOXEL,      PCOP_OUT_SOR,
+                                   PCOP_OUT_PLANE,    PCOP_OUT_REMAINING,  PCOP_OUT_REMAINING,  PCOP_OUT_CLUSTERS,
+                                   PCOP_OUT_CLUSTERS, PCOP_OUT_OBSTACLES,  PCOP_OUT_FOOTPRINTS, PCOP_OUT_FOOTPRINTS,
+                                   PCOP_OUT_FOOTPRINTS};
+  const int kPkElemD[PK_N] = {4, 4, 16, 4, 4, 16, 4, 4, 4, 16, 32, 4, 4};
   for (int k = warp; k < PK_N; k += blockDim.x / 32) {
     int run = 0;
     if (mask & kPkMaskD[k]) {
@@ -265,8 +267,8 @@ __global__ void k_pack_scan(int* __restrict__ counts, int maxB, int B, uint32_t 
     const unsigned long long start = cursor ? *cursor : 0ull;
     unsigned long long off = start;
     for (int k = 0; k < PK_N; ++k) {
-      meta->base[k] = off;
-      meta->total[k] = total[k];
+      meta->base_of(k) = off;
+      meta->total_of(k) = total[k];
       off += ((unsigned long long)total[k] * kPkElemD[k] + 255ull) & ~255ull;
     }
     meta->total_bytes = off - start;
@@ -318,11 +320,12 @@ __global__ void __launch_bounds__(256)
   const int wpe = ps.words_per_elem[which];
   const int n = counts[(size_t)ps.count_row[which] * maxB + f];
   const uint32_t* s = base + (size_t)f * ps.frame_stride_words[which];
-  uint32_t* dst = reinterpret_cast<uint32_t*>(pack + meta->base[which]) + (size_t)pack_off[(size_t)which * maxB + f] * wpe;
-  if (wpe == 4) {  // 16-byte elements; bases are 256-byte aligned and offsets are whole elements
+  uint32_t* dst = reinterpret_cast<uint32_t*>(pack + meta->base_of(which)) + (size_t)pack_off[(size_t)which * maxB + f] * wpe;
+  if (wpe % 4 == 0) {  // 16- / 32-byte elements; bases are 256-byte aligned and offsets are whole elements
     const uint4* s4 = reinterpret_cast<const uint4*>(s);
     uint4* d4 = reinterpret_cast<uint4*>(dst);
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) d4[i] = s4[i];
+    const int n4 = n * (wpe / 4);
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += gridDim.x * blockDim.x) d4[i] = s4[i];
   } else {
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) dst[i] = s[i];
   }
@@ -569,6 +572,7 @@ int run_wave_cluster(Lane* l, int B, int max_n, const WaveRoute& r) {
   {
     StageTimer t(l, PCOP_STAGE_CENTROID);
     if (p.enable_cluster && generic_centroid) run_centroid_radius(c, ca);
+    if (effective_outputs(p) & PCOP_OUT_FOOTPRINTS) TRY(enqueue_footprints(l, c, l->d_rem, h->cap));
   }
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail_cuda(h, e, "stage launches", __FILE__, __LINE__);
@@ -640,9 +644,11 @@ int enqueue_wave_pack(Lane* l, int B, int max_n, uint32_t mask, const WaveRoute&
                                              (unsigned long long)l->d_pack.size()));
   count_launch(c);
   const void* srcs[PK_N] = {l->d_crop_kept, l->d_vox_keys, l->d_vox,     l->d_sor_kept, l->d_inliers,
-                            l->d_rem,       l->d_rem_src,  l->d_offsets, l->d_indices,  l->d_obst};
+                            l->d_rem,       l->d_rem_src,  l->d_offsets, l->d_indices,  l->d_obst,
+                            l->d_fp_box,    l->d_fp_hoff,  l->d_fp_hidx};
   const size_t strides[PK_N] = {(size_t)h->cap, (size_t)h->cap, (size_t)h->cap,     (size_t)h->cap, (size_t)h->cap,
-                                (size_t)h->cap, (size_t)h->cap, (size_t)h->cap + 1, (size_t)h->cap, (size_t)h->cap};
+                                (size_t)h->cap, (size_t)h->cap, (size_t)h->cap + 1, (size_t)h->cap, (size_t)h->cap,
+                                (size_t)h->cap, (size_t)h->cap + 1, (size_t)h->cap};
   {
     PackSrc ps{};
     bool any = false;
@@ -661,17 +667,19 @@ int enqueue_wave_pack(Lane* l, int B, int max_n, uint32_t mask, const WaveRoute&
       m.words[nseg] = (int)(bytes / 4);
       ++nseg;
     };
-    seg(l->d_counts, l->h_counts, sizeof(int) * CNT_ROWS * h->maxB);
+    seg(l->d_counts, l->h_counts, sizeof(int) * count_rows(mask) * h->maxB);
     seg(l->d_warnings, l->h_warnings, sizeof(uint32_t) * B);
     seg(l->d_prec, l->h_prec, sizeof(PlaneRecord) * B);
-    seg(l->d_meta, l->h_meta, sizeof(PackMeta));
+    seg(l->d_meta, l->h_meta, meta_bytes(mask));
     if (r.vox != WaveRoute::VOX_GENERIC) seg(l->d_vf_flags, l->h_vf_flags, sizeof(uint32_t) * B);
     static_assert(PK_N >= 5, "one pack block per metadata segment");
     if (any) {  // the (frame < 4, array k < 5) blocks of the pack kernel also carry metadata segment k out
       // (parts per (frame, array): 16 for the batched waves; a call of a few large frames gets enough to fill the GPU)
       const int gx = std::max(1, std::min(cdiv(c.grid_cap, 256 * 4), std::max(16, 592 / B)));
       m.frames = std::min(B, 4);
-      KL(c, "k_pack", k_pack<<<dim3(gx, B, PK_N), 256, 0, l->stream>>>(ps, l->d_counts, h->maxB, l->d_pack_off, l->d_meta, l->d_pack, m));
+      // (the footprint arrays are the last pack entries: without them the grid stops before their slices)
+      const int arrays = (mask & PCOP_OUT_FOOTPRINTS) ? PK_N : PK_BOXES;
+      KL(c, "k_pack", k_pack<<<dim3(gx, B, arrays), 256, 0, l->stream>>>(ps, l->d_counts, h->maxB, l->d_pack_off, l->d_meta, l->d_pack, m));
       count_launch(c);
     } else {
       KL(c, "k_meta_out", k_meta_out<<<dim3(4, nseg), 256, 0, l->stream>>>(m));
@@ -907,7 +915,8 @@ int finish_wave(Lane* l, const WaveInput& wi, uint32_t mask, pcop_frame_result* 
     tr.bytes = dev_results ? 0 : (size_t)meta.total_bytes;
   }
   h->d2h_bytes += (dev_results ? 0.0 : (double)meta.total_bytes) +
-                  (double)(sizeof(int) * CNT_ROWS * h->maxB + sizeof(uint32_t) * B + sizeof(PlaneRecord) * B + sizeof(PackMeta));
+                  (double)(sizeof(int) * count_rows(mask) * h->maxB + sizeof(uint32_t) * B + sizeof(PlaneRecord) * B +
+                           meta_bytes(mask));
   ++l->wave_seq;
 
   size_t run[PK_N] = {0};
@@ -931,20 +940,27 @@ int finish_wave(Lane* l, const WaveInput& wi, uint32_t mask, pcop_frame_result* 
     memcpy(r.plane_pass_points, pr.pass_points, sizeof(pr.pass_points));
     memcpy(r.plane_pass_inliers, pr.pass_inliers, sizeof(pr.pass_inliers));
     memcpy(r.plane_pass_coeff, pr.pass_coeff, sizeof(pr.pass_coeff));
+    pcop_frame_footprints& fp = h->fp[(size_t)w0 + f];
+    memset(&fp, 0, sizeof(fp));
+    fp.n_clusters = r.n_clusters;
+    if (mask & PCOP_OUT_FOOTPRINTS) fp.n_hull_vertices = H(CNT_HULL, f);
     const void** slots[PK_N] = {(const void**)&r.crop_kept_idx,    (const void**)&r.voxel_keys,
                                 (const void**)&r.voxel_centroids,  (const void**)&r.sor_kept_idx,
                                 (const void**)&r.plane_inlier_idx, (const void**)&r.remaining_cloud,
                                 (const void**)&r.remaining_src_idx, (const void**)&r.cluster_offsets,
-                                (const void**)&r.cluster_indices,  (const void**)&r.obstacles};
+                                (const void**)&r.cluster_indices,  (const void**)&r.obstacles,
+                                (const void**)&fp.boxes,           (const void**)&fp.hull_offsets,
+                                (const void**)&fp.hull_indices};
     for (int k = 0; k < PK_N; ++k) {
       if (!(mask & kPkMask[k])) continue;
       if (dev_results) {  // device pointer into the pack buffer (it does not move)
-        *slots[k] = l->d_pack + (size_t)meta.base[k] + run[k] * kPkElem[k];
+        *slots[k] = l->d_pack + (size_t)meta.base_of(k) + run[k] * kPkElem[k];
       } else {
         // store the byte offset now; turned into a pointer once the host buffer can no longer move
-        const size_t off = base_off + (size_t)meta.base[k] + run[k] * kPkElem[k];
+        const size_t off = base_off + (size_t)meta.base_of(k) + run[k] * kPkElem[k];
         *slots[k] = (const void*)(uintptr_t)(off + 1);  // +1 so that offset 0 is distinguishable from NULL
-        l->fixups.push_back((size_t)((const unsigned char*)slots[k] - (const unsigned char*)out_all));
+        if (k < PK_BOXES) l->fixups.push_back((size_t)((const unsigned char*)slots[k] - (const unsigned char*)out_all));
+        else l->fp_fixups.push_back((size_t)((const unsigned char*)slots[k] - (const unsigned char*)h->fp.data()));
       }
       run[k] += (size_t)H(kPkCount[k], f);
     }
@@ -969,6 +985,9 @@ int finish_wave(Lane* l, const WaveInput& wi, uint32_t mask, pcop_frame_result* 
       b += 16.0 * r.n_remaining + 4.0 * r.n_cluster_points + 4.0 * (r.n_clusters + 1);
       b += 16.0 * r.n_remaining + 4.0 * r.n_cluster_points + 16.0 * r.n_clusters;
     }
+    if (mask & PCOP_OUT_FOOTPRINTS)  // offsets, indices and member points in; boxes and hull CSR out
+      b += 4.0 * (r.n_clusters + 1) + 20.0 * r.n_cluster_points + 32.0 * r.n_clusters + 4.0 * (r.n_clusters + 1) +
+           4.0 * fp.n_hull_vertices;
     h->alg_bytes += b;
   }
   for (int s = 0; s < PCOP_N_STAGES; ++s) {
@@ -998,6 +1017,7 @@ __global__ void k_zero_u32(uint32_t* p, int n) {
 int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, const int32_t* n, int32_t batch,
                  pcop_frame_result* out, const OccCall* occ, const Pc2Call* pc2) {
   if (!h) return fail(nullptr, PCOP_ERR_BAD_PARAM, "null handle");
+  h->fp_ok = false;  // (until this call succeeds)
   if ((!xyzw && !pc2) || !n || !out || batch < 0) return fail(h, PCOP_ERR_BAD_PARAM, "null argument");
   PCOP_CUDA_TRY(cudaSetDevice(h->device));
   for (int f = 0; f < batch; ++f) {
@@ -1039,6 +1059,7 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
       raw_need = std::max(raw_need, bytes);
       pc2_need = std::max(pc2_need, (size_t)(m1 - m0));
     }
+  h->fp.assign((size_t)batch, pcop_frame_footprints{});
   h->launches = 0;
   h->alg_bytes = 0.0;
   h->d2h_bytes = 0.0;
@@ -1056,9 +1077,11 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
     TRY(grow_raw(l, raw_need));
     TRY(grow(l, l->d_pc2, pc2_need));
     TRY(grow(l, l->h_pc2, pc2_need));
+    if (mask & PCOP_OUT_FOOTPRINTS) TRY(grow_footprints(l));
     l->h_pack_used = 0;
     l->h_pack_sel ^= 1;
     l->fixups.clear();
+    l->fp_fixups.clear();
     l->wave_seq = 0;
     l->call_lane_waves = cdiv((int)waves.size(), (int)lanes.size());
     l->trace_used = 0;
@@ -1131,7 +1154,13 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
       const size_t off = (size_t)(uintptr_t)(*slot) - 1;
       *slot = l->h_pack() + off;
     }
+    for (size_t fx : l->fp_fixups) {
+      const void** slot = (const void**)((unsigned char*)h->fp.data() + fx);
+      const size_t off = (size_t)(uintptr_t)(*slot) - 1;
+      *slot = l->h_pack() + off;
+    }
   }
+  h->fp_ok = true;
   return PCOP_OK;
 }
 
@@ -1156,6 +1185,35 @@ static int ingest_one(pcop_handle* h, const unsigned char* data, size_t bytes, b
     KL(c, "k_pc2_ingest", k_pc2_ingest<<<cdiv(d.n, PC2_TILE), PC2_THREADS, 0, l->stream>>>(l->d_pc2, 1, dst));
   count_launch(c);
   if (src != data) PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));  // the caller may reuse its buffer
+  return PCOP_OK;
+}
+
+int grow_footprints(Lane* l) {
+  const size_t B = (size_t)l->h->maxB, BC = B * (size_t)l->h->cap;
+  TRY(grow(l, l->d_fp_box, BC * 8));
+  TRY(grow(l, l->d_fp_count, BC + B));
+  TRY(grow(l, l->d_fp_stage, BC));
+  TRY(grow(l, l->d_fp_hoff, BC + B));
+  TRY(grow(l, l->d_fp_hidx, BC));
+  return PCOP_OK;
+}
+
+int enqueue_footprints(Lane* l, const Ctx& c, const float4* in, size_t in_stride) {
+  FootprintArgs a{};
+  a.in = in;
+  a.in_stride = in_stride;
+  a.offsets = l->d_offsets;
+  a.indices = l->d_indices;
+  a.n_clusters = l->cnt(CNT_CLUS);
+  a.boxes = l->d_fp_box;
+  a.hull_count = l->d_fp_count;
+  a.stage = l->d_fp_stage;
+  a.work = l->d_sorted;  // (the search-grid point list of clustering is dead once the clusters are final)
+  a.hull_offsets = l->d_fp_hoff;
+  a.hull_indices = l->d_fp_hidx;
+  a.n_hull = l->cnt(CNT_HULL);
+  const cudaError_t e = run_footprints(c, a);
+  if (e != cudaSuccess) return fail_cuda(l->h, e, "run_footprints (shared-memory opt-in or launch)", __FILE__, __LINE__);
   return PCOP_OK;
 }
 

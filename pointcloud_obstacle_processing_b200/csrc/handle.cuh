@@ -3,6 +3,7 @@
 #pragma once
 #include <algorithm>
 #include <cmath>
+#include <cstddef>
 #include <memory>
 #include <string>
 #include <utility>
@@ -27,6 +28,8 @@ enum {  // rows of the per-frame count table (device: d_counts[row*maxB + f])
   CNT_CELLS,  // occupied clique cells (ECE scratch)
   CNT_ROUTE,  // point count as seen by the generic clustering path (ECE scratch)
   CNT_GROUPS, // groups of the partition voxel path (scratch; the host sizes the next wave's reduce grid by it)
+  CNT_HULL,   // H: hull vertices of the frame's clusters (PCOP_OUT_FOOTPRINTS; the last row: without the bit the wave's
+              // metadata copy stops before it)
   CNT_ROWS
 };
 
@@ -41,13 +44,19 @@ enum {  // packed output arrays
   PK_OFFSETS,
   PK_INDICES,
   PK_OBSTACLES,
+  PK_BOXES,
+  PK_HULL_OFFSETS,
+  PK_HULL_INDICES,
   PK_N
 };
-const int kPkElem[PK_N] = {4, 4, 16, 4, 4, 16, 4, 4, 4, 16};
-const int kPkCount[PK_N] = {CNT_CROP, CNT_VOX, CNT_VOX, CNT_SOR, CNT_NINL, CNT_REM, CNT_REM, CNT_CLUS1, CNT_CLPTS, CNT_CLUS};
-const uint32_t kPkMask[PK_N] = {PCOP_OUT_CROP,      PCOP_OUT_VOXEL,     PCOP_OUT_VOXEL,    PCOP_OUT_SOR,
-                                PCOP_OUT_PLANE,     PCOP_OUT_REMAINING, PCOP_OUT_REMAINING, PCOP_OUT_CLUSTERS,
-                                PCOP_OUT_CLUSTERS,  PCOP_OUT_OBSTACLES};
+const int kPkElem[PK_N] = {4, 4, 16, 4, 4, 16, 4, 4, 4, 16, 32, 4, 4};
+const int kPkCount[PK_N] = {CNT_CROP, CNT_VOX,   CNT_VOX,  CNT_SOR,  CNT_NINL,  CNT_REM, CNT_REM,
+                            CNT_CLUS1, CNT_CLPTS, CNT_CLUS, CNT_CLUS, CNT_CLUS1, CNT_HULL};
+const uint32_t kPkMask[PK_N] = {PCOP_OUT_CROP,      PCOP_OUT_VOXEL,      PCOP_OUT_VOXEL,     PCOP_OUT_SOR,
+                                PCOP_OUT_PLANE,     PCOP_OUT_REMAINING,  PCOP_OUT_REMAINING, PCOP_OUT_CLUSTERS,
+                                PCOP_OUT_CLUSTERS,  PCOP_OUT_OBSTACLES,  PCOP_OUT_FOOTPRINTS, PCOP_OUT_FOOTPRINTS,
+                                PCOP_OUT_FOOTPRINTS};
+constexpr uint32_t kPkOutputs = (uint32_t)PCOP_OUT_ALL | (uint32_t)PCOP_OUT_FOOTPRINTS;  // the bits that pack arrays
 
 struct PlaneRecord {
   int n_passes;
@@ -58,12 +67,24 @@ struct PlaneRecord {
   float4 pass_coeff[PCOP_MAX_PLANE_PASSES_RECORDED];
 };
 
-struct PackMeta {  // device -> host in one copy
-  unsigned long long base[PK_N];  // byte offset of each array inside the pack buffer
+// device -> host in one copy.  The footprint arrays' entries come last, so that a wave without PCOP_OUT_FOOTPRINTS
+// copies only the part before them (meta_bytes), exactly the record of the arrays of PCOP_OUT_ALL.
+struct PackMeta {
+  unsigned long long base[PK_BOXES];  // byte offset of each array inside the pack buffer
   unsigned long long total_bytes;
-  int total[PK_N];  // elements
-  int overflow;     // the wave's arrays do not fit the pack buffer (nothing was packed)
+  int total[PK_BOXES];  // elements
+  int overflow;         // the wave's arrays do not fit the pack buffer (nothing was packed)
+  unsigned long long fp_base[PK_N - PK_BOXES];  // the same for the footprint arrays
+  int fp_total[PK_N - PK_BOXES];
+
+  __host__ __device__ unsigned long long& base_of(int k) { return k < PK_BOXES ? base[k] : fp_base[k - PK_BOXES]; }
+  __host__ __device__ unsigned long long base_of(int k) const { return k < PK_BOXES ? base[k] : fp_base[k - PK_BOXES]; }
+  __host__ __device__ int& total_of(int k) { return k < PK_BOXES ? total[k] : fp_total[k - PK_BOXES]; }
 };
+static_assert(offsetof(PackMeta, fp_base) == 136, "the record of the PCOP_OUT_ALL arrays keeps its 136 bytes");
+inline size_t meta_bytes(uint32_t mask) {
+  return (mask & PCOP_OUT_FOOTPRINTS) ? sizeof(PackMeta) : offsetof(PackMeta, fp_base);
+}
 
 // decode descriptor of one message (device memory): a PointCloud2 message, read by k_pc2_ingest, or a depth image,
 // read by k_depth_ingest (n = width * height pixels; point_step and the field offsets unused)
@@ -221,6 +242,9 @@ struct pcop_handle {
   double d2h_bytes = 0.0;
   unsigned long long sort_pass_keys = 0;
   pcop::KernelTimers kt;
+  // footprints of every frame of the last pcop_process* call (PCOP_OUT_FOOTPRINTS); fp_ok = 0 after a failed call
+  std::vector<pcop_frame_footprints> fp;
+  bool fp_ok = false;
 };
 
 namespace pcop {
@@ -275,6 +299,10 @@ struct Lane {
   // single-frame occupancy calls (lane 0): pcop_occupancy_grid's int64 counts, int64 row averages and int8 cells;
   // pcop_occupancy_shadows' grid cells, CSR copy, records and warning word
   Buffer<unsigned char> d_occ, d_shadow;
+  // PCOP_OUT_FOOTPRINTS (allocated by the first call with the bit, or the first pcop_cluster_footprints): boxes
+  // [maxB][cap][8], hull sizes and CSR offsets [maxB][cap + 1], staged and final hull indices [maxB][cap]
+  Buffer<float> d_fp_box;
+  Buffer<int> d_fp_count, d_fp_stage, d_fp_hoff, d_fp_hidx;
 
   // pinned host
   HostBuffer<int> h_counts;  // [CNT_ROWS][maxB]
@@ -297,6 +325,7 @@ struct Lane {
   int pend_max_n = 1;
   WaveRoute route;                  // of the wave in flight
   std::vector<size_t> fixups;  // result-pointer slots of the running call (byte offsets into the caller's array)
+  std::vector<size_t> fp_fixups;  // the same for the footprint pointers (byte offsets into pcop_handle::fp)
   struct TraceRec {
     int w0, B;
     size_t bytes;
@@ -348,18 +377,21 @@ int grow(Lane* l, Buffer<T, Pinned>& b, size_t n) {
 }
 
 inline uint32_t effective_outputs(const pcop_params& p) {
-  uint32_t m = p.outputs & (uint32_t)(PCOP_OUT_ALL | PCOP_OUT_DEVICE);
+  uint32_t m = p.outputs & (uint32_t)(PCOP_OUT_ALL | PCOP_OUT_FOOTPRINTS | PCOP_OUT_DEVICE);
   if (p.publish_point_clouds) m |= PCOP_OUT_ALL;  // od.cpp:945: intermediates wanted
   if (!p.enable_crop) m &= ~(uint32_t)PCOP_OUT_CROP;
   if (!p.enable_voxel) m &= ~(uint32_t)PCOP_OUT_VOXEL;
   if (!p.enable_sor) m &= ~(uint32_t)PCOP_OUT_SOR;
   if (!p.enable_plane) m &= ~(uint32_t)PCOP_OUT_PLANE;
-  if (!p.enable_cluster) m &= ~(uint32_t)(PCOP_OUT_CLUSTERS | PCOP_OUT_OBSTACLES);
+  if (!p.enable_cluster) m &= ~(uint32_t)(PCOP_OUT_CLUSTERS | PCOP_OUT_OBSTACLES | PCOP_OUT_FOOTPRINTS);
   return m;
 }
 
+// rows of the count table a wave copies to the host: CNT_HULL, the last row, only when footprints are requested
+inline int count_rows(uint32_t mask) { return (mask & PCOP_OUT_FOOTPRINTS) ? CNT_ROWS : CNT_HULL; }
+
 inline size_t pack_capacity_bytes(uint32_t mask, int B, int cap) {
-  mask &= (uint32_t)PCOP_OUT_ALL;
+  mask &= kPkOutputs;
   size_t bytes = 0;
   for (int k = 0; k < PK_N; ++k)
     if (mask & kPkMask[k]) bytes += ((size_t)B * (cap + 1)) * kPkElem[k] + 256;
@@ -604,6 +636,10 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
 int pc2_ingest(pcop_handle* h, const unsigned char* data, int32_t n, int32_t point_step, int32_t ox, int32_t oy,
                int32_t oz, const float* t16, int is_dense, float4* dst);
 int depth_ingest(pcop_handle* h, const pcop_depth_image& im, const float* t16, float4* dst);  // (validated image)
+// the footprint buffers of lane l hold a wave (grow(), on the first call that asks for footprints)
+int grow_footprints(Lane* l);
+// the footprints of lane l's wave in flight from its remaining cloud `in` (frame stride in_stride) and clusters
+int enqueue_footprints(Lane* l, const Ctx& c, const float4* in, size_t in_stride);
 __global__ void k_zero_u32(uint32_t* p, int n);  // batch.cu; upload_single zeroes one frame's warning word with it
 
 }  // namespace pcop

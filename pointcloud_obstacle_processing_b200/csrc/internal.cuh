@@ -275,6 +275,24 @@ bool run_cluster(const Ctx& c, const ClusterArgs& a, bool with_generic);
 void run_cluster_small(const Ctx& c, const ClusterArgs& a, int small_max, bool zero_skipped);
 void run_centroid_radius(const Ctx& c, const ClusterArgs& a);
 
+// ---- obstacle footprints (stage_footprint.cu; PCOP_OUT_FOOTPRINTS) ---------------------------------------------
+struct FootprintArgs {  // frame f of c.B at f * in_stride (cloud), f * (cap + 1) (offsets) and f * cap (the rest)
+  const float4* in;  // remaining cloud
+  size_t in_stride;
+  const int* offsets;     // cluster CSR
+  const int* indices;
+  const int* n_clusters;  // [B]
+  float* boxes;           // [B][cap][8] out
+  int* hull_count;        // [B][cap + 1] scratch: hull size of every cluster
+  int* stage;             // [B][cap] scratch: hull vertices at the cluster's (piece's) first member slot
+  float4* work;           // [B][cap] scratch of the hulls whose candidates exceed one shared-memory tile
+  int* hull_offsets;      // [B][cap + 1] out: CSR
+  int* hull_indices;      // [B][cap] out (scratch of the piece sizes until the CSR kernel)
+  int* n_hull;            // [B] out: H
+};
+// the box and hull of every cluster of every frame; returns the first error of the shared-memory opt-in or a launch
+cudaError_t run_footprints(const Ctx& c, const FootprintArgs& a);
+
 // ---- occupancy grid (stage_occupancy.cu; od.cpp:134-157, 175-269, 467-672, 817-833) ------------------------------
 struct OccGrid {
   float lim[6];  // crop box x_min,x_max,y_min,y_max,z_min,z_max (od.cpp:197-199)

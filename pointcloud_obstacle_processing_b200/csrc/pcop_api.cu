@@ -463,6 +463,7 @@ int pcop_process_batch_occupancy(pcop_handle* h, const float* xyzw, size_t frame
                                  int32_t batch, const float* world_to_sensor16, const float* sensor_to_world16,
                                  int8_t* grids, pcop_frame_result* out) {
   if (!h) return fail(nullptr, PCOP_ERR_BAD_PARAM, "null handle");
+  h->fp_ok = false;  // (a call that fails leaves no footprints)
   if (!world_to_sensor16 || !sensor_to_world16 || !grids || !out || batch < 0 || (!xyzw && batch != 1))
     return fail(h, PCOP_ERR_BAD_PARAM, "pcop_process_batch_occupancy: null argument (xyzw = NULL takes batch = 1)");
   OccCall oc{};
@@ -496,6 +497,7 @@ static int windows_call(pcop_handle* h, const char* who, Pc2Call& pc, int32_t n_
                         const float* world_to_sensor16, const float* sensor_to_world16, int8_t* grids,
                         pcop_frame_result* out) {
   const std::string w(who);
+  h->fp_ok = false;  // (a call that fails leaves no footprints)
   const int32_t* window_first = pc.window_first;
   if (!out || batch < 0 || n_msgs < 0 || (!pc.msgs && !pc.images && n_msgs > 0) || (!window_first && (batch > 0 || n_msgs > 0)) ||
       (grids && (!world_to_sensor16 || !sensor_to_world16)))
@@ -663,6 +665,7 @@ int pcop_accumulate_reset(pcop_handle* h) {
 }
 
 int pcop_process_accumulated(pcop_handle* h, pcop_frame_result* out) {
+  if (h) h->fp_ok = false;  // (a call that fails leaves no footprints)
   if (!h || !out) return fail(h, PCOP_ERR_BAD_PARAM, "null argument");
   const int32_t n = h->acc_count;
   // od.cpp:701: current_frame_count = 0; the accumulator is consumed by this run
@@ -1007,6 +1010,44 @@ int pcop_centroid_radius(pcop_handle* h, const float* xyzw, int32_t p, const int
   Ctx c = make_ctx(l, 1, p);
   run_centroid_radius(c, make_cluster_args(l, l->d_in, h->cap, l->cnt(CNT_REM)));
   TRY(download(h, obstacles, l->d_obst, (size_t)c_in * 16));
+  PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
+  return PCOP_OK;
+}
+
+int pcop_last_footprints(const pcop_handle* h, int32_t frame, pcop_frame_footprints* out) {
+  if (!h || !out || !h->fp_ok || frame < 0 || (size_t)frame >= h->fp.size()) return PCOP_ERR_BAD_PARAM;
+  *out = h->fp[(size_t)frame];
+  return PCOP_OK;
+}
+
+int pcop_cluster_footprints(pcop_handle* h, const float* xyzw, int32_t p, const int32_t* cluster_offsets,
+                            const int32_t* cluster_indices, int32_t c_in, float* boxes, int32_t* hull_offsets,
+                            int32_t* hull_indices, int32_t* n_hull) {
+  if (!h || !xyzw || !cluster_offsets || !cluster_indices || !boxes || !hull_offsets || !hull_indices || !n_hull ||
+      c_in < 0 || p < 0)
+    return fail(h, PCOP_ERR_BAD_PARAM, "null argument");
+  if (c_in > h->cap || p > h->cap) return fail(h, PCOP_ERR_CAPACITY, "more points or clusters than max_points");
+  if (cluster_offsets[0] != 0) return fail(h, PCOP_ERR_BAD_PARAM, "cluster_offsets[0] must be 0");
+  for (int32_t k = 0; k < c_in; ++k)
+    if (cluster_offsets[k + 1] < cluster_offsets[k]) return fail(h, PCOP_ERR_BAD_PARAM, "cluster_offsets decrease");
+  const int32_t len = cluster_offsets[c_in];
+  if (len > p) return fail(h, PCOP_ERR_BAD_PARAM, "cluster_offsets[c] exceeds the point count");
+  for (int32_t j = 0; j < len; ++j)
+    if (cluster_indices[j] < 0 || cluster_indices[j] >= p)
+      return fail(h, PCOP_ERR_BAD_PARAM, "cluster index " + std::to_string(j) + " outside [0, p)");
+  TRY(upload_single(h, xyzw, p, CNT_REM));
+  Lane* l = h->lanes[0].get();
+  TRY(grow_footprints(l));
+  l->h_n_in[1] = c_in;
+  PCOP_CUDA_TRY(cudaMemcpyAsync(l->cnt(CNT_CLUS), l->h_n_in + 1, sizeof(int), cudaMemcpyHostToDevice, l->stream));
+  PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_offsets, cluster_offsets, (size_t)(c_in + 1) * 4, cudaMemcpyHostToDevice, l->stream));
+  if (len > 0) PCOP_CUDA_TRY(cudaMemcpyAsync(l->d_indices, cluster_indices, (size_t)len * 4, cudaMemcpyHostToDevice, l->stream));
+  Ctx c = make_ctx(l, 1, p);
+  TRY(enqueue_footprints(l, c, l->d_in, h->cap));
+  TRY(fetch_word(h, l->cnt(CNT_HULL), n_hull));
+  TRY(download(h, boxes, l->d_fp_box, (size_t)c_in * 32));
+  TRY(download(h, hull_offsets, l->d_fp_hoff, (size_t)(c_in + 1) * 4));
+  TRY(download(h, hull_indices, l->d_fp_hidx, (size_t)*n_hull * 4));
   PCOP_CUDA_TRY(cudaStreamSynchronize(l->stream));
   return PCOP_OK;
 }

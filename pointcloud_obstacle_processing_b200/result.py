@@ -4,7 +4,7 @@ from typing import List, Optional
 
 import numpy as np
 
-from ._ctypes_abi import FrameResult, MAX_PASSES
+from ._ctypes_abi import FrameFootprints, FrameResult, MAX_PASSES
 
 
 def _arr(ptr, n, dtype, cols=None):
@@ -24,7 +24,9 @@ class Frame:
 
     `clusters` is the std::vector<pcl::PointIndices> of od.cpp:793 (indices into
     `remaining_cloud` = planar_cloud_y, od.cpp:765); `obstacles` is the
-    PointIndicesArray.points payload (msg/PointWithRad.msg:1-4).
+    PointIndicesArray.points payload (msg/PointWithRad.msg:1-4).  With outputs | OUT_FOOTPRINTS, `boxes` (C, 8) holds
+    every cluster's {min x, min y, min z, 0, max x, max y, max z, 0} and `hull_offsets` / `hull_indices` the CSR of its
+    ground-plane convex hull (counter-clockwise, indices into `remaining_cloud`); None otherwise.
     """
     status: int = 0
     warnings: int = 0
@@ -51,6 +53,24 @@ class Frame:
     cluster_offsets: Optional[np.ndarray] = None
     cluster_indices: Optional[np.ndarray] = None
     obstacles: Optional[np.ndarray] = None
+    boxes: Optional[np.ndarray] = None
+    hull_offsets: Optional[np.ndarray] = None
+    hull_indices: Optional[np.ndarray] = None
+
+    @property
+    def hulls(self):
+        """one index array per cluster: its hull vertices, counter-clockwise (None without OUT_FOOTPRINTS)"""
+        if self.hull_offsets is None or self.hull_indices is None:
+            return None
+        o = self.hull_offsets
+        return [self.hull_indices[o[k]:o[k + 1]] for k in range(len(o) - 1)]
+
+    def set_footprints(self, fp: FrameFootprints):
+        """copies the footprint arrays of a (host) pcop_frame_footprints; NULL pointers leave them None"""
+        self.boxes = _arr(fp.boxes, fp.n_clusters, np.float32, 8)
+        self.hull_offsets = _arr(fp.hull_offsets, fp.n_clusters + 1, np.int32)
+        self.hull_indices = _arr(fp.hull_indices, fp.n_hull_vertices, np.int32)
+        return self
 
     @property
     def clusters(self):
