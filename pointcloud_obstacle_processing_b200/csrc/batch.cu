@@ -223,11 +223,18 @@ __global__ void __launch_bounds__(CT_THREADS)
   }
 }
 
+struct PackSrc {  // the packed arrays of one wave, from kPack (enqueue_wave_pack)
+  const uint32_t* src[PK_N];  // nullptr: not requested
+  unsigned long long frame_stride_words[PK_N];
+  int count_row[PK_N];
+  int words_per_elem[PK_N];
+};
+
 // exclusive scans over the frames of every requested output's count row + array base offsets
 // (first the per-frame plane record + the derived count rows CNT_NINL / CNT_CLUS1, which the scans below read)
 // (PCOP_OUT_DEVICE: the arrays of all waves of a call stay in the pack buffer, so the wave's base is a device-side
 // cursor that this kernel advances; a wave that does not fit sets meta->overflow and is not packed)
-__global__ void k_pack_scan(int* __restrict__ counts, int maxB, int B, uint32_t mask, int* __restrict__ pack_off,
+__global__ void k_pack_scan(int* __restrict__ counts, int maxB, int B, PackSrc ps, int* __restrict__ pack_off,
                             PackMeta* __restrict__ meta, const PlaneFrame* __restrict__ pf, PlaneRecord* __restrict__ rec,
                             int plane_enabled, unsigned long long* __restrict__ cursor, unsigned long long capacity) {
   __shared__ int total[PK_N];
@@ -236,17 +243,10 @@ __global__ void k_pack_scan(int* __restrict__ counts, int maxB, int B, uint32_t 
                      counts + (size_t)CNT_CLUS1 * maxB, plane_enabled, f);
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int kPkCountD[PK_N] = {CNT_CROP,  CNT_VOX,   CNT_VOX,  CNT_SOR,  CNT_NINL,  CNT_REM, CNT_REM,
-                               CNT_CLUS1, CNT_CLPTS, CNT_CLUS, CNT_CLUS, CNT_CLUS1, CNT_HULL};
-  const uint32_t kPkMaskD[PK_N] = {PCOP_OUT_CROP,     PCOP_OUT_VOXEL,      PCOP_OUT_VOXEL,      PCOP_OUT_SOR,
-                                   PCOP_OUT_PLANE,    PCOP_OUT_REMAINING,  PCOP_OUT_REMAINING,  PCOP_OUT_CLUSTERS,
-                                   PCOP_OUT_CLUSTERS, PCOP_OUT_OBSTACLES,  PCOP_OUT_FOOTPRINTS, PCOP_OUT_FOOTPRINTS,
-                                   PCOP_OUT_FOOTPRINTS};
-  const int kPkElemD[PK_N] = {4, 4, 16, 4, 4, 16, 4, 4, 4, 16, 32, 4, 4};
   for (int k = warp; k < PK_N; k += blockDim.x / 32) {
     int run = 0;
-    if (mask & kPkMaskD[k]) {
-      const int* row = counts + (size_t)kPkCountD[k] * maxB;
+    if (ps.src[k]) {
+      const int* row = counts + (size_t)ps.count_row[k] * maxB;
       for (int base = 0; base < B; base += 32) {
         const int f = base + lane;
         const int v = (f < B) ? row[f] : 0;
@@ -269,7 +269,7 @@ __global__ void k_pack_scan(int* __restrict__ counts, int maxB, int B, uint32_t 
     for (int k = 0; k < PK_N; ++k) {
       meta->base_of(k) = off;
       meta->total_of(k) = total[k];
-      off += ((unsigned long long)total[k] * kPkElemD[k] + 255ull) & ~255ull;
+      off += ((unsigned long long)total[k] * (4 * ps.words_per_elem[k]) + 255ull) & ~255ull;
     }
     meta->total_bytes = off - start;
     meta->overflow = (off > capacity) ? 1 : 0;
@@ -300,12 +300,6 @@ __device__ __forceinline__ void meta_out(const MetaOut& m, int k, int first, int
 __global__ void __launch_bounds__(256) k_meta_out(MetaOut m) {
   meta_out(m, blockIdx.y, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
 }
-struct PackSrc {
-  const uint32_t* src[PK_N];  // nullptr: not requested
-  unsigned long long frame_stride_words[PK_N];
-  int count_row[PK_N];
-  int words_per_elem[PK_N];
-};
 
 // all requested output arrays of all frames of the wave in one launch: blockIdx.z = array, blockIdx.y = frame;
 // everything is moved as 32-bit words (the 16-byte arrays as uint4)
@@ -381,6 +375,18 @@ int ensure_host_pack(Lane* l, size_t need) {
   if (b.size()) memcpy(q, b, b.size());
   b = std::move(q);
   return PCOP_OK;
+}
+
+// A device-to-host copy on stream s, in 1 MB pieces: one large copy holds up the kernels of the other lanes for as
+// long as it runs (measured: 6.4 ms per 1024-frame call with one 17 MB copy per wave, 5.7 ms with 0.5-1 MB pieces,
+// 5.9 / 6.2 ms with 2 / 4 MB pieces, 6.3 ms with 256 KB pieces -- the host thread becomes the limit -- and 5.3 ms with
+// no copy at all)
+cudaError_t copy_d2h_in_pieces(void* dst, const void* src, size_t bytes, cudaStream_t s) {
+  const size_t piece = (size_t)1 << 20;
+  cudaError_t e = cudaSuccess;
+  for (size_t o = 0; o < bytes && e == cudaSuccess; o += piece)
+    e = cudaMemcpyAsync((char*)dst + o, (const char*)src + o, std::min(piece, bytes - o), cudaMemcpyDeviceToHost, s);
+  return e;
 }
 
 // The first route of a wave whose largest frame has max_n points, from the handle's plan and knobs and the lane's
@@ -639,52 +645,49 @@ int enqueue_wave_pack(Lane* l, int B, int max_n, uint32_t mask, const WaveRoute&
   StageTimer t(l, PCOP_STAGE_D2H);
   const bool dev_results = (mask & PCOP_OUT_DEVICE) != 0;  // the arrays stay in d_pack (bump-allocated over the call)
   if (!dev_results && l->wave_seq >= 1) PCOP_CUDA_TRY(cudaStreamWaitEvent(l->stream, l->ev_copied, 0));  // d_pack is free again
-  KL(c, "k_pack_scan", k_pack_scan<<<1, 320, 0, l->stream>>>(l->d_counts, h->maxB, B, mask, l->d_pack_off, l->d_meta, l->d_pf, l->d_prec,
+  const void* srcs[] = {l->d_crop_kept, l->d_vox_keys, l->d_vox,     l->d_sor_kept, l->d_inliers,
+                        l->d_rem,       l->d_rem_src,  l->d_offsets, l->d_indices,  l->d_obst,
+                        l->d_fp_box,    l->d_fp_hoff,  l->d_fp_hidx};  // the lane buffer of each packed array, by PK_*
+  static_assert(sizeof(srcs) / sizeof(srcs[0]) == PK_N, "one source per packed array");
+  PackSrc ps{};
+  bool any = false;
+  for (int k = 0; k < PK_N; ++k) {
+    const PackArray& a = kPack[k];
+    ps.src[k] = (mask & a.bit) ? (const uint32_t*)srcs[k] : nullptr;
+    ps.words_per_elem[k] = a.elem_bytes / 4;
+    ps.frame_stride_words[k] = (unsigned long long)(h->cap + (a.csr ? 1 : 0)) * ps.words_per_elem[k];
+    ps.count_row[k] = a.count_row;
+    any = any || ps.src[k];
+  }
+  KL(c, "k_pack_scan", k_pack_scan<<<1, 320, 0, l->stream>>>(l->d_counts, h->maxB, B, ps, l->d_pack_off, l->d_meta, l->d_pf, l->d_prec,
                                              h->params.enable_plane ? 1 : 0, dev_results ? l->d_pack_cursor.get() : nullptr,
                                              (unsigned long long)l->d_pack.size()));
   count_launch(c);
-  const void* srcs[PK_N] = {l->d_crop_kept, l->d_vox_keys, l->d_vox,     l->d_sor_kept, l->d_inliers,
-                            l->d_rem,       l->d_rem_src,  l->d_offsets, l->d_indices,  l->d_obst,
-                            l->d_fp_box,    l->d_fp_hoff,  l->d_fp_hidx};
-  const size_t strides[PK_N] = {(size_t)h->cap, (size_t)h->cap, (size_t)h->cap,     (size_t)h->cap, (size_t)h->cap,
-                                (size_t)h->cap, (size_t)h->cap, (size_t)h->cap + 1, (size_t)h->cap, (size_t)h->cap,
-                                (size_t)h->cap, (size_t)h->cap + 1, (size_t)h->cap};
-  {
-    PackSrc ps{};
-    bool any = false;
-    for (int k = 0; k < PK_N; ++k) {
-      ps.src[k] = (mask & kPkMask[k]) ? (const uint32_t*)srcs[k] : nullptr;
-      ps.frame_stride_words[k] = (unsigned long long)strides[k] * (kPkElem[k] / 4);
-      ps.count_row[k] = kPkCount[k];
-      ps.words_per_elem[k] = kPkElem[k] / 4;
-      any = any || ps.src[k];
-    }
-    MetaOut m{};
-    int nseg = 0;
-    auto seg = [&](const void* src, void* dst, size_t bytes) {
-      m.src[nseg] = (const uint32_t*)src;
-      m.dst[nseg] = (uint32_t*)dst;
-      m.words[nseg] = (int)(bytes / 4);
-      ++nseg;
-    };
-    seg(l->d_counts, l->h_counts, sizeof(int) * count_rows(mask) * h->maxB);
-    seg(l->d_warnings, l->h_warnings, sizeof(uint32_t) * B);
-    seg(l->d_prec, l->h_prec, sizeof(PlaneRecord) * B);
-    seg(l->d_meta, l->h_meta, meta_bytes(mask));
-    if (r.vox != WaveRoute::VOX_GENERIC) seg(l->d_vf_flags, l->h_vf_flags, sizeof(uint32_t) * B);
-    static_assert(PK_N >= 5, "one pack block per metadata segment");
-    if (any) {  // the (frame < 4, array k < 5) blocks of the pack kernel also carry metadata segment k out
-      // (parts per (frame, array): 16 for the batched waves; a call of a few large frames gets enough to fill the GPU)
-      const int gx = std::max(1, std::min(cdiv(c.grid_cap, 256 * 4), std::max(16, 592 / B)));
-      m.frames = std::min(B, 4);
-      // (the footprint arrays are the last pack entries: without them the grid stops before their slices)
-      const int arrays = (mask & PCOP_OUT_FOOTPRINTS) ? PK_N : PK_BOXES;
-      KL(c, "k_pack", k_pack<<<dim3(gx, B, arrays), 256, 0, l->stream>>>(ps, l->d_counts, h->maxB, l->d_pack_off, l->d_meta, l->d_pack, m));
-      count_launch(c);
-    } else {
-      KL(c, "k_meta_out", k_meta_out<<<dim3(4, nseg), 256, 0, l->stream>>>(m));
-      count_launch(c);
-    }
+  MetaOut m{};
+  int nseg = 0;
+  auto seg = [&](const void* src, void* dst, size_t bytes) {
+    m.src[nseg] = (const uint32_t*)src;
+    m.dst[nseg] = (uint32_t*)dst;
+    m.words[nseg] = (int)(bytes / 4);
+    ++nseg;
+  };
+  seg(l->d_counts, l->h_counts, sizeof(int) * count_rows(mask) * h->maxB);
+  seg(l->d_warnings, l->h_warnings, sizeof(uint32_t) * B);
+  seg(l->d_prec, l->h_prec, sizeof(PlaneRecord) * B);
+  seg(l->d_meta, l->h_meta, meta_bytes(mask));
+  if (r.vox != WaveRoute::VOX_GENERIC) seg(l->d_vf_flags, l->h_vf_flags, sizeof(uint32_t) * B);
+  static_assert(PK_N >= 5, "one pack block per metadata segment");
+  if (any) {  // the (frame < 4, array k < 5) blocks of the pack kernel also carry metadata segment k out
+    // (parts per (frame, array): 16 for the batched waves; a call of a few large frames gets enough to fill the GPU)
+    const int gx = std::max(1, std::min(cdiv(c.grid_cap, 256 * 4), std::max(16, 592 / B)));
+    m.frames = std::min(B, 4);
+    // (the footprint arrays are the last pack entries: without them the grid stops before their slices)
+    const int arrays = (mask & PCOP_OUT_FOOTPRINTS) ? PK_N : PK_BOXES;
+    KL(c, "k_pack", k_pack<<<dim3(gx, B, arrays), 256, 0, l->stream>>>(ps, l->d_counts, h->maxB, l->d_pack_off, l->d_meta, l->d_pack, m));
+    count_launch(c);
+  } else {
+    KL(c, "k_meta_out", k_meta_out<<<dim3(4, nseg), 256, 0, l->stream>>>(m));
+    count_launch(c);
   }
   if (h->trace) {
     if (l->trace_used == l->trace_recs.size()) {
@@ -882,27 +885,18 @@ int finish_wave(Lane* l, const WaveInput& wi, uint32_t mask, pcop_frame_result* 
     // costs ~0.4 ms per MB, and every regrowth copies what is already there)
     if (base_off + meta.total_bytes + 256 > l->h_pack().size())
       TRY(ensure_host_pack(l, base_off + (size_t)((double)(meta.total_bytes + 256) * 1.1 * std::max(1, l->call_lane_waves - l->wave_seq))));
-    // payload copy on the copy stream (the pack kernels have finished: ev_meta follows them), in pieces: one large
-    // device-to-host copy holds up the kernels of the other lanes for as long as it runs (measured: 6.4 ms per
-    // 1024-frame call with one 17 MB copy per wave, 5.7 ms with 0.5-1 MB pieces, 5.9 / 6.2 ms with 2 / 4 MB pieces,
-    // 6.3 ms with 256 KB pieces -- the host thread becomes the limit -- and 5.3 ms with no copy at all)
-    const size_t piece = (size_t)1 << 20;
-    for (size_t o = 0; o < meta.total_bytes; o += piece)
-      PCOP_CUDA_TRY(cudaMemcpyAsync(l->h_pack() + base_off + o, l->d_pack + o, std::min<size_t>(piece, meta.total_bytes - o),
-                                    cudaMemcpyDeviceToHost, l->cstream));
+    // payload copy on the copy stream (the pack kernels have finished: ev_meta follows them)
+    PCOP_CUDA_TRY(copy_d2h_in_pieces(l->h_pack() + base_off, l->d_pack, meta.total_bytes, l->cstream));
     PCOP_CUDA_TRY(cudaEventRecord(l->ev_copied, l->cstream));
     l->h_pack_used = base_off + meta.total_bytes;
   }
   if (wi.occ) {  // the wave's grids, after its last repeat, on the copy stream beside the payload
     const size_t bytes = (size_t)B * (size_t)wi.occ->g.cells;
     int8_t* dst = wi.occ->grids + (size_t)w0 * (size_t)wi.occ->g.cells;
-    const unsigned char* src = reinterpret_cast<const unsigned char*>(l->d_occ_grids.get());
     if (wi.occ->grids_on_device) {
-      PCOP_CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, l->cstream));
+      PCOP_CUDA_TRY(cudaMemcpyAsync(dst, l->d_occ_grids, bytes, cudaMemcpyDeviceToDevice, l->cstream));
     } else {
-      const size_t piece = (size_t)1 << 20;  // (pieces: as the payload above)
-      for (size_t o = 0; o < bytes; o += piece)
-        PCOP_CUDA_TRY(cudaMemcpyAsync(dst + o, src + o, std::min<size_t>(piece, bytes - o), cudaMemcpyDeviceToHost, l->cstream));
+      PCOP_CUDA_TRY(copy_d2h_in_pieces(dst, l->d_occ_grids, bytes, l->cstream));
       h->d2h_bytes += (double)bytes;
     }
     PCOP_CUDA_TRY(cudaEventRecord(l->ev_grids_copied, l->cstream));
@@ -944,25 +938,20 @@ int finish_wave(Lane* l, const WaveInput& wi, uint32_t mask, pcop_frame_result* 
     memset(&fp, 0, sizeof(fp));
     fp.n_clusters = r.n_clusters;
     if (mask & PCOP_OUT_FOOTPRINTS) fp.n_hull_vertices = H(CNT_HULL, f);
-    const void** slots[PK_N] = {(const void**)&r.crop_kept_idx,    (const void**)&r.voxel_keys,
-                                (const void**)&r.voxel_centroids,  (const void**)&r.sor_kept_idx,
-                                (const void**)&r.plane_inlier_idx, (const void**)&r.remaining_cloud,
-                                (const void**)&r.remaining_src_idx, (const void**)&r.cluster_offsets,
-                                (const void**)&r.cluster_indices,  (const void**)&r.obstacles,
-                                (const void**)&fp.boxes,           (const void**)&fp.hull_offsets,
-                                (const void**)&fp.hull_indices};
     for (int k = 0; k < PK_N; ++k) {
-      if (!(mask & kPkMask[k])) continue;
+      const PackArray& a = kPack[k];
+      if (!(mask & a.bit)) continue;
+      const void** slot = (const void**)((unsigned char*)(a.fp ? (void*)&fp : (void*)&r) + a.slot);
+      const size_t off = (size_t)meta.base_of(k) + run[k] * a.elem_bytes;
       if (dev_results) {  // device pointer into the pack buffer (it does not move)
-        *slots[k] = l->d_pack + (size_t)meta.base_of(k) + run[k] * kPkElem[k];
+        *slot = l->d_pack + off;
       } else {
-        // store the byte offset now; turned into a pointer once the host buffer can no longer move
-        const size_t off = base_off + (size_t)meta.base_of(k) + run[k] * kPkElem[k];
-        *slots[k] = (const void*)(uintptr_t)(off + 1);  // +1 so that offset 0 is distinguishable from NULL
-        if (k < PK_BOXES) l->fixups.push_back((size_t)((const unsigned char*)slots[k] - (const unsigned char*)out_all));
-        else l->fp_fixups.push_back((size_t)((const unsigned char*)slots[k] - (const unsigned char*)h->fp.data()));
+        // store the byte offset now; turned into a pointer once the host buffer can no longer move (out_all and h->fp,
+        // which hold the slots, do not move during the call)
+        *slot = (const void*)(uintptr_t)(base_off + off + 1);  // +1 so that offset 0 is distinguishable from NULL
+        l->fixups.push_back(slot);
       }
-      run[k] += (size_t)H(kPkCount[k], f);
+      run[k] += (size_t)H(a.count_row, f);
     }
     // algorithmic bytes (SURVEY 8d)
     double b = 0.0;
@@ -1081,7 +1070,6 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
     l->h_pack_used = 0;
     l->h_pack_sel ^= 1;
     l->fixups.clear();
-    l->fp_fixups.clear();
     l->wave_seq = 0;
     l->call_lane_waves = cdiv((int)waves.size(), (int)lanes.size());
     l->trace_used = 0;
@@ -1149,16 +1137,7 @@ int process_impl(pcop_handle* h, const float* xyzw, size_t frame_stride_points, 
   for (Lane* l : lanes) {
     h->sort_pass_keys += *l->h_stats;
     // the host pack buffers are final now: turn the stored offsets into pointers
-    for (size_t fx : l->fixups) {
-      const void** slot = (const void**)((unsigned char*)out + fx);
-      const size_t off = (size_t)(uintptr_t)(*slot) - 1;
-      *slot = l->h_pack() + off;
-    }
-    for (size_t fx : l->fp_fixups) {
-      const void** slot = (const void**)((unsigned char*)h->fp.data() + fx);
-      const size_t off = (size_t)(uintptr_t)(*slot) - 1;
-      *slot = l->h_pack() + off;
-    }
+    for (const void** slot : l->fixups) *slot = l->h_pack() + ((size_t)(uintptr_t)*slot - 1);
   }
   h->fp_ok = true;
   return PCOP_OK;

@@ -49,14 +49,36 @@ enum {  // packed output arrays
   PK_HULL_INDICES,
   PK_N
 };
-const int kPkElem[PK_N] = {4, 4, 16, 4, 4, 16, 4, 4, 4, 16, 32, 4, 4};
-const int kPkCount[PK_N] = {CNT_CROP, CNT_VOX,   CNT_VOX,  CNT_SOR,  CNT_NINL,  CNT_REM, CNT_REM,
-                            CNT_CLUS1, CNT_CLPTS, CNT_CLUS, CNT_CLUS, CNT_CLUS1, CNT_HULL};
-const uint32_t kPkMask[PK_N] = {PCOP_OUT_CROP,      PCOP_OUT_VOXEL,      PCOP_OUT_VOXEL,     PCOP_OUT_SOR,
-                                PCOP_OUT_PLANE,     PCOP_OUT_REMAINING,  PCOP_OUT_REMAINING, PCOP_OUT_CLUSTERS,
-                                PCOP_OUT_CLUSTERS,  PCOP_OUT_OBSTACLES,  PCOP_OUT_FOOTPRINTS, PCOP_OUT_FOOTPRINTS,
-                                PCOP_OUT_FOOTPRINTS};
-constexpr uint32_t kPkOutputs = (uint32_t)PCOP_OUT_ALL | (uint32_t)PCOP_OUT_FOOTPRINTS;  // the bits that pack arrays
+struct PackArray {  // one packed output array: row PK_* of kPack
+  uint32_t bit;     // the output bit that requests it
+  int count_row;    // elements of each frame's part
+  int elem_bytes;
+  bool csr;         // the lane buffer holds cap + 1 elements per frame (CSR offsets), not cap
+  bool fp;          // the result pointer is a field of pcop_frame_footprints, not of pcop_frame_result
+  size_t slot;      // offsetof that field
+};
+constexpr PackArray kPack[] = {
+    {PCOP_OUT_CROP, CNT_CROP, 4, false, false, offsetof(pcop_frame_result, crop_kept_idx)},
+    {PCOP_OUT_VOXEL, CNT_VOX, 4, false, false, offsetof(pcop_frame_result, voxel_keys)},
+    {PCOP_OUT_VOXEL, CNT_VOX, 16, false, false, offsetof(pcop_frame_result, voxel_centroids)},
+    {PCOP_OUT_SOR, CNT_SOR, 4, false, false, offsetof(pcop_frame_result, sor_kept_idx)},
+    {PCOP_OUT_PLANE, CNT_NINL, 4, false, false, offsetof(pcop_frame_result, plane_inlier_idx)},
+    {PCOP_OUT_REMAINING, CNT_REM, 16, false, false, offsetof(pcop_frame_result, remaining_cloud)},
+    {PCOP_OUT_REMAINING, CNT_REM, 4, false, false, offsetof(pcop_frame_result, remaining_src_idx)},
+    {PCOP_OUT_CLUSTERS, CNT_CLUS1, 4, true, false, offsetof(pcop_frame_result, cluster_offsets)},
+    {PCOP_OUT_CLUSTERS, CNT_CLPTS, 4, false, false, offsetof(pcop_frame_result, cluster_indices)},
+    {PCOP_OUT_OBSTACLES, CNT_CLUS, 16, false, false, offsetof(pcop_frame_result, obstacles)},
+    {PCOP_OUT_FOOTPRINTS, CNT_CLUS, 32, false, true, offsetof(pcop_frame_footprints, boxes)},
+    {PCOP_OUT_FOOTPRINTS, CNT_CLUS1, 4, true, true, offsetof(pcop_frame_footprints, hull_offsets)},
+    {PCOP_OUT_FOOTPRINTS, CNT_HULL, 4, false, true, offsetof(pcop_frame_footprints, hull_indices)},
+};
+static_assert(sizeof(kPack) / sizeof(kPack[0]) == PK_N, "one kPack row per PK_* entry");
+// (footprint rows last: a wave without PCOP_OUT_FOOTPRINTS packs and copies only the rows and counts before them)
+constexpr bool pack_row_ok(const PackArray& a, bool fp) {
+  return a.elem_bytes % 4 == 0 && a.fp == fp && (a.bit == PCOP_OUT_FOOTPRINTS) == fp && (a.count_row != CNT_HULL || fp);
+}
+constexpr bool pack_rows_ok(int k = 0) { return k == PK_N || (pack_row_ok(kPack[k], k >= PK_BOXES) && pack_rows_ok(k + 1)); }
+static_assert(pack_rows_ok(), "kPack: elements of whole 32-bit words (k_pack), footprint rows last");
 
 struct PlaneRecord {
   int n_passes;
@@ -324,8 +346,7 @@ struct Lane {
   int pend_w0 = 0, pend_B = 0;
   int pend_max_n = 1;
   WaveRoute route;                  // of the wave in flight
-  std::vector<size_t> fixups;  // result-pointer slots of the running call (byte offsets into the caller's array)
-  std::vector<size_t> fp_fixups;  // the same for the footprint pointers (byte offsets into pcop_handle::fp)
+  std::vector<const void**> fixups;  // result pointers of the running call that hold a pinned-buffer offset (finish_wave)
   struct TraceRec {
     int w0, B;
     size_t bytes;
@@ -391,10 +412,9 @@ inline uint32_t effective_outputs(const pcop_params& p) {
 inline int count_rows(uint32_t mask) { return (mask & PCOP_OUT_FOOTPRINTS) ? CNT_ROWS : CNT_HULL; }
 
 inline size_t pack_capacity_bytes(uint32_t mask, int B, int cap) {
-  mask &= kPkOutputs;
   size_t bytes = 0;
-  for (int k = 0; k < PK_N; ++k)
-    if (mask & kPkMask[k]) bytes += ((size_t)B * (cap + 1)) * kPkElem[k] + 256;
+  for (const PackArray& a : kPack)
+    if (mask & a.bit) bytes += ((size_t)B * (cap + 1)) * a.elem_bytes + 256;
   return (bytes + 256 + 255) & ~(size_t)255;
 }
 
